@@ -2,7 +2,7 @@
 """Headline benchmark (BASELINE.json): Chromoformer-clf default config, inference over 18,955
 synthetic genes per GPU (configs[1]); genes/s, weak scaling over N GPUs with no collective.
 
-    python bench.py [--gpus N --steps K --warmup W] [--mode infer|train] [--impl reference]
+    python bench.py [--gpus N --steps K --warmup W] [--mode infer|train] [--impl reference] [--dump-outputs DIR]
 
 One JSON line on rank 0.  A "step" is one full sweep of the hot path over this rank's 18,955
 genes.  `value` = genes of all ranks / max-over-ranks device time with inputs resident in HBM;
@@ -281,7 +281,9 @@ def workload_config(args):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=100,
+                    help="timed sweeps of the headline region (`value`); the ragged and e2e figures derive their own "
+                         "counts from it, and a headline region under 0.6 s is followed by a separate `sustained` one")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--mode", choices=["infer", "train"], default="infer")
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
@@ -295,7 +297,13 @@ def main():
     ap.add_argument("--no-train", action="store_true")
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--ref-batch", type=int, default=64, help="genes per step of the CPU reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the logits of the last timed sweep of the headline region (rank 0's genes) to "
+                         "DIR/logits.npy in float32; the inputs and weights are seeded, so two builds run with the same "
+                         "arguments compare array for array (not with --impl reference)")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path; it does not apply to --impl reference")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -307,6 +315,7 @@ def main():
     real_stdout = os.dup(1)
     os.dup2(2, 1)
 
+    import numpy as np
     import torch
     import torch.distributed as dist
     from chromoformer_b200 import ChromoformerClassifier, ChromoformerRegressor, _lib, synthetic
@@ -366,6 +375,9 @@ def main():
     launches_per_step = int(lib.chromo_launch_counter(1))
     t0 = time.time()
     ms = timed(lambda: eng.predict_device(resident, out), args.steps, args.warmup)
+    if args.dump_outputs and rank == 0:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        np.save(os.path.join(args.dump_outputs, "logits.npy"), out.cpu().numpy())
     # `value` is EXACTLY --steps sweeps (the driver's contract); a short region (20 steps = 0.13 s) is followed by a second,
     # >= 0.6 s region of the same step so that the clock samples and a sustained figure exist regardless of --steps
     sustained = None
@@ -583,7 +595,6 @@ def main():
                                   "hbm_peak_gbs": peaks["hbm_gbs"]}}
 
     # ---------------- input path kernel (data.py:68-113 on the device): HBM-bound byte work -------
-    import numpy as np
     n_reg, L = 4096, 40000                                  # 2.29 GB of FP16 depth: larger than L2
     raw = (torch.rand(n_reg * 7 * L // 2, device=dev) * 3).to(torch.float16)
     raw = torch.cat([raw, raw])[: n_reg * 7 * L]

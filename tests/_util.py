@@ -71,11 +71,12 @@ def as_dict(lst):
 
 
 def reference_available():
-    return os.path.isdir(os.environ.get("CHROMOFORMER_REF", "/root/reference"))
+    """True when $CHROMOFORMER_REF names a checkout of the upstream chromoformer repository."""
+    return os.path.isdir(os.environ.get("CHROMOFORMER_REF", ""))
 
 
 def import_reference():
-    ref = os.environ.get("CHROMOFORMER_REF", "/root/reference")
+    ref = os.environ["CHROMOFORMER_REF"]
     if not getattr(torch.Tensor.cuda, "_patched_identity", False) and not torch.cuda.is_available():
         ident_t = lambda self, *a, **k: self
         ident_t._patched_identity = True

@@ -114,9 +114,9 @@ def test_input_path_golden():
         assert np.abs(it["interaction_freq"] - items["freq"][idx]).max() < 1e-6
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not mounted (GPU box)")
+@pytest.mark.skipif(not reference_available(), reason="upstream chromoformer checkout not supplied ($CHROMOFORMER_REF)")
 def test_oracle_equals_live_reference():
-    """Direct comparison with the unmodified reference imported from /root/reference."""
+    """Direct comparison with the unmodified reference imported from $CHROMOFORMER_REF."""
     net, _ = import_reference()
     ref = net.ChromoformerRegressor(7, 128, 128, dict(KWS[0]), dict(KWS[1]), dict(KWS[2]), seed=5)
     batch = synthetic.make_batch(3, i_max=8, ragged=True, full_masks=True, seed=11, stress=True)

@@ -1,7 +1,7 @@
 """SURVEY §8c: the pretrained-checkpoint goldens (`demo/prediction.out`, `demo/prediction.reg.out`, AUC 0.9330 /
 AP 0.9417 / ACC 0.83 of demo/img/demo_result.png; R2 0.6224 / r 0.7944) pin the path as soon as the two `.pt` files of
 the reference's `.MISSING_LARGE_BLOBS` are supplied.  This test switches on automatically when either file is found under
-$CHROMOFORMER_PT_DIR, $CHROMOFORMER_REF/demo, /root/reference/demo or baseline/_ref/demo, and is skipped otherwise
+$CHROMOFORMER_PT_DIR, $CHROMOFORMER_REF/demo or baseline/_ref/demo, and is skipped otherwise
 (the published predictions themselves are committed: tests/golden/demo_pretrained_predictions.npz).
 
 Tolerances: FP32 path 2e-5 on the published predictions (as for random_prediction.out); BF16 path logits within 1e-2,
@@ -20,8 +20,8 @@ REG_PT = "chromoformer-reg-reproduction-E003-conf1-fold1.pt"
 
 
 def _find(name):
-    dirs = [os.environ.get("CHROMOFORMER_PT_DIR"), os.path.join(os.environ.get("CHROMOFORMER_REF", "/root/reference"), "demo"),
-            "/root/reference/demo", os.path.join(ROOT, "baseline", "_ref", "demo")]
+    dirs = [os.environ.get("CHROMOFORMER_PT_DIR"), os.path.join(os.environ.get("CHROMOFORMER_REF", ""), "demo"),
+            os.path.join(ROOT, "baseline", "_ref", "demo")]
     for d in dirs:
         if d and os.path.exists(os.path.join(d, name)):
             return os.path.join(d, name)

@@ -7,11 +7,12 @@ computes every bin of every slot, as the reference does) - no GPU, no plan invol
      features nor its pad mask nor its interaction_freq entry.
 
 Both are asserted bit-for-bit: the plan's eliminations are exact, not approximate."""
+import numpy as np
 import pytest
 import torch
 
-from _util import KWS, import_reference, reference_available
-from chromoformer_b200 import ChromoformerClassifier, synthetic
+from _util import KWS, golden, import_reference, reference_available
+from chromoformer_b200 import ChromoformerClassifier, ChromoformerRegressor, synthetic
 from oracle import chromoformer_oracle as oracle
 
 
@@ -52,9 +53,27 @@ def test_masked_bins_and_dummy_slots_cannot_reach_the_logits():
     assert torch.equal(_logits(sd, _perturbed(batch)), _logits(sd, batch))
 
 
-@pytest.mark.skipif(not reference_available(), reason="/root/reference not mounted (GPU box)")
+@pytest.mark.parametrize("tag", ["clf", "reg"])
+def test_junk_batch_gives_the_stored_reference_logits(tag):
+    """tests/golden/train_golden.npz holds the unmodified reference's logits of its seed-123 models on the seed-7 ragged
+    batch (genes with dummy pCRE slots and padded bins).  The oracle fed the same genes with junk under every pad mask and
+    in every dummy slot must reproduce them."""
+    g = golden("train_golden.npz")
+    batch = synthetic.make_batch(6, ragged=True, seed=7)
+    chk = np.array([batch["pcre_feats"][100].double().sum().item(), batch["interaction_freq"].double().sum().item(),
+                    float(batch["n_partners"].sum())])
+    if not np.allclose(chk, g["input_checksum"], rtol=0, atol=1e-9):
+        pytest.skip("torch RNG stream differs from the one the fixture was generated with")
+    assert (batch["n_partners"] < 8).any()
+    cls = ChromoformerClassifier if tag == "clf" else ChromoformerRegressor
+    model = cls(7, 128, 128, dict(KWS[0]), dict(KWS[1]), dict(KWS[2]), seed=123)
+    sd = {k: v.detach().clone() for k, v in model.state_dict().items()}
+    assert np.abs(_logits(sd, _perturbed(batch)).numpy() - g[f"{tag}_logits"]).max() < 2e-6
+
+
+@pytest.mark.skipif(not reference_available(), reason="upstream chromoformer checkout not supplied ($CHROMOFORMER_REF)")
 def test_same_facts_on_the_unmodified_reference():
-    """The reference's own forward (imported from /root/reference, CPU) gives identical logits for the two batches."""
+    """The reference's own forward (imported from $CHROMOFORMER_REF, CPU) gives identical logits for the two batches."""
     net, _ = import_reference()
     ref = net.ChromoformerClassifier(7, 128, 128, dict(KWS[0]), dict(KWS[1]), dict(KWS[2]), seed=5).eval()
     batch = synthetic.make_batch(6, ragged=True, seed=77)

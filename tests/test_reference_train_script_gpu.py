@@ -1,5 +1,5 @@
 """The reference's OWN training script (chromoformer/train.py, unmodified text) run against this package: the file is copied
-at test time from the staged reference (baseline/_ref, or /root/reference in the build container) into a temporary package
+at test time from the staged reference (baseline/_ref, or an upstream checkout named by $CHROMOFORMER_REF) into a temporary package
 whose `data` / `net` / `util` modules are this repo's drop-in names, and executed as `python -m <pkg>.train` with the
 reference's command line (train.py:26-37) on a tiny dataset - stock torch.optim.AdamW + StepLR on the flat-buffer
 parameters, `loss.backward()` through the C ABI, sklearn / scipy metrics on `out.cpu()`, checkpoint keys of train.py:322-343.
@@ -32,9 +32,9 @@ def log(*a, **k):
 
 
 def _reference_train_py():
-    for base in (os.path.join(ROOT, "baseline", "_ref"), os.environ.get("CHROMOFORMER_REF", "/root/reference")):
+    for base in (os.path.join(ROOT, "baseline", "_ref"), os.environ.get("CHROMOFORMER_REF", "")):
         p = os.path.join(base, "chromoformer", "train.py")
-        if os.path.exists(p):
+        if base and os.path.exists(p):
             return p
     return None
 

@@ -1,11 +1,15 @@
 """`python -m chromoformer.train` (reference CLI, train.py:26-37) end to end on a tiny synthetic dataset:
 same arguments and config schema, checkpoint written with the reference's keys (train.py:322-343) and
 loadable into a fresh model through the reference's inference path (run_demo.py:86-92)."""
+import os
+
 import numpy as np
 import pandas as pd
 import pytest
 import torch
 import yaml
+
+from _util import ROOT
 
 pytestmark = pytest.mark.gpu
 
@@ -39,7 +43,7 @@ def test_train_cli_writes_reference_checkpoint(tmp_path, regression):
     import chromoformer.train as train_cli
     from chromoformer import ChromoformerClassifier, ChromoformerDataset, ChromoformerRegressor
     meta = _make_dataset(tmp_path)
-    cfg = yaml.safe_load(open("chromoformer/configs/default.yaml"))
+    cfg = yaml.safe_load(open(os.path.join(ROOT, "chromoformer", "configs", "default.yaml")))
     cfg.update(num_epoch=3, bsz=4)                      # range(1, 3): two epochs
     cfg_path = tmp_path / "config.yaml"
     yaml.safe_dump(cfg, open(cfg_path, "w"))
