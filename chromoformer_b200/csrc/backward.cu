@@ -655,7 +655,6 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
     float* gcur = ws + o_tR0;           // gradient arriving at the layer's output
     float* gnext = ws + o_tR1;
     cudaStream_t wst = st;
-    static const bool wgrad_at_end = getenv("CHROMO_WGRAD_AT_END") != nullptr;
     if (part1) {
     // ---- head (net.py:377-380) ------------------------------------------------
     {
@@ -696,8 +695,7 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
             for (int r = 0; r < NR; ++r) a.imask[r] = in->imask[r];
             a.dgamma_f = G + ra.gamma_f; a.dgamma_z = L.reg_stride;
             dim3 grid((unsigned)(((long long)B * Hr + 7) / 8), NR);
-            static const bool per_warp = getenv("CHROMO_REG_ATTN_PER_THREAD") != nullptr;
-            if (Hr == 8 && S <= 17 && !per_warp) {       // one CTA per gene, rows staged in shared memory
+            if (Hr == 8 && S <= 17) {       // one CTA per gene, rows staged in shared memory
                 const size_t smem = ((size_t)S * (4 * dmr + RAB_PAD) + (size_t)S * dmr + 2 * (size_t)Hr * S * S + Hr * S) * sizeof(float);
                 static bool configured = false;
                 if (!configured) {
@@ -717,7 +715,7 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
         CHROMO_TRY(bwd_data(cx, dProj, 4 * dmr, GS, P + ra.att, L.reg_stride, gcur, D, GS, T, 4 * dmr, D, resid, NR));
         // gcur = dX of this layer = the gradient arriving at the output of layer l-1; gnext is free again
         // this layer's weight gradients start now, on the side stream and on 64 SMs, under the next layer's chain
-        if (tc && !wgrad_at_end) {
+        if (tc) {
             CHROMO_TRY(aux_fork(st, &wst));
             if (wst != st) CHROMO_TRY(queue.flush(wst, 64));
         }
@@ -789,7 +787,7 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
         CHROMO_TRY(gemm_auto(g, true, false, NR, st, tc));
     }
 
-    if (tc && !wgrad_at_end) {     // the Pairwise weight gradients follow on the side stream (ordered behind st)
+    if (tc) {     // the Pairwise weight gradients follow on the side stream (ordered behind st)
         CHROMO_TRY(aux_fork(st, &wst));
         if (wst != st) CHROMO_TRY(queue.flush(wst, 64));
     }
@@ -864,5 +862,5 @@ extern "C" int chromo_backward(const chromo_config_t* cfg, const float* params, 
     const bool only1 = (flags & CHROMO_F_BWD_HEAD_REG) != 0, only2 = (flags & CHROMO_F_BWD_REST) != 0;
     if (only1 && only2) { set_error("chromo_backward: CHROMO_F_BWD_HEAD_REG and CHROMO_F_BWD_REST are exclusive"); return CHROMO_EINVAL; }
     return backward_impl(cfg, params, in, dlogits, grads, workspace, w, (cudaStream_t)stream,
-                         (flags & CHROMO_F_BF16) != 0 && !getenv("CHROMO_BWD_FP32"), !only2, !only1);
+                         (flags & CHROMO_F_BF16) != 0, !only2, !only1);
 }

@@ -529,8 +529,7 @@ int launch_reg_attention(const RegAttnArgs& a, int nz, cudaStream_t st) {
         if (a.S <= 9) launch_pdl(reg_attention_kernel<9, __nv_bfloat16>, dim3(grid), dim3(wpb * 32), 0, st, a);
         else launch_pdl(reg_attention_kernel<17, __nv_bfloat16>, dim3(grid), dim3(wpb * 32), 0, st, a);
     } else {
-        static const bool per_thread = getenv("CHROMO_REG_ATTN_PER_THREAD") != nullptr;
-        if (a.H == 8 && a.S <= 17 && !per_thread) {       // one CTA per gene, rows staged in shared memory
+        if (a.H == 8 && a.S <= 17) {       // one CTA per gene, rows staged in shared memory
             const size_t smem = (size_t)a.S * (4 * 32 * a.H + RA_PAD) * sizeof(float);
             static bool configured = false;
             if (!configured) {
@@ -750,6 +749,14 @@ static int pack_all_weights(const chromo_config_t* c, const ParamLayout& L, cons
 
 struct RegOnly { int layer; const float* x; float* y; long long xy_stride; };
 
+// The side stream of aux_fork: joined back into `st` by join(), or on leaving the scope when an error return comes first
+// (a fork left open invalidates a stream capture).
+struct AuxStream {
+    cudaStream_t st, aux;
+    int join() { const cudaStream_t s = aux; aux = st; return aux_join(st, s); }
+    ~AuxStream() { join(); }
+};
+
 static int forward_impl(const chromo_config_t* c, const float* P, const chromo_batch_t* in, float* logits,
                         float* ws, const WsLayout& w, int flags, cudaStream_t st, const RegOnly* only = nullptr) {
     const ParamLayout& L = get_layout(c);
@@ -830,30 +837,38 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
         if (!have_tiles) CHROMO_TRY(sqa_pack_qk(qk, RS, reinterpret_cast<__nv_bfloat16*>(qkt), 2 * RS, regions * H, NR, st));
         return launch_sqa_fused(f, st);
     };
-    const bool tail = fold && w.tail_fused && !getenv("CHROMO_NO_TAIL_FUSED");
-    const bool cb16 = tail && !getenv("CHROMO_CBAR_FP32");     // Cbar handed from sqa_fused to the fused tail in BF16
+    const bool tail = fold && w.tail_fused;
+    const bool cb16 = tail;                     // Cbar handed from sqa_fused to the fused tail in BF16
+    // the query GEMM of a stage written as the operand tiles of sqa_fused
+    auto qk_tiles = [&](GemmArgs g, float* qkt) { g.c_sqa_tiles = 1; g.C = qkt; g.sC1 = 2 * RS; return g; };
     // the query GEMM of a stage: straight into the operand tiles of sqa_fused when that kernel will run and the tensor
     // GEMM takes the shape, FP32 rows otherwise
     auto qk_gemm = [&](const GemmArgs& g, float* qkt, bool sqa_ok, bool* tiles) -> int {
-        *tiles = false;
-        if (sqa_ok && !getenv("CHROMO_QK_FP32")) {
-            GemmArgs t = g;
-            t.c_sqa_tiles = 1; t.C = qkt; t.sC1 = 2 * RS;
-            if (umma_supported(t)) { *tiles = true; return lin(t, NR); }
-        }
-        if (g.a_rows || g.m_dev) { set_error("internal: ragged plan without the persistent query GEMM"); return CHROMO_EINVAL; }
-        return lin(g, NR);
+        const GemmArgs t = qk_tiles(g, qkt);
+        *tiles = sqa_ok && umma_supported(t);
+        return lin(*tiles ? t : g, NR);
+    };
+    // the folded query GEMM of Pairwise layer l over its input rows: QK = P_l M^T
+    auto pw_qk = [&](int l, const float* pin, int pin_div) {
+        GemmArgs g = gemm_args();
+        g.A = pin; g.lda = D; g.sA1 = RS; g.a_div = pin_div;
+        g.B = ws + w.fold_f32 + w.fold_slot[1 + l]; g.ldb = D; g.sB1 = w.fold_stride;
+        g.C = ws + w.p_qk + (long long)w.pslot(l) * w.p_slot; g.ldc = c->pw_heads * D; g.sC1 = RS;
+        g.M = R; g.N = c->pw_heads * D; g.K = D;
+        return g;
     };
     // Ragged plan (ragged.cu): the Pairwise stage runs over the live pCRE slots only, sorted by valid length, each tile
-    // of the attention over its own key window.  Needs the fused kernels of the stage (they take the row maps).
+    // of the attention over its own key window.  Built when every consumer of the stage takes it, as their own predicates
+    // say for layer 0: sqa_fused, the fused tail, and the query GEMM in its operand-tile form on the persistent kernel
+    // (qk_tiles_kernel).  Later layers differ from layer 0 only by workspace offsets, which keep the 16-byte alignment.
     RaggedArgs ra;
-    cudaStream_t plan_stream = st;
-    if (tail && w.rg_plan && c->pw_layers > 0 && c->pw_heads * D == 256 && D == 128 && (R + 127) / 128 >= 8 && !(flags & CHROMO_F_DENSE) && !getenv("CHROMO_NO_RAGGED") &&
-        !getenv("CHROMO_QK_FP32") && !getenv("CHROMO_QK_ONE_TILE")) {
+    AuxStream plan_stream{st, st};
+    if (tail && w.rg_plan && c->pw_layers > 0 && !(flags & CHROMO_F_DENSE)) {
         bool ok = false;
         CHROMO_TRY(sqa_fused(R, c->pw_heads, in->x_pcre, in->mask_pcre, in->mask_pcre_stride, in->mask_pcre_row_offset,
                              L.pw[0].lin_proj_pcre, L.pw_stride, 1, c->pw_d_model, ws + w.p_qk, ws + w.p_qkt, ws + w.p_cbar, cb16, true, false, &ok));
-        if (ok) {
+        const GemmArgs q0 = qk_tiles(pw_qk(0, ws + w.p_pp, I), ws + w.p_qkt);
+        if (ok && umma_supported(q0) && umma_qk_persistent(q0)) {
             ra.B = B; ra.I = I; ra.n_res = NR;
             for (int r = 0; r < NR; ++r) {
                 ra.n[r] = c->n_bins[r]; ra.ns[r] = c->n_bins[r] <= 32 ? 32 : c->n_bins[r];
@@ -864,7 +879,7 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
             // on a side stream next to the Embedding stage: forked here, launched behind that stage's kernels (which then
             // come first for the block scheduler; the plan's small latency-bound kernels fill the room they leave), joined
             // in front of the Pairwise stage
-            CHROMO_TRY(aux_fork(st, &plan_stream));
+            CHROMO_TRY(aux_fork(st, &plan_stream.aux));
             ragged = true;
         }
     }
@@ -972,8 +987,8 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
         CHROMO_TRY(lin(g, NR));
     }
     if (ragged) {
-        CHROMO_TRY(build_ragged_plan(ra, ws + w.rg_plan, &plan, plan_stream));
-        CHROMO_TRY(aux_join(st, plan_stream));
+        CHROMO_TRY(build_ragged_plan(ra, ws + w.rg_plan, &plan, plan_stream.aux));
+        CHROMO_TRY(plan_stream.join());
     }
     const RaggedPlan* rp = ragged ? &plan : nullptr;
     for (int l = 0; l < c->pw_layers; ++l) {
@@ -988,11 +1003,7 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
                              L.pw[0].lin_proj_pcre, L.pw_stride, 1, dmp, ws + w.p_qk + so, ws + w.p_qkt + so, ws + w.p_cbar + so,
                              cb16, true, false, &p_fused));
         if (fold) {   // QK = P_l M^T
-            GemmArgs g = gemm_args();
-            g.A = pin; g.lda = D; g.sA1 = RS; g.a_div = pin_div;
-            g.B = ws + w.fold_f32 + w.fold_slot[1 + l]; g.ldb = D; g.sB1 = w.fold_stride;
-            g.C = ws + w.p_qk + so; g.ldc = Hp * D; g.sC1 = RS;
-            g.M = R; g.N = Hp * D; g.K = D;
+            GemmArgs g = pw_qk(l, pin, pin_div);
             if (rp) { g.m_dev = rp->live; g.a_rows = l == 0 ? rp->perm : nullptr; }   // (later layers read the compacted rows)
             CHROMO_TRY(qk_gemm(g, ws + w.p_qkt + so, p_fused, &p_tiles));
         } else {      // Q = P_l W_q^T                             modules.py:159
@@ -1006,7 +1017,6 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
         CHROMO_TRY(sqa_fused(R, Hp, in->x_pcre, in->mask_pcre, in->mask_pcre_stride, in->mask_pcre_row_offset,
                              L.pw[0].lin_proj_pcre, L.pw_stride, 1, dmp, ws + w.p_qk + so, ws + w.p_qkt + so, ws + w.p_cbar + so,
                              cb16, false, p_tiles, &p_fused, rp));
-        if (rp && !(p_fused && p_tiles)) { set_error("internal: ragged plan without the fused single-query attention"); return CHROMO_EINVAL; }
         ResStreams prs;
         if (!p_fused) CHROMO_TRY(res_fork(st, NR, prs));
         for (int r = 0; r < NR && !p_fused; ++r) {
@@ -1100,14 +1110,14 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
         float* xout = ws + w.r_out + so;
         long long x_z = RS, y_z = RS;
         if (only) { xin = only->x; xout = only->y; x_z = y_z = only->xy_stride; }
-        if (w.reg_fused && !reg_fp32 && !getenv("CHROMO_NO_REG_FUSED")) {
-            // whole layer in one launch (reg_fused.cu); with the tensor-pipe attention ALL layers in one launch:
-            // a CTA keeps its 14 genes on chip from layer to layer (the tokens of a gene only attend to each other)
-            const bool all = (!only || only->layer < 0) && reg_fused_tensor_attention() && !getenv("CHROMO_REG_PER_LAYER");
+        if (w.reg_fused && !reg_fp32) {
+            // ALL layers in one launch (reg_fused.cu), unless the caller asked for one layer: a CTA keeps its 14 genes on
+            // chip from layer to layer (the tokens of a gene only attend to each other)
+            const bool all = !only || only->layer < 0;
             if (all && l > 0) continue;
             RegFusedArgs a;
             a.B = B; a.S = S; a.G = 128 / S; a.n_tiles = (B + a.G - 1) / a.G;
-            if (ragged && all && !getenv("CHROMO_NO_RAGGED_REG")) {
+            if (ragged && all) {
                 // token classes of the plan: a tile holds genes of one class with their live tokens only
                 a.plan_tiles = plan.reg_tiles; a.plan_rows = plan.reg_rows; a.n_tiles = plan.reg_tiles_max;
                 reg_plan = true;
@@ -1263,8 +1273,7 @@ extern "C" int chromo_regulation_layer(const chromo_config_t* cfg, const float* 
         if (!imask[r]) { set_error("chromo_regulation_layer: null interaction mask"); return CHROMO_EINVAL; }
         in.imask[r] = imask[r];
     }
-    if (layer < 0 && !((flags & CHROMO_F_BF16) && w.reg_fused && reg_fused_tensor_attention() && !getenv("CHROMO_NO_REG_FUSED") &&
-                       !getenv("CHROMO_REG_PER_LAYER"))) {
+    if (layer < 0 && !((flags & CHROMO_F_BF16) && w.reg_fused)) {
         set_error("chromo_regulation_layer: layer < 0 (all layers in one launch) needs the fused BF16 kernel");
         return CHROMO_EINVAL;
     }

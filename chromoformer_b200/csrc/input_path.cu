@@ -259,7 +259,7 @@ extern "C" int chromo_bin_regions(const uint16_t* raw, const chromo_region_t* re
         for (int r = 1; r < n_res; ++r) if (a.bin[r] < a.bin[fine]) fine = r;
         long long max_width = 0;      // longer regions are truncated to n_bins anyway (data.py requires L <= w_max)
         for (int r = 0; r < n_res; ++r) max_width = max_width > (long long)a.nb[r] * a.bin[r] ? max_width : (long long)a.nb[r] * a.bin[r];
-        bool ok = max_width > 0 && !getenv("CHROMO_BIN_GENERIC");
+        bool ok = max_width > 0;
         long long l = 1;
         for (int r = 0; r < n_res && ok; ++r) {
             if (a.bin[r] % a.bin[fine] != 0) { ok = false; break; }

@@ -326,10 +326,9 @@ SideStreams g_side[16];
 }  // namespace
 
 static SideStreams* side_streams() {
-    static const bool off = getenv("CHROMO_NO_RES_STREAMS") != nullptr;
     int dev = 0;
     cudaGetDevice(&dev);
-    if (off || dev < 0 || dev >= 16) return nullptr;
+    if (dev < 0 || dev >= 16) return nullptr;
     SideStreams& g = g_side[dev];
     if (g.device != dev) {
         for (int r = 1; r < CHROMO_MAX_RES; ++r) {

@@ -1,23 +1,24 @@
-// One Regulation-transformer layer (modules.py:28-30,37-88,100-101 with gate=True) as ONE kernel.
+// Regulation-transformer layers (modules.py:28-30,37-88,100-101 with gate=True) as ONE kernel: one layer or all of them.
 //
-// A CTA owns a tile of G genes (G*S <= 128 token rows) for the whole layer; activations never
-// leave the SM between the fused projection and the layer output:
+// A CTA owns a tile of G genes (G*S <= 128 token rows) from the first layer of the launch to the last (the tokens of a
+// gene only attend to each other); activations never leave the SM inside a layer, and between layers only the FP32
+// residual rows go out, to a scratch slot that stays in L2:
 //
 //   X (FP32, HBM) -> BF16 A-operand in shared memory
-//   for each pair of heads t = 0..3:
-//       [q|k] and [v|gate] = X W^T          2 x (8 tcgen05.mma 128x128x16) -> TMEM (double buffered)
-//       k, v  TMEM -> shared (BF16);  one thread per (token, head): scores vs the gene's S keys,
-//       gamma*freq bias, mask(-1e9), softmax, P.V, sigmoid gate -> BF16 into the out-proj A-operand
+//   per layer, for each pair of heads t = 0..3:
+//       [q|k] and [v|gate] = X W^T          2 x (8 tcgen05.mma 128x128x16) -> TMEM
+//       S = Q K^T on the tensor pipe (q, k in BF16), block-diagonal over the genes of the tile -> TMEM;
+//       gamma*freq bias, mask(-1e9), softmax over the gene's own S keys -> P (BF16, TMEM);
+//       O = P V on the tensor pipe -> sigmoid gate -> BF16 into the out-proj A-operand
 //   out-proj (K = 256, two chunks) -> TMEM -> + bias + residual X -> LayerNorm -> U (registers + BF16 operand)
 //   FFN-1 (N = 256, two chunks)    -> TMEM -> + bias, ReLU -> BF16 operand
-//   FFN-2 (K = 256, two chunks)    -> TMEM -> + bias + U -> LayerNorm -> Y (FP32, HBM, coalesced)
+//   FFN-2 (K = 256, two chunks)    -> TMEM -> + bias + U -> LayerNorm -> Y (next layer's operand; FP32, HBM, coalesced)
 //
 // The 14 weight chunks of a layer ([128 x 128] BF16 each, 448 KB, pre-packed in consumption
 // order by pack_reg_stream) are streamed through a 3-deep ring of 32 KB stages by 1-D TMA bulk
-// copies; a dedicated driver warp issues the copies and all tcgen05.mma, eight compute warps do
-// the TMEM epilogues and the attention.  mbarriers carry every hand-off.
-#include <stdlib.h>
-
+// copies.  Warps 0..15 compute (attention, TMEM epilogues), warp 16 issues the dense tcgen05.mma, warp 17 loads the
+// weight stream, warps 18 and 19 issue S = Q K^T and O = P V of one head each.  mbarriers carry every hand-off.
+// Under a ragged plan (ragged.cu) a tile holds genes of one token class with their live tokens only.
 #include "common.cuh"
 #include "kernels.cuh"
 #include "reg_fused.cuh"
@@ -27,7 +28,6 @@ namespace chromo {
 
 namespace {
 
-constexpr int RF_THREADS = 288;            // 8 compute warps + 1 driver warp
 constexpr int RF_NSTAGE = 3;
 constexpr int RF_CHUNK_ELEMS = 128 * 128;
 constexpr uint32_t RF_CHUNK_BYTES = RF_CHUNK_ELEMS * 2;
@@ -37,15 +37,12 @@ constexpr int RF_NCHUNK = 14;
 constexpr uint32_t OFF_XB = 0;                              // [128 x 128] BF16 operand (X, later U)
 constexpr uint32_t OFF_ATT = 32768;                         // [128 x 256] BF16 operand (att, later F, later store staging)
 constexpr uint32_t OFF_STAGE = OFF_ATT + 65536;             // 3 x 32 KB weight ring
-constexpr uint32_t OFF_K = OFF_STAGE + RF_NSTAGE * RF_CHUNK_BYTES;   // [128 x 64] BF16, 16-byte chunks XOR-swizzled by row
-constexpr uint32_t OFF_V = OFF_K + 16384;
+constexpr uint32_t OFF_K = OFF_STAGE + RF_NSTAGE * RF_CHUNK_BYTES;   // k of the two heads in flight (BF16, K-major, 8 KB each)
+constexpr uint32_t OFF_V = OFF_K + 16384;                   // v of the two heads in flight (BF16, MN-major, 8 KB each)
 constexpr uint32_t OFF_CTL = OFF_V + 16384;                 // mbarriers + TMEM slot
 constexpr uint32_t OFF_ROWMAP = OFF_CTL + 256;              // ragged plan: [B*S, 128]-layout row of every tile row (128 ints)
 constexpr uint32_t RF_SMEM = OFF_ROWMAP + 512;
 static_assert(RF_SMEM <= 227 * 1024, "shared memory budget");
-
-enum { B_FULL0 = 0, B_FREE0 = 3, B_ACCQ0 = 6, B_ACCQFREE0 = 8, B_XREADY = 10, B_ATTREADY, B_UREADY, B_FREADY,
-       B_ACCO, B_ACCF1, B_ACCF2, B_QKVR0, B_SR0 = B_QKVR0 + 2, B_PR0 = B_SR0 + 2, B_OR0 = B_PR0 + 2, B_QKFREE = B_OR0 + 2, B_ACCVG, B_COUNT };
 
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
     asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
@@ -54,14 +51,8 @@ __device__ __forceinline__ void warp_arrive(uint64_t* bar, int lane) {
     __syncwarp();
     if (lane == 0) mbar_arrive(bar);
 }
-__device__ __forceinline__ void compute_barrier() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
-// the four warps that serve one of the two heads in flight
-__device__ __forceinline__ void group_barrier(int ch) {
-    if (ch) asm volatile("bar.sync 3, 128;" ::: "memory");
-    else asm volatile("bar.sync 2, 128;" ::: "memory");
-}
 
-// o * sigmoid(g) with sigmoid(g) = 0.5 + 0.5 tanh(g / 2): one MUFU (tanh.approx, abs. error 2^-11, well inside the
+// sigmoid(g) = 0.5 + 0.5 tanh(g / 2): one MUFU (tanh.approx, abs. error 2^-11, well inside the
 // BF16 rounding of the result) instead of ex2 + rcp.  (Rows past the tile's last gene carry finite garbage that only
 // reaches their own, never stored, output rows.)
 __device__ __forceinline__ float gate_factor(float g) {
@@ -69,22 +60,9 @@ __device__ __forceinline__ float gate_factor(float g) {
     asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.5f * g));
     return fmaf(0.5f, t, 0.5f);
 }
-__device__ __forceinline__ float gated(float o, float g) {
-    float t;
-    asm("tanh.approx.f32 %0, %1;" : "=f"(t) : "f"(0.5f * g));
-    return o * fmaf(0.5f, t, 0.5f);
-}
 __device__ __forceinline__ uint32_t pack2(float a, float b) {
     __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
     return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ void unpack8(const uint4& u, float* v) {
-    const uint32_t w[4] = {u.x, u.y, u.z, u.w};
-#pragma unroll
-    for (int k = 0; k < 4; ++k) {
-        v[2 * k] = __uint_as_float(w[k] << 16);
-        v[2 * k + 1] = __uint_as_float(w[k] & 0xffff0000u);
-    }
 }
 // byte offset of the 16-byte chunk holding columns [8*kc, 8*kc+8) of `row` in a K-major operand of K columns
 __device__ __forceinline__ uint32_t op_chunk(int row, int kc, int K) {
@@ -170,449 +148,8 @@ __device__ __forceinline__ void build_p_window(const float* p, int c, uint32_t* 
 
 }  // namespace
 
-template <int SMAX>
-__global__ void __launch_bounds__(RF_THREADS, 1) reg_layer_cc_kernel(const RegFusedArgs a) {
-    extern __shared__ __align__(1024) uint8_t smem[];
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + OFF_CTL);
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + B_COUNT);
-    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int z = blockIdx.y, tile = blockIdx.x;
-    constexpr int S = SMAX;                                   // exact tokens per gene: no per-key predicates
-    const int G = a.G;
-    const long long row0 = (long long)tile * G * S;            // first token row of this tile
-    const int rows_valid = min((long long)G * S, (long long)a.B * S - row0);
-
-    if (warp == 0) tmem_alloc(tmem_slot, 512);
-    if (tid == 0) {
-        for (int i = 0; i < RF_NSTAGE; ++i) { mbar_init(&bars[B_FULL0 + i], 1); mbar_init(&bars[B_FREE0 + i], 1); }
-        mbar_init(&bars[B_ACCQ0], 1); mbar_init(&bars[B_ACCQ0 + 1], 1);
-        mbar_init(&bars[B_ACCQFREE0], 8); mbar_init(&bars[B_ACCQFREE0 + 1], 8);
-        mbar_init(&bars[B_XREADY], 8); mbar_init(&bars[B_ATTREADY], 8);
-        mbar_init(&bars[B_UREADY], 8); mbar_init(&bars[B_FREADY], 8);
-        mbar_init(&bars[B_ACCO], 1); mbar_init(&bars[B_ACCF1], 1); mbar_init(&bars[B_ACCF2], 1);
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&bars[B_QKVR0 + i], 4); mbar_init(&bars[B_SR0 + i], 1);
-            mbar_init(&bars[B_PR0 + i], 4); mbar_init(&bars[B_OR0 + i], 1);
-        }
-        mbar_init(&bars[B_QKFREE], 8);
-        mbar_init(&bars[B_ACCVG], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem = *tmem_slot;
-
-    if (warp == 8) {
-        // ===================================================== driver: TMA + tcgen05.mma ====
-        if (lane == 0) {
-            const __nv_bfloat16* wsrc = a.wstream + z * a.w_z;
-            const int n_chunks = RF_NCHUNK * a.n_layers;   // the layers' chunks follow each other in the stream
-            const uint32_t idesc = umma_idesc_bf16(128, 128);
-            const uint32_t s_xb = smem_u32(smem + OFF_XB), s_att = smem_u32(smem + OFF_ATT);
-            auto issue_load = [&](int c) {
-                const int st = c % RF_NSTAGE;
-                if (c >= RF_NSTAGE) mbar_wait(&bars[B_FREE0 + st], ((c / RF_NSTAGE) - 1) & 1);
-                mbar_expect_tx(&bars[B_FULL0 + st], RF_CHUNK_BYTES);
-                tma_bulk_g2s(smem + OFF_STAGE + st * RF_CHUNK_BYTES, wsrc + (long long)c * RF_CHUNK_ELEMS, RF_CHUNK_BYTES,
-                             &bars[B_FULL0 + st]);
-            };
-            auto consume = [&](int c, uint32_t a_addr, uint32_t a_sbo, uint32_t col, bool accumulate) {
-                const int st = c % RF_NSTAGE;
-                mbar_wait(&bars[B_FULL0 + st], (c / RF_NSTAGE) & 1);
-                tc_fence_after();
-                const uint32_t b_addr = smem_u32(smem + OFF_STAGE + st * RF_CHUNK_BYTES);
-                // descriptors once per chunk, then plain adds (+256 B = +16 in the address field): building them per MMA
-                // costs the issuing thread ~120 cycles per instruction against the 64-cycle MMA (tools/bench_micro/mma_rate.cu)
-                const uint64_t ad = umma_smem_desc(a_addr, 128, a_sbo), bd = umma_smem_desc(b_addr, 128, 2048);
-#pragma unroll
-                for (int k = 0; k < 8; ++k)
-                    umma_bf16(tmem + col, ad + 16 * k, bd + 16 * k, idesc, (accumulate || k > 0) ? 1u : 0u);
-                umma_commit(&bars[B_FREE0 + st]);
-                // refill the ring behind the MMAs just queued (waits for chunk c-1 only)
-                if (c + 2 < n_chunks && c >= 1) issue_load(c + 2);
-            };
-            issue_load(0);
-            issue_load(1);
-            issue_load(2);
-            for (int li = 0; li < a.n_layers; ++li) {
-            const int cb = li * RF_NCHUNK;
-            const uint32_t lp = li & 1;
-            mbar_wait(&bars[B_XREADY], lp);
-            for (int t = 0; t < 4; ++t) {
-                const int buf = t & 1;
-                if (t >= 2) mbar_wait(&bars[B_ACCQFREE0 + buf], 0);
-                consume(cb + 2 * t, s_xb, 2048, 256 * buf, false);          // [q | k] of heads 2t, 2t+1
-                consume(cb + 2 * t + 1, s_xb, 2048, 256 * buf + 128, false); // [v | gate]
-                umma_commit(&bars[B_ACCQ0 + buf]);
-            }
-            mbar_wait(&bars[B_ATTREADY], lp);
-            consume(cb + 8, s_att, 4096, 0, false);                     // out-projection, K halves
-            consume(cb + 9, s_att + 2048, 4096, 0, true);
-            umma_commit(&bars[B_ACCO]);
-            mbar_wait(&bars[B_UREADY], lp);
-            consume(cb + 10, s_xb, 2048, 256, false);                   // FFN-1, N halves
-            consume(cb + 11, s_xb, 2048, 384, false);
-            umma_commit(&bars[B_ACCF1]);
-            mbar_wait(&bars[B_FREADY], lp);
-            consume(cb + 12, s_att, 4096, 0, false);                    // FFN-2, K halves
-            consume(cb + 13, s_att + 2048, 4096, 0, true);
-            umma_commit(&bars[B_ACCF2]);
-            }   // layers
-        }
-    } else {
-        // ===================================================== compute warps =================
-        const int lq = warp & 3, ch = warp >> 2;
-        const int row = lq * 32 + lane;                      // tile row == TMEM lane
-        const bool valid = row < rows_valid;
-        const long long grow = row0 + row;
-        const uint32_t trow = tmem + ((uint32_t)(lq * 32) << 16);
-        const float* X = a.x + z * a.x_z;
-        float v[32];
-
-        // ---- phase 0 (first layer only; later layers get their operand from phase 4): X -> BF16 operand
-        {
-            float4 x[8][2];                                   // all 16 loads of the thread in flight at once
-            int r_[8], kc_[8];
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                const int u = warp + (q >> 2) * 32 + (q & 3) * 8;
-                r_[q] = (u & 15) * 8 + (lane >> 2);
-                kc_[q] = (u >> 4) * 4 + (lane & 3);
-                x[q][0] = x[q][1] = make_float4(0.f, 0.f, 0.f, 0.f);
-                if (r_[q] < rows_valid) {
-                    const float* p = X + (row0 + r_[q]) * 128 + kc_[q] * 8;
-                    x[q][0] = __ldg(reinterpret_cast<const float4*>(p));
-                    x[q][1] = __ldg(reinterpret_cast<const float4*>(p + 4));
-                }
-            }
-#pragma unroll
-            for (int q = 0; q < 8; ++q) {
-                uint4 pk;
-                pk.x = pack2(x[q][0].x, x[q][0].y); pk.y = pack2(x[q][0].z, x[q][0].w);
-                pk.z = pack2(x[q][1].x, x[q][1].y); pk.w = pack2(x[q][1].z, x[q][1].w);
-                *reinterpret_cast<uint4*>(smem + OFF_XB + op_chunk(r_[q], kc_[q], 128)) = pk;
-            }
-            fence_async_smem();
-            warp_arrive(&bars[B_XREADY], lane);
-        }
-
-        // ---- phase 1: per pair of heads: k, v -> shared; attention; att -> BF16 operand
-        const int gl = row / S, qi = row % S;                 // gene within tile, query token
-        const long long gene = (long long)tile * G + gl;
-        const float* freq = a.freq + (valid ? (gene * S + qi) * S : 0);
-        const uint8_t* mask = a.imask[z] + (valid ? (gene * S + qi) * S : 0);
-        const float scale = 0.17677669529663687f;            // 1/sqrt(32)
-        float fr[SMAX];
-        unsigned mbits = 0;
-#pragma unroll
-        for (int j = 0; j < SMAX; ++j) {
-            fr[j] = 0.f;
-            if (j < S && valid) {
-                fr[j] = freq[j];
-                if (mask[j]) mbits |= 1u << j;
-            }
-        }
-        for (int li = 0; li < a.n_layers; ++li) {
-        const uint32_t lp = li & 1;
-        const long long po = z * a.p_z + li * a.p_l;          // this (resolution, layer)'s parameters
-        for (int t = 0; t < 4; ++t) {
-            const int buf = t & 1;
-            const uint32_t qb = trow + 256 * buf;
-            mbar_wait(&bars[B_ACCQ0 + buf], (t >> 1) & 1);
-            tc_fence_after();
-            compute_barrier();                                // previous pair's readers are done with sK / sV
-            {   // ch 0 copies k (cols 64..127), ch 1 copies v (cols 128..191)
-                uint8_t* dst = smem + (ch == 0 ? OFF_K : OFF_V) + row * 128;
-#pragma unroll
-                for (int half = 0; half < 2; ++half) {
-                    tmem_ld32(qb + 64 + 64 * ch + 32 * half, v);
-#pragma unroll
-                    for (int c = 0; c < 4; ++c) {
-                        uint4 pk;
-                        pk.x = pack2(v[8 * c], v[8 * c + 1]); pk.y = pack2(v[8 * c + 2], v[8 * c + 3]);
-                        pk.z = pack2(v[8 * c + 4], v[8 * c + 5]); pk.w = pack2(v[8 * c + 6], v[8 * c + 7]);
-                        *reinterpret_cast<uint4*>(dst + (((half * 4 + c) ^ (row & 7)) << 4)) = pk;
-                    }
-                }
-            }
-            compute_barrier();
-            // one thread per (token row, head 2t + ch)
-            const int head = 2 * t + ch;
-            float q[32];
-            tmem_ld32(qb + 32 * ch, q);
-            const float gamma = a.gamma_f[po + head];
-            float s[SMAX];
-            float mx = -INFINITY;
-#pragma unroll
-            for (int j = 0; j < SMAX; ++j) {
-                s[j] = -INFINITY;
-                if (j < S) {
-                    const int kr = gl * S + j;
-                    const uint8_t* kp = smem + OFF_K + (kr & 127) * 128;
-                    float d0 = 0.f, d1 = 0.f;
-#pragma unroll
-                    for (int c = 0; c < 4; ++c) {
-                        float kv[8];
-                        unpack8(*reinterpret_cast<const uint4*>(kp + (((4 * ch + c) ^ (kr & 7)) << 4)), kv);
-#pragma unroll
-                        for (int e = 0; e < 8; e += 2) {
-                            d0 = fmaf(q[8 * c + e], kv[e], d0);
-                            d1 = fmaf(q[8 * c + e + 1], kv[e + 1], d1);
-                        }
-                    }
-                    float sc = fmaf(gamma, fr[j], (d0 + d1) * scale);
-                    if ((mbits >> j) & 1u) sc = -1e9f;
-                    s[j] = sc;
-                    mx = fmaxf(mx, sc);
-                }
-            }
-            float sum = 0.f;
-#pragma unroll
-            for (int j = 0; j < SMAX; ++j)
-                if (j < S) { s[j] = __expf(s[j] - mx); sum += s[j]; }
-            const float inv = 1.f / sum;
-            float o[32];
-#pragma unroll
-            for (int d = 0; d < 32; ++d) o[d] = 0.f;
-#pragma unroll
-            for (int j = 0; j < SMAX; ++j) {
-                if (j < S) {
-                    const float p = s[j] * inv;
-                    const int kr = gl * S + j;
-                    const uint8_t* vp = smem + OFF_V + (kr & 127) * 128;
-#pragma unroll
-                    for (int c = 0; c < 4; ++c) {
-                        float vv[8];
-                        unpack8(*reinterpret_cast<const uint4*>(vp + (((4 * ch + c) ^ (kr & 7)) << 4)), vv);
-#pragma unroll
-                        for (int e = 0; e < 8; ++e) o[8 * c + e] = fmaf(p, vv[e], o[8 * c + e]);
-                    }
-                }
-            }
-            tmem_ld32(qb + 192 + 32 * ch, v);                 // gate
-            tc_fence_before();
-            warp_arrive(&bars[B_ACCQFREE0 + buf], lane);      // this TMEM half may be overwritten
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-                float r[8];
-#pragma unroll
-                for (int e = 0; e < 8; ++e) r[e] = gated(o[8 * c + e], v[8 * c + e]);
-                uint4 pk;
-                pk.x = pack2(r[0], r[1]); pk.y = pack2(r[2], r[3]); pk.z = pack2(r[4], r[5]); pk.w = pack2(r[6], r[7]);
-                *reinterpret_cast<uint4*>(smem + OFF_ATT + op_chunk(row, 8 * t + 4 * ch + c, 256)) = pk;
-            }
-        }
-        fence_async_smem();
-        warp_arrive(&bars[B_ATTREADY], lane);
-
-        // residual rows of phase 2 (FP32): issued now so that their latency hides behind the out-projection MMA; u_keep
-        // then carries U and is the residual of phase 4.  First layer: the caller's row-major X.  Later layers: what THIS
-        // thread parked in the scratch slot at the end of the previous layer, in a lane-major order (float4 index
-        // ((ch*2 + ci)*8 + j/4)*128 + row inside the tile's 64 KB block) so that every warp access is 512 contiguous bytes.
-        float u_keep[2][32];
-        if (li == 0) {
-#pragma unroll
-            for (int ci = 0; ci < 2; ++ci) {
-                const int c = (2 * ci + ch) * 32;
-#pragma unroll
-                for (int j = 0; j < 32; j += 4) {
-                    float4 r4 = make_float4(0.f, 0.f, 0.f, 0.f);
-                    if (valid) r4 = __ldg(reinterpret_cast<const float4*>(X + grow * 128 + c + j));
-                    u_keep[ci][j] = r4.x; u_keep[ci][j + 1] = r4.y; u_keep[ci][j + 2] = r4.z; u_keep[ci][j + 3] = r4.w;
-                }
-            }
-        } else {
-            const float4* park = reinterpret_cast<const float4*>(a.y_mid + z * a.y_mid_z + ((li - 1) & 1) * a.y_l) +
-                                 (long long)tile * 4096 + row;
-#pragma unroll
-            for (int ci = 0; ci < 2; ++ci)
-#pragma unroll
-                for (int j = 0; j < 32; j += 4) {
-                    const float4 r4 = __ldcg(park + ((ch * 2 + ci) * 8 + (j >> 2)) * 128);
-                    u_keep[ci][j] = r4.x; u_keep[ci][j + 1] = r4.y; u_keep[ci][j + 2] = r4.z; u_keep[ci][j + 3] = r4.w;
-                }
-        }
-        // small FP32 vectors of the layer -> shared (the v tile is dead): bo, ln1w, ln1b, b2, ln2w, ln2b, b1[256]
-        float* prm = reinterpret_cast<float*>(smem + OFF_V);
-        compute_barrier();                                    // every warp is done reading v
-        {
-            const float* srcs[6] = {a.bo, a.ln1w, a.ln1b, a.b2, a.ln2w, a.ln2b};
-            const int ct = warp * 32 + lane;                  // 0..255
-#pragma unroll
-            for (int k = 0; k < 6; ++k)
-                if (ct < 128) prm[k * 128 + ct] = srcs[k][po + ct];
-            prm[768 + ct] = a.b1[po + ct];
-        }
-        compute_barrier();
-        // ---- phase 2: out-projection epilogue: + bias + residual, LayerNorm -> U
-        float* red = reinterpret_cast<float*>(smem + OFF_K);  // [2][2][128][2] partial sums (k, v are dead)
-        {
-            mbar_wait(&bars[B_ACCO], lp);
-            tc_fence_after();
-            const float* bo = prm;
-            float sum = 0.f, sq = 0.f;
-#pragma unroll
-            for (int ci = 0; ci < 2; ++ci) {
-                const int c = (2 * ci + ch) * 32;
-                tmem_ld32(trow + c, v);
-#pragma unroll
-                for (int j = 0; j < 32; j += 4) {
-                    const float4 b4 = *reinterpret_cast<const float4*>(bo + c + j);
-                    const float t0 = v[j] + b4.x + u_keep[ci][j], t1 = v[j + 1] + b4.y + u_keep[ci][j + 1];
-                    const float t2 = v[j + 2] + b4.z + u_keep[ci][j + 2], t3 = v[j + 3] + b4.w + u_keep[ci][j + 3];
-                    u_keep[ci][j] = t0; u_keep[ci][j + 1] = t1; u_keep[ci][j + 2] = t2; u_keep[ci][j + 3] = t3;
-                    sum += (t0 + t1) + (t2 + t3);
-                    sq += (t0 * t0 + t1 * t1) + (t2 * t2 + t3 * t3);
-                }
-            }
-            tc_fence_before();
-            red[(ch * 128 + row) * 2] = sum;
-            red[(ch * 128 + row) * 2 + 1] = sq;
-            compute_barrier();
-            sum += red[((1 - ch) * 128 + row) * 2];
-            sq += red[((1 - ch) * 128 + row) * 2 + 1];
-            const float mean = sum * (1.f / 128.f);
-            const float rstd = rsqrtf(fmaxf(sq * (1.f / 128.f) - mean * mean, 0.f) + 1e-5f);
-            const float* lw = prm + 128;
-            const float* lb = prm + 256;
-#pragma unroll
-            for (int ci = 0; ci < 2; ++ci) {
-                const int c = (2 * ci + ch) * 32;
-#pragma unroll
-                for (int j = 0; j < 32; j += 8) {
-                    float r[8];
-#pragma unroll
-                    for (int e = 0; e < 8; ++e) {
-                        r[e] = (u_keep[ci][j + e] - mean) * rstd * lw[c + j + e] + lb[c + j + e];
-                        u_keep[ci][j + e] = r[e];
-                    }
-                    uint4 pk;
-                    pk.x = pack2(r[0], r[1]); pk.y = pack2(r[2], r[3]); pk.z = pack2(r[4], r[5]); pk.w = pack2(r[6], r[7]);
-                    *reinterpret_cast<uint4*>(smem + OFF_XB + op_chunk(row, (c + j) >> 3, 128)) = pk;
-                }
-            }
-            fence_async_smem();
-            warp_arrive(&bars[B_UREADY], lane);
-        }
-
-        // ---- phase 3: FFN-1 epilogue: + bias, ReLU -> BF16 operand (over the dead att tile)
-        {
-            mbar_wait(&bars[B_ACCF1], lp);
-            tc_fence_after();
-            const float* b1 = prm + 768;
-#pragma unroll
-            for (int ci = 0; ci < 4; ++ci) {
-                const int c = (2 * ci + ch) * 32;
-                tmem_ld32(trow + 256 + c, v);
-#pragma unroll
-                for (int j = 0; j < 32; j += 8) {
-                    float r[8];
-#pragma unroll
-                    for (int e = 0; e < 8; ++e) r[e] = fmaxf(v[j + e] + b1[c + j + e], 0.f);
-                    uint4 pk;
-                    pk.x = pack2(r[0], r[1]); pk.y = pack2(r[2], r[3]); pk.z = pack2(r[4], r[5]); pk.w = pack2(r[6], r[7]);
-                    *reinterpret_cast<uint4*>(smem + OFF_ATT + op_chunk(row, (c + j) >> 3, 256)) = pk;
-                }
-            }
-            tc_fence_before();
-            fence_async_smem();
-            warp_arrive(&bars[B_FREADY], lane);
-        }
-
-        // ---- phase 4: FFN-2 epilogue: + bias + U, LayerNorm -> Y (coalesced through shared)
-        {
-            mbar_wait(&bars[B_ACCF2], lp);
-            tc_fence_after();
-            const float* b2 = prm + 384;
-            float* red2 = red + 512;
-            float sum = 0.f, sq = 0.f;
-#pragma unroll
-            for (int ci = 0; ci < 2; ++ci) {
-                const int c = (2 * ci + ch) * 32;
-                tmem_ld32(trow + c, v);
-#pragma unroll
-                for (int j = 0; j < 32; ++j) {
-                    const float t0 = v[j] + b2[c + j] + u_keep[ci][j];
-                    u_keep[ci][j] = t0;
-                    sum += t0;
-                    sq += t0 * t0;
-                }
-            }
-            tc_fence_before();
-            red2[(ch * 128 + row) * 2] = sum;
-            red2[(ch * 128 + row) * 2 + 1] = sq;
-            compute_barrier();
-            sum += red2[((1 - ch) * 128 + row) * 2];
-            sq += red2[((1 - ch) * 128 + row) * 2 + 1];
-            const float mean = sum * (1.f / 128.f);
-            const float rstd = rsqrtf(fmaxf(sq * (1.f / 128.f) - mean * mean, 0.f) + 1e-5f);
-            const float* lw = prm + 512;
-            const float* lb = prm + 640;
-            const bool more = li + 1 < a.n_layers;
-            if (more) {
-                // Y is the next layer's operand (BF16, over X in shared memory) and residual (FP32, parked in the scratch
-                // slot by the thread that will read it back, lane-major).  Operand first: the driver starts the next
-                // layer's projections on B_XREADY while the rows are being parked.  (No CTA barrier is needed for prm / red:
-                // nobody gets past the next B_ACCQ0 before every warp has arrived here.)
-#pragma unroll
-                for (int ci = 0; ci < 2; ++ci) {
-                    const int c = (2 * ci + ch) * 32;
-#pragma unroll
-                    for (int j = 0; j < 32; ++j) u_keep[ci][j] = (u_keep[ci][j] - mean) * rstd * lw[c + j] + lb[c + j];
-#pragma unroll
-                    for (int j = 0; j < 32; j += 8) {
-                        uint4 pk;
-                        pk.x = pack2(u_keep[ci][j], u_keep[ci][j + 1]); pk.y = pack2(u_keep[ci][j + 2], u_keep[ci][j + 3]);
-                        pk.z = pack2(u_keep[ci][j + 4], u_keep[ci][j + 5]); pk.w = pack2(u_keep[ci][j + 6], u_keep[ci][j + 7]);
-                        *reinterpret_cast<uint4*>(smem + OFF_XB + op_chunk(row, (c + j) >> 3, 128)) = pk;
-                    }
-                }
-                fence_async_smem();
-                warp_arrive(&bars[B_XREADY], lane);
-                float4* park = reinterpret_cast<float4*>(a.y_mid + z * a.y_mid_z + (li & 1) * a.y_l) + (long long)tile * 4096 + row;
-#pragma unroll
-                for (int ci = 0; ci < 2; ++ci)
-#pragma unroll
-                    for (int j = 0; j < 32; j += 4)
-                        __stcg(park + ((ch * 2 + ci) * 8 + (j >> 2)) * 128,
-                               make_float4(u_keep[ci][j], u_keep[ci][j + 1], u_keep[ci][j + 2], u_keep[ci][j + 3]));
-            } else {
-                // last layer: Y row-major to the caller, coalesced through a shared-memory transpose
-                float* Y = a.y + z * a.y_z;
-                float* stage = reinterpret_cast<float*>(smem + OFF_ATT) + warp * (32 * 33);   // FFN-2 MMAs are complete
-#pragma unroll
-                for (int ci = 0; ci < 2; ++ci) {
-                    const int c = (2 * ci + ch) * 32;
-#pragma unroll
-                    for (int j = 0; j < 32; ++j)
-                        stage[lane * 33 + j] = (u_keep[ci][j] - mean) * rstd * lw[c + j] + lb[c + j];
-                    __syncwarp();
-                    const int cq = (lane & 7) * 4;
-#pragma unroll
-                    for (int it = 0; it < 8; ++it) {
-                        const int r = it * 4 + (lane >> 3);
-                        const float* sp = stage + r * 33 + cq;
-                        const int trw = lq * 32 + r;
-                        if (trw < rows_valid)
-                            *reinterpret_cast<float4*>(Y + (row0 + trw) * 128 + c + cq) = make_float4(sp[0], sp[1], sp[2], sp[3]);
-                    }
-                    __syncwarp();
-                }
-            }
-        }
-        }   // layers
-    }
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 0) tmem_dealloc(tmem, 512);
-}
-
-
 // ------------------------------------------------------------------------------------------------
-// Tensor-pipe attention variant (the default): 16 compute warps + 1 driver warp.
-//
-// TMEM lane quarter lq = warp & 3 (hardware rule); role = warp >> 2:
+// Compute warps.  TMEM lane quarter lq = warp & 3 (hardware rule); role = warp >> 2:
 //   role 0, 1  "score" warps of the two heads in flight (ch = role & 1): q -> BF16 A operand in TMEM, k -> shared,
 //              issue S = Q K^T, softmax on the gene's own S keys, P -> BF16 A operand in TMEM, issue O = P V;
 //   role 2, 3  "value" warps of the same two heads: v -> shared (MN-major), sigmoid(gate) kept in registers,
@@ -622,7 +159,7 @@ __global__ void __launch_bounds__(RF_THREADS, 1) reg_layer_cc_kernel(const RegFu
 // In the epilogue phases (out-projection + LayerNorm, FFN-1, FFN-2 + LayerNorm) role = column quarter: every row is
 // served by four threads, 32 columns each (64 of the 256 FFN-1 columns), and FFN-1 / FFN-2 are chained per half of the
 // hidden width, so that one half's bias + ReLU epilogue runs under the other half's MMAs.
-constexpr int RF2_THREADS = 640;            // 16 compute warps + dense-MMA issuer + weight loader + 2 attention issuers
+constexpr int RF_THREADS = 640;            // 16 compute warps + dense-MMA issuer + weight loader + 2 attention issuers
 enum { C_FULL0 = 0, C_FREE0 = 3, C_XREADY = 6, C_ATTREADY, C_UREADY, C_FREADY0, C_FREADY1, C_ACCQ, C_ACCVG, C_ACCO, C_ACCF1A,
        C_ACCF1B, C_ACCF2, C_OFREE, C_SR0, C_OR0 = C_SR0 + 2, C_QKS0 = C_OR0 + 2, C_PST0 = C_QKS0 + 2,
        C_VR0 = C_PST0 + 2, C_COUNT = C_VR0 + 2 };
@@ -722,7 +259,7 @@ __device__ __noinline__ void score_rows_call(uint64_t* bars, uint32_t trow, int 
 }
 
 template <int SMAX, bool TRACE, bool PLAN>
-__global__ void __launch_bounds__(RF2_THREADS, 1) reg_layer_fused_kernel(const RegFusedArgs a) {
+__global__ void __launch_bounds__(RF_THREADS, 1) reg_layer_fused_kernel(const RegFusedArgs a) {
     extern __shared__ __align__(1024) uint8_t smem[];
     uint64_t* bars = reinterpret_cast<uint64_t*>(smem + OFF_CTL);
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + C_COUNT);
@@ -1324,24 +861,16 @@ int pack_reg_stream(const RegStreamArgs& a, int n_res, cudaStream_t st) {
 static long long* g_trace = nullptr;
 void reg_fused_set_trace(long long* buf) { g_trace = buf; }
 
-bool reg_fused_tensor_attention() {
-    static int tc = -1;
-    if (tc < 0) { const char* e = getenv("CHROMO_REG_TC"); tc = (e && e[0] == '0') ? 0 : 1; }
-    return tc != 0;
-}
-
 int launch_reg_layer_fused(const RegFusedArgs& a, int n_res, cudaStream_t st) {
     static bool configured = false;
     if (!configured) {
-        cudaError_t e1 = cudaFuncSetAttribute(reg_layer_cc_kernel<9>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
-        cudaError_t e2 = cudaFuncSetAttribute(reg_layer_cc_kernel<17>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
-        cudaError_t e3 = cudaFuncSetAttribute(reg_layer_fused_kernel<9, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
-        cudaError_t e4 = cudaFuncSetAttribute(reg_layer_fused_kernel<17, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
-        cudaError_t e5 = cudaFuncSetAttribute(reg_layer_fused_kernel<9, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
-        cudaError_t e6 = cudaFuncSetAttribute(reg_layer_fused_kernel<17, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
-        cudaError_t e7 = cudaFuncSetAttribute(reg_layer_fused_kernel<9, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
-        cudaError_t e8 = cudaFuncSetAttribute(reg_layer_fused_kernel<17, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
-        for (cudaError_t e : {e1, e2, e3, e4, e5, e6, e7, e8})
+        cudaError_t e1 = cudaFuncSetAttribute(reg_layer_fused_kernel<9, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
+        cudaError_t e2 = cudaFuncSetAttribute(reg_layer_fused_kernel<17, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
+        cudaError_t e3 = cudaFuncSetAttribute(reg_layer_fused_kernel<9, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
+        cudaError_t e4 = cudaFuncSetAttribute(reg_layer_fused_kernel<17, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
+        cudaError_t e5 = cudaFuncSetAttribute(reg_layer_fused_kernel<9, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
+        cudaError_t e6 = cudaFuncSetAttribute(reg_layer_fused_kernel<17, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)RF_SMEM);
+        for (cudaError_t e : {e1, e2, e3, e4, e5, e6})
             if (e != cudaSuccess) { set_error("reg_fused smem attribute: %s", cudaGetErrorString(e)); return CHROMO_ECUDA; }
         configured = true;
     }
@@ -1354,24 +883,18 @@ int launch_reg_layer_fused(const RegFusedArgs& a, int n_res, cudaStream_t st) {
             int dev = 0;
             if (cudaGetDevice(&dev) != cudaSuccess || cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess || sms < 1) sms = 1 << 30;
         }
-        at.park_by_sm = (a.n_layers > 1 && a.n_tiles >= sms && !getenv("CHROMO_REG_PARK_BY_TILE")) ? 1 : 0;   // (%smid < SM count)
+        at.park_by_sm = (a.n_layers > 1 && a.n_tiles >= sms) ? 1 : 0;   // (%smid < SM count)
     }
-    // Attention on the tensor pipe (block-diagonal Q K^T / P V with Q and P rounded to BF16, as in every flash-attention
-    // kernel) is the default (profiles/r01_precision.md).  CHROMO_REG_TC=0 selects the CUDA-core variant (FP32 q and
-    // probabilities, one layer per launch).
-    const int tc = reg_fused_tensor_attention() ? 1 : 0;
-    if (a.n_layers < 1 || (a.n_layers > 1 && !tc)) { set_error("reg_layer_fused: multi-layer launches need the tensor-pipe attention"); return CHROMO_EINVAL; }
+    if (a.n_layers < 1) { set_error("reg_layer_fused: n_layers must be >= 1"); return CHROMO_EINVAL; }
     const bool plan = a.plan_tiles != nullptr;
-    if (plan && !(tc && (a.S == 9 || a.S == 17) && a.plan_rows)) { set_error("reg_layer_fused: ragged plan without the tensor-pipe attention"); return CHROMO_EINVAL; }
+    if (plan && !a.plan_rows) { set_error("reg_layer_fused: ragged plan without its row map"); return CHROMO_EINVAL; }
     if (plan) at.trace = nullptr;
-    if (a.S == 9 && plan) reg_layer_fused_kernel<9, false, true><<<grid, RF2_THREADS, RF_SMEM, st>>>(at);
-    else if (a.S == 17 && plan) reg_layer_fused_kernel<17, false, true><<<grid, RF2_THREADS, RF_SMEM, st>>>(at);
-    else if (a.S == 9 && tc && at.trace) reg_layer_fused_kernel<9, true, false><<<grid, RF2_THREADS, RF_SMEM, st>>>(at);
-    else if (a.S == 17 && tc && at.trace) reg_layer_fused_kernel<17, true, false><<<grid, RF2_THREADS, RF_SMEM, st>>>(at);
-    else if (a.S == 9 && tc) reg_layer_fused_kernel<9, false, false><<<grid, RF2_THREADS, RF_SMEM, st>>>(at);
-    else if (a.S == 9) reg_layer_cc_kernel<9><<<grid, RF_THREADS, RF_SMEM, st>>>(a);
-    else if (a.S == 17 && tc) reg_layer_fused_kernel<17, false, false><<<grid, RF2_THREADS, RF_SMEM, st>>>(at);
-    else if (a.S == 17) reg_layer_cc_kernel<17><<<grid, RF_THREADS, RF_SMEM, st>>>(a);
+    if (a.S == 9 && plan) reg_layer_fused_kernel<9, false, true><<<grid, RF_THREADS, RF_SMEM, st>>>(at);
+    else if (a.S == 17 && plan) reg_layer_fused_kernel<17, false, true><<<grid, RF_THREADS, RF_SMEM, st>>>(at);
+    else if (a.S == 9 && at.trace) reg_layer_fused_kernel<9, true, false><<<grid, RF_THREADS, RF_SMEM, st>>>(at);
+    else if (a.S == 17 && at.trace) reg_layer_fused_kernel<17, true, false><<<grid, RF_THREADS, RF_SMEM, st>>>(at);
+    else if (a.S == 9) reg_layer_fused_kernel<9, false, false><<<grid, RF_THREADS, RF_SMEM, st>>>(at);
+    else if (a.S == 17) reg_layer_fused_kernel<17, false, false><<<grid, RF_THREADS, RF_SMEM, st>>>(at);
     else { set_error("reg_layer_fused: tokens per gene must be 9 or 17"); return CHROMO_EINVAL; }
     CHROMO_CHECK_LAUNCH("reg_layer_fused");
     return CHROMO_OK;

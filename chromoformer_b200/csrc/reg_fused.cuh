@@ -21,7 +21,7 @@ struct RegFusedArgs {
     long long* trace = nullptr;             // profiling hook (chromo_debug_trace): CTA (0,0) logs (event << 48 | clock64) here
     int y_head_only = 0;                    // 1 (with a plan): only token 0 of every gene is stored by the last layer (what fc_head consumes, net.py:377)
     int park_by_sm = 0;                     // 1: a CTA parks its rows in the block of its SM (set by the launcher when the slots allow)
-    // ragged plan (ragged.cu; tensor-pipe attention only): tile t holds plan_tiles[t].y genes (0: the tile is unused - the
+    // ragged plan (ragged.cu): tile t holds plan_tiles[t].y genes (0: the tile is unused - the
     // grid is an upper bound) with their first plan_tiles[t].z tokens each (the others are masked for every token that
     // reaches the head); its rows are gathered from / scattered to rows plan_rows[t][0..128) of the [B*S, 128] layout
     const int4* plan_tiles = nullptr; const int* plan_rows = nullptr;
@@ -61,7 +61,6 @@ int launch_row_tail_fused(const RowTailArgs& a, int n_res, cudaStream_t st);
 long long reg_stream_elems_per_layer();
 int pack_reg_stream(const RegStreamArgs& a, int n_res, cudaStream_t st);
 void reg_fused_set_trace(long long* buf);
-bool reg_fused_tensor_attention();      // CHROMO_REG_TC != 0: attention on the tensor pipe; allows multi-layer launches
 int launch_reg_layer_fused(const RegFusedArgs& a, int n_res, cudaStream_t st);
 
 }  // namespace chromo

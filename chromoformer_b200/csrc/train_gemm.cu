@@ -561,7 +561,7 @@ int tc_gemm_launch(const TcGemm& in, int nz, cudaStream_t st) {
     // with FP32 atomics: to the output itself when the call accumulates in place, to a zeroed output otherwise.
     a.ksplit = 1;
     const int chunks = (a.Kc + TG_KCH - 1) / TG_KCH;
-    if (chunks >= 4 && (a.epi & ~TC_RES) == 0 && a.c_div == 1 && a.c_mul == 1 && a.c_add == 0 && !getenv("CHROMO_TG_NO_KSPLIT")) {
+    if (chunks >= 4 && (a.epi & ~TC_RES) == 0 && a.c_div == 1 && a.c_mul == 1 && a.c_add == 0) {
         const bool in_place = (a.epi & TC_RES) && a.res == a.C && a.ldres == a.ldc && a.res_z == a.c_z && a.res_div == 1;
         const int ctas = (a.N / a.NT) * ((a.M + 127) / 128) * nz;
         int ks = 1;
@@ -580,12 +580,11 @@ int tc_gemm_launch(const TcGemm& in, int nz, cudaStream_t st) {
     }
     dim3 grid(a.N / a.NT, (a.M + 127) / 128, nz * a.ksplit);
     {
-        static const bool no_pdl = getenv("CHROMO_NO_PDL") != nullptr;
         cudaLaunchConfig_t cfg = {};
         cfg.gridDim = grid; cfg.blockDim = dim3(TG_THREADS); cfg.dynamicSmemBytes = smem; cfg.stream = st;
         cudaLaunchAttribute attr[1];
         attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        attr[0].val.programmaticStreamSerializationAllowed = no_pdl ? 0 : 1;
+        attr[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
         cfg.attrs = attr; cfg.numAttrs = 1;
         long long* tb = g_tg_trace ? g_tg_trace + 2048 : nullptr;
         cudaError_t e = cudaLaunchKernelEx(&cfg, tc_gemm_kernel, a, tb);

@@ -15,7 +15,6 @@
 // from two resident CTAs per SM (A/B staging of one under the MMA/epilogue of the other).
 #include <algorithm>
 #include <cuda_bf16.h>
-#include <stdlib.h>
 
 #include "common.cuh"
 #include "gemm_simt.cuh"
@@ -70,7 +69,6 @@ struct UmmaArgs {
     const __nv_bfloat16* Bp;      // packed weights (same z strides as g.B)
     int NT;                       // N tile (multiple of 16, <= 256, divides N)
     int tmem_cols;                // power of two >= max(32, NT)
-    int direct_store;             // debug/tuning: skip the shared-memory transpose in the epilogue
 };
 
 // Write one 32x32 FP32 tile held as (lane = row, v[0..31] = columns) to C so that every store
@@ -318,7 +316,7 @@ __global__ void __launch_bounds__(UTHREADS) umma_linear_kernel(const UmmaArgs a)
                 }
             } else {
                 float* C = g.C + z1 * g.sC1 + z2 * g.sC2;
-                if (g.accumulate || a.direct_store) {
+                if (g.accumulate) {
                     if (ok) {
                         float* out = C + crow * g.ldc + n0 + c;
 #pragma unroll
@@ -540,20 +538,14 @@ bool umma_supported(const GemmArgs& g) {
 
 // the persistent query GEMM (qk_tiles_kernel) takes this call: the only GEMM that honours a ragged plan
 bool umma_qk_persistent(const GemmArgs& g) {
-    return g.c_sqa_tiles && g.K == 128 && g.N == 256 && g.zdiv == 1 && (g.M + UM - 1) / UM >= 8 && !getenv("CHROMO_QK_ONE_TILE");
+    return g.c_sqa_tiles && g.K == 128 && g.N == 256 && g.zdiv == 1 && (g.M + UM - 1) / UM >= 8;
 }
 
 int umma_launch(const GemmArgs& g, const __nv_bfloat16* Bp, int nz, cudaStream_t st) {
-    static int direct = -1;
-    if (direct < 0) {
-        const char* e = getenv("CHROMO_UMMA_DIRECT_STORE");
-        direct = (e && e[0] == '1') ? 1 : 0;
-    }
     UmmaArgs a;
     a.g = g; a.Bp = Bp; a.NT = choose_nt(g.N);
     a.tmem_cols = 32;
     while (a.tmem_cols < a.NT) a.tmem_cols *= 2;
-    a.direct_store = direct;
     const size_t smem = umma_smem_bytes(a.NT, g.K);
     static size_t configured = 0;
     if (smem > configured) {

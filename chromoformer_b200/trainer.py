@@ -11,7 +11,6 @@ run, so their all-reduce is issued there and overlaps the Pairwise / Embedding p
 (``CHROMO_F_BWD_REST``); only the small second bucket is exposed.
 """
 import ctypes
-import os
 
 import torch
 import torch.distributed as dist
@@ -59,8 +58,7 @@ class TrainStep:
                                 if off < model.n_active and model._lib_name(name).startswith(("regulation.", "fc_head.")))
         # measured (B200, batch 64 per rank): 2 ranks 1.47 ms single bucket / 1.49 ms two buckets, 4 ranks 1.52 / 1.49: the
         # second graph launch and NCCL call cost what the overlap saves until the all-reduce takes ~0.1 ms
-        ov = os.environ.get("CHROMO_DP_OVERLAP")
-        self.overlap = self.world > 1 and (ov == "1" if ov is not None else self.world > 2)
+        self.overlap = self.world > 2
 
     # ---- forward + loss + backward into self.grad (everything a CUDA graph may hold) -------------------------
     def _chain(self, io, target, logits, dlogits, part=0):

@@ -2,11 +2,9 @@
 
 The plan only uses what the masks themselves guarantee (data.py:156-203: centred valid spans, dummy slots behind a
 block-form interaction mask), so its results must agree with the CPU oracle - which computes every slot and every bin as
-the reference does - within the BF16 tolerance, and with the same kernels run without the plan (CHROMO_NO_RAGGED=1) to
-rounding noise.  The adversarial cases are the ones where an elimination would be WRONG if the plan trusted the data
+the reference does - within the BF16 tolerance, and with the same kernels run without the plan (the CHROMO_F_DENSE hint)
+to rounding noise.  The adversarial cases are the ones where an elimination would be WRONG if the plan trusted the data
 layout instead of the masks."""
-import os
-
 import pytest
 import torch
 
@@ -32,18 +30,11 @@ def _oracle_logits(sd, batch, idx):
         return oracle.chromoformer_forward(sd, *synthetic.forward_args(part))
 
 
-def _run(model, batch, ragged, hint=False):
-    if ragged:
-        os.environ.pop("CHROMO_NO_RAGGED", None)
-    else:
-        os.environ["CHROMO_NO_RAGGED"] = "1"
-    try:
-        eng = InferenceEngine(model, chunk=batch["interaction_freq"].size(0))
-        dev = eng.to_device(batch)
-        dev["dense"] = hint            # (to_device sets the CHROMO_F_DENSE hint for batches without padding: plan not built)
-        return eng.predict_device(dev).cpu()
-    finally:
-        os.environ.pop("CHROMO_NO_RAGGED", None)
+def _run(model, batch, ragged):
+    eng = InferenceEngine(model, chunk=batch["interaction_freq"].size(0))
+    dev = eng.to_device(batch)
+    dev["dense"] = not ragged          # the CHROMO_F_DENSE hint: the plan is not built
+    return eng.predict_device(dev).cpu()
 
 
 def test_ragged_batch_with_and_without_plan():
@@ -70,21 +61,20 @@ def test_ragged_batch_with_and_without_plan():
     assert torch.equal(_run(model, full, True), _run(model, sub, True))
 
 
-def test_dense_batch_keeps_its_numbers():
+def test_dense_batch_same_with_and_without_plan():
     """All slots live, all spans full: the stable sort keeps the order and every window is the whole table - bit-identical
-    to the run without the plan."""
+    to the run without the plan, so the hint never changes the results of a batch it is derived for."""
     n = 256
     model = _mk(seed=3)
     batch = synthetic.make_batch(n, ragged=False, seed=2)
     model.cuda().eval()
     model.precision = "bf16"
     assert torch.equal(_run(model, batch, True), _run(model, batch, False))
-    # the engine recognises such a batch on the host and passes the hint; the hint itself never changes results
+    # the engine recognises such a batch on the host and passes the hint
     eng = InferenceEngine(model, chunk=n)
     assert eng.to_device(batch)["dense"] is True
     rag = synthetic.make_batch(n, ragged=True, seed=2)
     assert eng.to_device(rag)["dense"] is False
-    assert torch.equal(_run(model, rag, True, hint=True), _run(model, rag, False))
 
 
 def test_masks_decide_not_the_layout():

@@ -18,5 +18,3 @@ for shift in (1, 3, 7, 14, 64, 100):
     got = eng.predict_device(sub).cpu()
     d = (got - base[shift:]).abs()
     print(f"shift {shift}: max {d.max().item():.3e}, genes differing {(d.max(1).values > 0).sum().item()} / {d.size(0)}")
-for env in ("CHROMO_NO_SQA_FUSED", "CHROMO_REG_TC"):
-    pass

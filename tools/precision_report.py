@@ -16,8 +16,6 @@ from chromoformer_b200 import ChromoformerClassifier, synthetic  # noqa: E402
 
 VARIANTS = [
     ("this library, bf16 (default kernels)", {}),
-    ("bf16, Regulation attention on CUDA cores (CHROMO_REG_TC=0)", {"CHROMO_REG_TC": "0"}),
-    ("bf16, Regulation attention on the tensor pipe (CHROMO_REG_TC=1)", {"CHROMO_REG_TC": "1"}),
     ("bf16, unfused single-query attention (CHROMO_NO_SQA_FUSED=1)", {"CHROMO_NO_SQA_FUSED": "1"}),
 ]
 

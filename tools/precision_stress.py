@@ -88,7 +88,6 @@ def main():
         for tag, env in (("stress, head GEMMs in FP32 (CHROMO_HEAD_FP32)", {"CHROMO_HEAD_FP32": "1"}),
                          ("stress, Regulation stack in FP32 (CHROMO_REG_FP32)", {"CHROMO_REG_FP32": "1"}),
                          ("stress, Regulation + head in FP32", {"CHROMO_REG_FP32": "1", "CHROMO_HEAD_FP32": "1"}),
-                         ("stress, Regulation attention on CUDA cores (CHROMO_REG_TC=0)", {"CHROMO_REG_TC": "0"}),
                          ("stress, unfused single-query attention (CHROMO_NO_SQA_FUSED)", {"CHROMO_NO_SQA_FUSED": "1"})):
             e = dict(os.environ, CHROMO_PRECISION_CHILD=tag, **env)
             out = subprocess.run([sys.executable, os.path.abspath(__file__)], env=e, capture_output=True, text=True)

@@ -1,5 +1,5 @@
 """genes/s of the device-resident 18,955-gene sweep (BF16), dense and ragged genes, with and without the ragged plan
-(csrc/ragged.cu; CHROMO_NO_RAGGED=1 switches it off)."""
+(csrc/ragged.cu; the CHROMO_F_DENSE hint switches it off)."""
 import os
 import sys
 
@@ -20,11 +20,7 @@ for name, ragged in (("dense", False), ("ragged", True)):
     out = torch.empty(N, 2, device="cuda")
     outs = {}
     for plan in (True, False):
-        res["dense"] = False                     # (no CHROMO_F_DENSE hint: the plan is built whenever it is switched on)
-        if plan:
-            os.environ.pop("CHROMO_NO_RAGGED", None)
-        else:
-            os.environ["CHROMO_NO_RAGGED"] = "1"
+        res["dense"] = not plan                  # (CHROMO_F_DENSE hint only for the plan-off leg: the plan is built otherwise)
         for _ in range(3):
             eng.predict_device(res, out)
         torch.cuda.synchronize()
@@ -42,4 +38,3 @@ for name, ragged in (("dense", False), ("ragged", True)):
     print(f"{name:6s} max |dlogit| plan on/off = {(outs[True] - outs[False]).abs().max().item():.2e}")
     del res
     model._ws_cache.clear()
-os.environ.pop("CHROMO_NO_RAGGED", None)
