@@ -56,6 +56,14 @@ class Batch(Structure):
     ]
 
 
+class InputGrads(Structure):
+    """``chromo_input_grads_t`` — where chromo_backward_inputs writes the feature gradients (NULL: not wanted)."""
+    _fields_ = [
+        ("x_p", c_void_p * MAX_RES),
+        ("x_pcre", c_void_p * MAX_RES),
+    ]
+
+
 class Region(Structure):
     """``chromo_region_t``"""
     _fields_ = [("offset", c_int64), ("length", c_int32), ("start", c_int32), ("width", c_int32),
@@ -84,6 +92,8 @@ EXPORTS = {
     "chromo_debug_trace": (c_int32, [c_void_p]),
     "chromo_backward": (c_int32, [POINTER(Config), c_void_p, POINTER(Batch), c_void_p, c_void_p, c_void_p,
                                   c_int64, c_int32, c_void_p]),
+    "chromo_backward_inputs": (c_int32, [POINTER(Config), c_void_p, POINTER(Batch), c_void_p, c_void_p,
+                                         POINTER(InputGrads), c_void_p, c_int64, c_int32, c_void_p]),
     "chromo_matmul": (c_int32, [c_void_p, c_int64, c_int32, c_void_p, c_int64, c_int32, c_void_p, c_int64, c_int32, c_int32,
                                 c_int32, c_int32, c_int32, c_void_p]),
     "chromo_mse_loss": (c_int32, [c_void_p, c_void_p, c_int32, c_float, c_void_p, c_void_p, c_void_p]),

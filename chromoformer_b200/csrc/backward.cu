@@ -69,7 +69,7 @@ __global__ void __launch_bounds__(256) ln_bwd_kernel(LnBwdArgs a) {
 #pragma unroll
     for (int k = 0; k < 4; ++k) { s_dg[warp][lane * 4 + k] = dg[k]; s_db[warp][lane * 4 + k] = db[k]; }
     __syncthreads();
-    if (threadIdx.x < 128) {
+    if (threadIdx.x < 128 && a.dgamma) {     // (no dgamma: data gradient only, chromo_backward_inputs without grads)
         float x = 0.f, y = 0.f;
 #pragma unroll
         for (int w = 0; w < 8; ++w) { x += s_dg[w][threadIdx.x]; y += s_db[w][threadIdx.x]; }
@@ -211,7 +211,7 @@ __global__ void __launch_bounds__(256) reg_attention_bwd_kernel(RegAttnBwdArgs a
             dproj[(long long)j * 4 * dm + 2 * dm] = dv[j];
         }
     }
-    if (lane == 0) atomicAdd(a.dgamma_f + z * a.dgamma_z + h, dgam);
+    if (lane == 0 && a.dgamma_f) atomicAdd(a.dgamma_f + z * a.dgamma_z + h, dgam);
 }
 
 // The same backward with one CTA per gene (counterpart of reg_attention_gene_kernel): the gene's rows of q | k | v | gate
@@ -309,7 +309,7 @@ __global__ void __launch_bounds__(SMAX * 32) reg_attention_gene_bwd_kernel(RegAt
         if (sub == 0) sm_gam[item] = dgam;
     }
     __syncthreads();
-    if (tid < H) {      // one atomic per (gene, head), summed in a fixed order
+    if (tid < H && a.dgamma_f) {      // one atomic per (gene, head), summed in a fixed order
         float t = 0.f;
         for (int q = 0; q < S; ++q) t += sm_gam[tid * S + q];
         atomicAdd(a.dgamma_f + z * a.dgamma_z + tid, t);
@@ -404,6 +404,79 @@ __global__ void __launch_bounds__(256) attn_rows_bwd_kernel(AttnRowsBwdArgs a) {
     }
 }
 
+// Gradient with respect to the raw features of single-query attention regions (chromo_backward_inputs).  Keys and values
+// are h_j = W_in x_j + PE_j, so with dS as attn_rows_bwd_kernel leaves it (the gradient of the pre-scale score, zero on
+// masked bins) and dCbar / qk of the region's H rows:
+//     dx[j, :] (=|+=) sum_h P[h, j] a_h + dS[h, j] u_h,   a_h = W_in^T dCbar_h,  u_h = W_in^T qk_h
+// plus W_in^T dhc at the centre bin n/2 when `dhc` is set (the promoter's query / residual input).  One warp per region;
+// every element of the region is written, so the output needs no memset and no atomics.
+struct InputGradArgs {
+    int regions, H, n, F, D;
+    const float* P;       // [regions * H, n] probabilities
+    const float* dS;      // [regions * H, n]
+    const float* dcbar;   // [regions * H, D]
+    const float* qk;      // [regions * H, D]
+    const float* w_in;    // [D, F]
+    const float* dhc;     // [regions, D] or nullptr
+    float* dx;            // [regions, n, F]
+    int accumulate;
+};
+__global__ void __launch_bounds__(256) input_grad_rows_kernel(InputGradArgs a) {
+    CHROMO_PDL_ENTER();
+    __shared__ float w_s[128 * 8];
+    __shared__ float au_s[8][2 * 8 * 8 + 8];      // per warp: a[h][f], u[h][f], centre term [f]
+    for (int i = threadIdx.x; i < a.D * a.F; i += blockDim.x) w_s[i] = a.w_in[i];
+    __syncthreads();
+    const int wib = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    const long long region = (long long)blockIdx.x * 8 + wib;
+    if (region >= a.regions) return;
+    const int n = a.n, F = a.F, D = a.D, H = a.H;
+    float* au = au_s[wib];
+    // W_in^T v for the 2H + 1 vectors v of the region (lanes over d, then a butterfly per feature)
+    for (int v = 0; v < 2 * H + 1; ++v) {
+        const float* src = v < H ? a.dcbar + (region * H + v) * D
+                         : v < 2 * H ? a.qk + (region * H + v - H) * D
+                         : a.dhc ? a.dhc + region * D : nullptr;
+        float s[8];
+#pragma unroll
+        for (int f = 0; f < 8; ++f) s[f] = 0.f;
+        if (src) {
+            for (int d = lane; d < D; d += 32) {
+                const float c = src[d];
+                const float* w = w_s + d * F;
+#pragma unroll
+                for (int f = 0; f < 8; ++f)
+                    if (f < F) s[f] = fmaf(w[f], c, s[f]);
+            }
+#pragma unroll
+            for (int f = 0; f < 8; ++f)
+#pragma unroll
+                for (int o = 16; o > 0; o >>= 1) s[f] += __shfl_xor_sync(0xffffffffu, s[f], o);
+        }
+        const int base = v < H ? v * 8 : v < 2 * H ? 64 + (v - H) * 8 : 128;
+        if (lane == 0) {
+#pragma unroll
+            for (int f = 0; f < 8; ++f) au[base + f] = s[f];
+        }
+    }
+    __syncwarp();
+    const float* P = a.P + region * H * n;
+    const float* dS = a.dS + region * H * n;
+    float* dx = a.dx + region * n * F;
+    const int c = n / 2;
+    for (int e = lane; e < n * F; e += 32) {       // consecutive lanes, consecutive elements
+        const int j = e / F, f = e - j * F;
+        float g = 0.f;
+        for (int h = 0; h < H; ++h) {
+            g = fmaf(P[h * n + j], au[h * 8 + f], g);
+            g = fmaf(dS[h * n + j], au[64 + h * 8 + f], g);
+        }
+        if (j == c) g += au[128 + f];
+        if (a.accumulate) g += dx[e];
+        dx[e] = g;
+    }
+}
+
 // ------------------------------------------------------------ host helpers ---
 namespace {
 
@@ -415,6 +488,7 @@ struct Ctx {
     int NR;
     bool tc = false;            // CHROMO_F_BF16: contractions on the tensor pipe (train_gemm.cu)
     WgradQueue* q = nullptr;    // tc: the deferred weight / bias gradients
+    bool wgrad = true;          // false: data gradients only (chromo_backward_inputs with grads == NULL)
 };
 
 // Split-K factor: the training batch is small (bsz 64 => a few hundred rows), so most gradient
@@ -468,6 +542,7 @@ int bwd_data(const Ctx& c, const float* dY, int ldy, long long dy_z, const float
 // dW += dY^T X          dY [M,N], X [M/x_div rows broadcast, K] (ld ldx), dW [N,K] row-major
 int bwd_weight(const Ctx& c, const float* dY, int ldy, long long dy_z, const float* X, int ldx, int x_div,
                long long x_z, float* dW, int lddw, long long dw_z, int M, int N, int K, int nz) {
+    if (!c.wgrad) return CHROMO_OK;
     if (c.q) {      // both operands MN-major (rows = tokens = the contraction); runs at the end of the pass
         c.q->add_weight(dY, ldy, dy_z, X, ldx, x_div, x_z, dW, lddw, dw_z, M, N, K, nz);
         return CHROMO_OK;
@@ -484,6 +559,7 @@ int bwd_weight(const Ctx& c, const float* dY, int ldy, long long dy_z, const flo
 
 int bwd_bias(const Ctx& c, const float* dY, int ld, long long dy_z, float* db, long long db_z, int M, int N,
              int nz) {
+    if (!c.wgrad) return CHROMO_OK;
     if (c.q) {
         c.q->add_bias(dY, ld, dy_z, db, db_z, M, N, nz);
         return CHROMO_OK;
@@ -497,7 +573,7 @@ int bwd_bias(const Ctx& c, const float* dY, int ld, long long dy_z, float* db, l
 
 int ln_bwd(const Ctx& c, const float* pre, long long pre_z, const float* gin, float* gout, long long g_z,
            const float* gamma, float* dgamma, float* dbeta, long long p_z, int M, int nz) {
-    LnBwdArgs a{M, pre, pre_z, gin, gout, g_z, gamma, dgamma, dbeta, p_z};
+    LnBwdArgs a{M, pre, pre_z, gin, gout, g_z, gamma, c.wgrad ? dgamma : nullptr, dbeta, p_z};
     int blocks = (M + 7) / 8;
     if (blocks > 296) blocks = 296;
     launch_pdl(ln_bwd_kernel, dim3(dim3(blocks, nz)), dim3(256), 0, c.st, a);
@@ -549,7 +625,7 @@ int sqa_bwd(const Ctx& c, const SqaBwd& s) {
         for (int h = 0; h < s.H; ++h)
             CHROMO_TRY(bwd_weight(c1, s.dAv + h * dh, s.dm, 0, s.cbar + (long long)h * D, s.H * D, 1, 0,
                                   s.g_wv + (long long)h * dh * D, D, 0, s.rows, dh, D, 1));
-    } else {
+    } else if (c.wgrad) {   // (the queue exists only with wgrad)
         GemmArgs g = gemm_args();
         g.A = s.dAv; g.lda = s.dm; g.sA2 = dh;
         g.B = s.cbar; g.ldb = s.H * D; g.sB2 = D;
@@ -595,7 +671,7 @@ int sqa_bwd(const Ctx& c, const SqaBwd& s) {
         for (int h = 0; h < s.H; ++h)
             CHROMO_TRY(bwd_weight(c1, s.q + h * dh, s.dm, 0, s.dQK + (long long)h * D, s.H * D, 1, 0,
                                   s.g_wk + (long long)h * dh * D, D, 0, s.rows, dh, D, 1));
-    } else {
+    } else if (c.wgrad) {   // (the queue exists only with wgrad)
         GemmArgs g = gemm_args();
         g.A = s.q; g.lda = s.dm; g.sA2 = dh;
         g.B = s.dQK; g.ldb = s.H * D; g.sB2 = D;
@@ -606,10 +682,24 @@ int sqa_bwd(const Ctx& c, const SqaBwd& s) {
     return CHROMO_OK;
 }
 
+// dx (=|+=) the feature gradient of the regions sqa_bwd(s) has just run for (its P, dS, dCbar, qk and W_in)
+int input_grad(cudaStream_t st, const SqaBwd& s, const float* dhc, float* dx, bool accumulate) {
+    InputGradArgs a;
+    a.regions = s.rows; a.H = s.H; a.n = s.n; a.F = s.F; a.D = s.D;
+    a.P = s.P; a.dS = s.dS; a.dcbar = s.dCbar; a.qk = s.qk; a.w_in = s.w_in; a.dhc = dhc; a.dx = dx;
+    a.accumulate = accumulate ? 1 : 0;
+    launch_pdl(input_grad_rows_kernel, dim3((unsigned)((s.rows + 7) / 8)), dim3(256), 0, st, a);
+    CHROMO_CHECK_LAUNCH("input_grad_rows");
+    return CHROMO_OK;
+}
+
 }  // namespace
 
+// G == nullptr: no parameter gradient (no weight / bias contraction, no LayerNorm or gamma_f reduction); dx: feature
+// gradients to write (nullptr or NULL entries: none) - chromo_backward passes (G, nullptr).
 static int backward_impl(const chromo_config_t* c, const float* P, const chromo_batch_t* in, const float* dlogits,
-                         float* G, float* ws, const WsLayout& w, cudaStream_t st, bool tc, bool part1, bool part2) {
+                         float* G, float* ws, const WsLayout& w, cudaStream_t st, bool tc, bool part1, bool part2,
+                         const chromo_input_grads_t* dx = nullptr) {
     const ParamLayout& L = get_layout(c);
     const int B = w.B, I = w.I, S = w.S, R = w.R, T = w.T, D = w.D, F = c->n_feats, NR = c->n_res;
     const long long RS = w.res_stride;
@@ -617,7 +707,8 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
     const int dmp = c->pw_d_model, Hp = c->pw_heads, dffp = c->pw_d_ff;
     const int dmr = c->reg_d_model, Hr = c->reg_heads, dffr = c->reg_d_ff;
     WgradQueue queue;
-    Ctx cx{st, NR, tc, tc ? &queue : nullptr};
+    const bool wgrad = G != nullptr;
+    Ctx cx{st, NR, tc, tc && wgrad ? &queue : nullptr, wgrad};
     Ctx c1 = cx; c1.NR = 1;
 
     // ---- gradient scratch: one buffer per gradient tensor and layer (see Ctx) -------------------------------------
@@ -693,7 +784,7 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
             a.dproj = dProj; a.dproj_z = GS;
             a.freq = in->freq;
             for (int r = 0; r < NR; ++r) a.imask[r] = in->imask[r];
-            a.dgamma_f = G + ra.gamma_f; a.dgamma_z = L.reg_stride;
+            a.dgamma_f = wgrad ? G + ra.gamma_f : nullptr; a.dgamma_z = L.reg_stride;
             dim3 grid((unsigned)(((long long)B * Hr + 7) / 8), NR);
             if (Hr == 8 && S <= 17) {       // one CTA per gene, rows staged in shared memory
                 const size_t smem = ((size_t)S * (4 * dmr + RAB_PAD) + (size_t)S * dmr + 2 * (size_t)Hr * S * S + Hr * S) * sizeof(float);
@@ -715,7 +806,7 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
         CHROMO_TRY(bwd_data(cx, dProj, 4 * dmr, GS, P + ra.att, L.reg_stride, gcur, D, GS, T, 4 * dmr, D, resid, NR));
         // gcur = dX of this layer = the gradient arriving at the output of layer l-1; gnext is free again
         // this layer's weight gradients start now, on the side stream and on 64 SMs, under the next layer's chain
-        if (tc) {
+        if (cx.q) {
             CHROMO_TRY(aux_fork(st, &wst));
             if (wst != st) CHROMO_TRY(queue.flush(wst, 64));
         }
@@ -727,7 +818,7 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
     }   // part1
     float* gR = gcur;                   // dX_in incl. the residual of net.py:378 (the Regulation loop ends in the buffer it began in)
     if (!part2) {
-        if (tc) CHROMO_TRY(queue.flush(st));
+        if (cx.q) CHROMO_TRY(queue.flush(st));
         return aux_join(st, wst);
     }
 
@@ -768,6 +859,9 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
             s.dS = ws + o_dSp[r];
             Ctx cr = cx; cr.st = prs.s[r];
             CHROMO_TRY(sqa_bwd(cr, s));
+            // both layers read the same pCRE embedding: the last layer writes, lower ones add (before the next layer's
+            // sqa_bwd reuses dS on this stream)
+            if (dx && dx->x_pcre[r]) CHROMO_TRY(input_grad(prs.s[r], s, nullptr, dx->x_pcre[r], l != c->pw_layers - 1));
         }
         CHROMO_TRY(res_join(prs));
         CHROMO_TRY(bwd_weight(cx, ws + o_dQp[l], dmp, GS, pin, D, pin_div, RS, G + pa.p_att, D, L.pw_stride, R, dmp, D, NR));
@@ -787,7 +881,7 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
         CHROMO_TRY(gemm_auto(g, true, false, NR, st, tc));
     }
 
-    if (tc) {     // the Pairwise weight gradients follow on the side stream (ordered behind st)
+    if (cx.q) {   // the Pairwise weight gradients follow on the side stream (ordered behind st)
         CHROMO_TRY(aux_fork(st, &wst));
         if (wst != st) CHROMO_TRY(queue.flush(wst, 64));
     }
@@ -809,8 +903,9 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
         CHROMO_TRY(bwd_data(cx, gC, D, GS, P + ea.ffw, L.embed_stride, ws + o_dAve, dme, GS, B, D, dme, DataEpi(), NR));
         ResStreams ers;
         CHROMO_TRY(res_fork(st, NR, ers));
+        SqaBwd es[CHROMO_MAX_RES];
         for (int r = 0; r < NR; ++r) {
-            SqaBwd s;
+            SqaBwd& s = es[r];
             s.rows = B; s.H = He; s.dm = dme; s.D = D; s.n = c->n_bins[r]; s.F = F;
             s.q = ws + r * RS + w.e_q; s.qk = ws + r * RS + w.e_qk; s.P = ws + w.e_p[r];
             s.xbar = ws + r * RS + w.e_xbar; s.cbar = ws + r * RS + w.e_cbar;
@@ -838,8 +933,11 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
             CHROMO_TRY(bwd_weight(c1, dHc + r * GS, D, 0, in->x_p[r] + (long long)(n / 2) * F, n * F, 1, 0,
                                   G + L.embed[r].lin_proj, F, 0, B, D, F, 1));
         }
+        // promoter features: keys / values of every bin, and the centre bin's Hc through dHc
+        for (int r = 0; r < NR; ++r)
+            if (dx && dx->x_p[r]) CHROMO_TRY(input_grad(st, es[r], dHc + r * GS, dx->x_p[r], false));
     }
-    if (tc) CHROMO_TRY(queue.flush(st));
+    if (cx.q) CHROMO_TRY(queue.flush(st));
     return aux_join(st, wst);
 }
 
@@ -847,20 +945,43 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
 
 using namespace chromo;
 
+// The checks both entry points share (`out`: the entry point's required output); fills *w.
+static int backward_args(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in, const float* dlogits,
+                         const void* out, float* workspace, int64_t workspace_floats, int32_t flags, const char* who,
+                         WsLayout* w) {
+    CHROMO_TRY(validate_config(cfg));
+    if (!params || !in || !dlogits || !out || !workspace) { set_error("null pointer argument"); return CHROMO_EINVAL; }
+    if (!(flags & CHROMO_F_TRAINING)) { set_error("%s needs the CHROMO_F_TRAINING workspace", who); return CHROMO_EINVAL; }
+    if (in->batch < 1) { set_error("batch must be >= 1"); return CHROMO_EINVAL; }
+    *w = make_ws_layout(cfg, in->batch, flags);
+    if (workspace_floats < w->total) {
+        set_error("workspace too small: need %lld floats, got %lld", (long long)w->total, (long long)workspace_floats);
+        return CHROMO_ENOMEM;
+    }
+    return CHROMO_OK;
+}
+
 extern "C" int chromo_backward(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
                                const float* dlogits, float* grads, float* workspace, int64_t workspace_floats,
                                int32_t flags, void* stream) {
-    CHROMO_TRY(validate_config(cfg));
-    if (!params || !in || !dlogits || !grads || !workspace) { set_error("null pointer argument"); return CHROMO_EINVAL; }
-    if (!(flags & CHROMO_F_TRAINING)) { set_error("chromo_backward needs the CHROMO_F_TRAINING workspace"); return CHROMO_EINVAL; }
-    if (in->batch < 1) { set_error("batch must be >= 1"); return CHROMO_EINVAL; }
-    WsLayout w = make_ws_layout(cfg, in->batch, flags);
-    if (workspace_floats < w.total) {
-        set_error("workspace too small: need %lld floats, got %lld", (long long)w.total, (long long)workspace_floats);
-        return CHROMO_ENOMEM;
-    }
+    WsLayout w;
+    CHROMO_TRY(backward_args(cfg, params, in, dlogits, grads, workspace, workspace_floats, flags, "chromo_backward", &w));
     const bool only1 = (flags & CHROMO_F_BWD_HEAD_REG) != 0, only2 = (flags & CHROMO_F_BWD_REST) != 0;
     if (only1 && only2) { set_error("chromo_backward: CHROMO_F_BWD_HEAD_REG and CHROMO_F_BWD_REST are exclusive"); return CHROMO_EINVAL; }
     return backward_impl(cfg, params, in, dlogits, grads, workspace, w, (cudaStream_t)stream,
                          (flags & CHROMO_F_BF16) != 0, !only2, !only1);
+}
+
+extern "C" int chromo_backward_inputs(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                                      const float* dlogits, float* grads, const chromo_input_grads_t* dx,
+                                      float* workspace, int64_t workspace_floats, int32_t flags, void* stream) {
+    WsLayout w;
+    CHROMO_TRY(backward_args(cfg, params, in, dlogits, dx, workspace, workspace_floats, flags, "chromo_backward_inputs",
+                             &w));
+    if (flags & (CHROMO_F_BWD_HEAD_REG | CHROMO_F_BWD_REST)) {
+        set_error("chromo_backward_inputs runs the whole pass: CHROMO_F_BWD_HEAD_REG / CHROMO_F_BWD_REST are not accepted");
+        return CHROMO_EINVAL;
+    }
+    return backward_impl(cfg, params, in, dlogits, grads, workspace, w, (cudaStream_t)stream,
+                         (flags & CHROMO_F_BF16) != 0, true, true, dx);
 }

@@ -174,15 +174,16 @@ class RegulationTransformer(nn.Module):
 # autograd bridge
 # --------------------------------------------------------------------------------------
 class _ChromoFunction(torch.autograd.Function):
-    """loss.backward() support for the unchanged training loop (train.py:182-196).
+    """loss.backward() support for the unchanged training loop (train.py:182-196), and gradients with respect to the
+    histone-mark features (``promoter_feats`` / ``pcre_feats``, passed as ``feats``: every x_p, then every x_pcre).
 
     Limits (by design: the backward kernels write straight into the flat gradient buffer): parameter gradients
-    arrive as a side effect on ``p.grad`` (``torch.autograd.grad(loss, params)`` sees only the zero anchor), there is
-    no gradient with respect to the input features, and a forward's activations are released by its first
+    arrive as a side effect on ``p.grad`` (``torch.autograd.grad(loss, params)`` sees only the zero anchor), the
+    masks and ``interaction_freq`` get no gradient, and a forward's activations are released by its first
     backward (no ``retain_graph``)."""
 
     @staticmethod
-    def forward(ctx, anchor, model, io):
+    def forward(ctx, anchor, model, io, *feats):
         logits, ws = model._launch_forward(io, _lib.F_TRAINING | model._precision_flag())
         ctx.model, ctx.io, ctx.ws = model, io, ws
         return logits
@@ -193,9 +194,10 @@ class _ChromoFunction(torch.autograd.Function):
         if ws is None:
             raise RuntimeError("chromoformer_b200: this forward's activations were released by its first backward "
                                "(retain_graph is not supported: run the forward again)")
-        model._launch_backward(io, ws, dlogits.contiguous())
+        want = ctx.needs_input_grad[3:]
+        dx = model._launch_backward(io, ws, dlogits.contiguous(), want if any(want) else None)
         ctx.ws = None
-        return None, None, None
+        return (None, None, None) + tuple(dx if dx is not None else [None] * len(want))
 
 
 class _BatchIO:
@@ -214,6 +216,7 @@ class _BatchIO:
             raise _lib.ChromoLibError("Chromoformer parameters are on %s; the sm_100a kernels need "
                                       "model.cuda() (there is no CPU fallback)" % dev)
         self.keep = []
+        self.x_p, self.x_pcre = [], []            # the FP32 contiguous features (their gradients take these shapes)
         st = _lib.Batch()
         B = int(mask_p[0].size(0))
         S = cfg.i_max + 1
@@ -223,6 +226,7 @@ class _BatchIO:
         def dev_tensor(t, dtype, what):
             if t.device != dev:
                 raise ValueError(f"{what} is on {t.device}, model on {dev}")
+            t = t.detach()        # (a feature that requires grad reaches the kernels through _ChromoFunction)
             if t.dtype != dtype:
                 t = t.to(dtype)
             t = t.contiguous()
@@ -240,6 +244,8 @@ class _BatchIO:
                                  f"[{B},{cfg.i_max},{n},{cfg.n_feats}]")
             st.x_p[r] = xp.data_ptr()
             st.x_pcre[r] = xc.data_ptr()
+            self.x_p.append(xp)
+            self.x_pcre.append(xc)
             for name, m, regions in (("p", mask_p[r], 1), ("pcre", mask_pcre[r], cfg.i_max)):
                 m = dev_tensor(m, torch.bool, "pad mask")
                 if m.numel() == B * regions * n * n:          # [B,regions,1,n,n] as in data.py:156-198
@@ -424,10 +430,28 @@ class _ChromoformerCore(nn.Module):
             object.__setattr__(self, "_packed_key", packed_key)
         return logits, ws
 
-    def _launch_backward(self, io, ws, dlogits):
+    def _launch_backward(self, io, ws, dlogits, want_dx=None):
+        """Parameter gradients into ``p.grad`` (chromo_backward).  ``want_dx``: one flag per feature tensor (every x_p,
+        then every x_pcre); the pass then also returns those features' gradients (chromo_backward_inputs), and leaves
+        the parameter gradients out entirely when no active parameter requires grad."""
         lib = _lib.load()
         flat = self._flat
         active = self.active_parameters()
+        stream = torch.cuda.current_stream(flat.device).cuda_stream
+        flags = _lib.F_TRAINING | self._precision_flag()
+        dx, dx_struct = None, None
+        if want_dx is not None:
+            nr = len(io.x_p)
+            dx = [torch.empty_like(t) if w else None for t, w in zip(io.x_p + io.x_pcre, want_dx)]
+            dx_struct = _lib.InputGrads()
+            for r in range(nr):
+                dx_struct.x_p[r] = dx[r].data_ptr() if dx[r] is not None else None
+                dx_struct.x_pcre[r] = dx[nr + r].data_ptr() if dx[nr + r] is not None else None
+            if not any(p.requires_grad for p in active):
+                _lib.check(lib.chromo_backward_inputs(ctypes.byref(io.cfg), flat.data_ptr(), ctypes.byref(io.struct),
+                                                      dlogits.data_ptr(), None, ctypes.byref(dx_struct), ws.data_ptr(),
+                                                      ws.numel(), flags, stream), "chromo_backward_inputs")
+                return dx
         fresh = all(p.grad is None for p in active)
         ours = self._flat_grad is not None and not fresh and all(
             p.grad is not None and p.grad.data_ptr() == self._flat_grad.data_ptr() + 4 * off
@@ -442,11 +466,14 @@ class _ChromoformerCore(nn.Module):
             target = self._flat_grad
         else:
             target = torch.zeros_like(flat)
-        stream = torch.cuda.current_stream(flat.device).cuda_stream
-        flags = _lib.F_TRAINING | self._precision_flag()
-        _lib.check(lib.chromo_backward(ctypes.byref(io.cfg), flat.data_ptr(), ctypes.byref(io.struct),
-                                       dlogits.data_ptr(), target.data_ptr(), ws.data_ptr(), ws.numel(),
-                                       flags, stream), "chromo_backward")
+        if dx_struct is None:
+            _lib.check(lib.chromo_backward(ctypes.byref(io.cfg), flat.data_ptr(), ctypes.byref(io.struct),
+                                           dlogits.data_ptr(), target.data_ptr(), ws.data_ptr(), ws.numel(),
+                                           flags, stream), "chromo_backward")
+        else:
+            _lib.check(lib.chromo_backward_inputs(ctypes.byref(io.cfg), flat.data_ptr(), ctypes.byref(io.struct),
+                                                  dlogits.data_ptr(), target.data_ptr(), ctypes.byref(dx_struct),
+                                                  ws.data_ptr(), ws.numel(), flags, stream), "chromo_backward_inputs")
         if fresh:
             for (_, p, off, numel) in self._slots:
                 if off < self._n_active and p.requires_grad:
@@ -456,6 +483,7 @@ class _ChromoformerCore(nn.Module):
                 if off < self._n_active and p.requires_grad:
                     g = target[off:off + numel].view(p.shape)
                     p.grad = g.clone() if p.grad is None else p.grad + g
+        return dx
 
     # ---- checkpoints: every key generation of the reference loads into every class (misc/convert_weight.py) ----
     def _own_key(self, canon):
@@ -484,8 +512,10 @@ class _ChromoformerCore(nn.Module):
 
     def _run(self, x_p, mask_p, x_pcre, mask_pcre, imask, freq, dense=False):
         io = _BatchIO(self, x_p, mask_p, x_pcre, mask_pcre, imask, freq)
-        if torch.is_grad_enabled() and any(p.requires_grad for p in self.parameters()):
-            return _ChromoFunction.apply(self._anchor, self, io)
+        feats = list(x_p) + list(x_pcre)
+        if torch.is_grad_enabled() and (any(p.requires_grad for p in self.parameters()) or
+                                        any(t.requires_grad for t in feats)):
+            return _ChromoFunction.apply(self._anchor, self, io, *feats)
         logits, _ = self._launch_forward(io, self._precision_flag() | (_lib.F_DENSE if dense else 0))
         return logits
 

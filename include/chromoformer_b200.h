@@ -166,6 +166,22 @@ int chromo_backward(const chromo_config_t* cfg, const float* params, const chrom
                     const float* dlogits /* [B,n_out] */, float* grads, float* workspace,
                     int64_t workspace_floats, int32_t flags, void* stream);
 
+/* ---- gradients with respect to the input features (saliency, integrated gradients) --------------------------
+ * The same pass as chromo_backward (same CHROMO_F_TRAINING workspace of the same batch, CHROMO_F_BF16 honoured)
+ * that also WRITES (=) the gradient of the histone-mark features of every resolution whose pointer is non-NULL:
+ * every element, zeros on padded bins and dummy pCRE slots included.  grads == NULL: no parameter gradient at all
+ * (no weight / bias contraction runs), otherwise grads is accumulated into exactly as by chromo_backward.  The
+ * masks, interaction_freq and the position tables get no gradient.  CHROMO_F_BWD_HEAD_REG / CHROMO_F_BWD_REST are
+ * rejected (CHROMO_EINVAL).                                                                                   */
+typedef struct chromo_input_grads {
+    float* x_p[CHROMO_MAX_RES];       /* [B,1,n_r,F], written (=) when non-NULL */
+    float* x_pcre[CHROMO_MAX_RES];    /* [B,I,n_r,F], written (=) when non-NULL */
+} chromo_input_grads_t;
+int chromo_backward_inputs(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                           const float* dlogits /* [B,n_out] */, float* grads /* NULL: no parameter gradient */,
+                           const chromo_input_grads_t* dx, float* workspace, int64_t workspace_floats,
+                           int32_t flags, void* stream);
+
 /* ---- the contraction of the training step on the tensor pipe (train.py:195: autograd of nn.Linear) --------
  * C[M,N] (=|+=) opA . opB^T with BF16 operands converted on the fly and FP32 accumulation (tcgen05 / TMEM):
  *   a_transposed = 0: A is [M,K] (ld lda); 1: A is [K,M]        b_transposed = 0: B is [N,K] (ld ldb); 1: B is [K,N]
