@@ -17,6 +17,7 @@ F_PACKED = 4
 F_DENSE = 64
 F_BWD_HEAD_REG = 16
 F_BWD_REST = 32
+F_FREQ_GRAD = 128
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libchromo_b200.so")
@@ -57,10 +58,12 @@ class Batch(Structure):
 
 
 class InputGrads(Structure):
-    """``chromo_input_grads_t`` — where chromo_backward_inputs writes the feature gradients (NULL: not wanted)."""
+    """``chromo_input_grads_t`` — where chromo_backward_inputs writes the feature gradients (NULL: not wanted) and,
+    with ``F_FREQ_GRAD``, the interaction_freq gradient."""
     _fields_ = [
         ("x_p", c_void_p * MAX_RES),
         ("x_pcre", c_void_p * MAX_RES),
+        ("freq", c_void_p),
     ]
 
 

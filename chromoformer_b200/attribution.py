@@ -1,20 +1,23 @@
-"""Feature attribution: which histone-mark bins of the promoter and of each pCRE drive a prediction.
+"""Input attribution: which histone-mark bins of the promoter and of each pCRE, and which pCRE-promoter interaction
+frequencies, drive a prediction.
 
 Both helpers take a batch in the ``forward_batch`` convention (the six forward arguments, dicts keyed by bin size,
 as ``synthetic.make_batch`` or the reference's DataLoader produce them) and return
-``{"promoter_feats": {b: ...}, "pcre_feats": {b: ...}}`` in the layouts of the inputs ([B,1,n,F] / [B,I,n,F]).
-The gradients come from the sm_100a backward (``chromo_backward_inputs``); the parameters are held fixed: they do not
-require grad during the call, and nothing is written to ``p.grad``.  The masks and ``interaction_freq`` are inputs
-held fixed, not attributed.
+``{"promoter_feats": {b: ...}, "pcre_feats": {b: ...}}`` in the layouts of the inputs ([B,1,n,F] / [B,I,n,F]); with
+``freq=True`` also ``"interaction_freq"`` ([B,S,S], S = I + 1).  Without it ``interaction_freq`` is held fixed, not
+attributed.  The gradients come from the sm_100a backward (``chromo_backward_inputs``); the parameters are held fixed:
+they do not require grad during the call, and nothing is written to ``p.grad``.  The masks are inputs held fixed.
+``pcre_scores`` folds a result into one score per pCRE slot.
 """
 import contextlib
 
 import torch
 
-__all__ = ["input_gradients", "integrated_gradients"]
+__all__ = ["input_gradients", "integrated_gradients", "pcre_scores"]
 
 _FEATS = ("promoter_feats", "pcre_feats")
 _MASKS = ("promoter_pad_masks", "pcre_pad_masks")
+_FREQ = "interaction_freq"
 
 
 def _default_target(model, target):
@@ -49,29 +52,40 @@ def _to_device(batch, model, bins):
     return out
 
 
-def _grads(model, batch, target, bins):
-    """d logits[:, target].sum() / d features of a device batch keyed by int bin size."""
+def _grads(model, batch, target, bins, freq=False):
+    """d logits[:, target].sum() / d features (and d interaction_freq with ``freq``) of a device batch keyed by int bin
+    size."""
     leaves = {key: {b: batch[key][b].detach().requires_grad_(True) for b in bins} for key in _FEATS}
+    if freq:
+        leaves[_FREQ] = batch[_FREQ].detach().requires_grad_(True)
     with torch.enable_grad():
         logits = model.forward_batch({**batch, **leaves})
-        flat = [leaves[key][b] for key in _FEATS for b in bins]
+        flat = [leaves[key][b] for key in _FEATS for b in bins] + ([leaves[_FREQ]] if freq else [])
         g = torch.autograd.grad(logits[:, target].sum(), flat)
     it = iter(g)
-    return {key: {b: next(it) for b in bins} for key in _FEATS}
+    out = {key: {b: next(it) for b in bins} for key in _FEATS}
+    if freq:
+        out[_FREQ] = next(it)
+    return out
 
 
 def _relabel(out, batch, bins):
-    return {key: {_key(batch[key], b): out[key][b] for b in bins} for key in _FEATS}
+    res = {key: {_key(batch[key], b): out[key][b] for b in bins} for key in _FEATS}
+    if _FREQ in out:
+        res[_FREQ] = out[_FREQ]
+    return res
 
 
-def input_gradients(model, batch, target=None):
-    """Saliency: the gradient of ``logits[:, target].sum()`` with respect to every feature tensor of ``batch``.  Genes
-    are independent, so row g of the result is the gradient of gene g's own logit.  ``target`` defaults to column 1
-    for the classifier and 0 for the regressor."""
+def input_gradients(model, batch, target=None, freq=False):
+    """Saliency: the gradient of ``logits[:, target].sum()`` with respect to every feature tensor of ``batch``, and
+    with ``freq=True`` with respect to ``interaction_freq`` too.  Genes are independent, so row g of the result is the
+    gradient of gene g's own logit.  ``target`` defaults to column 1 for the classifier and 0 for the regressor.  With
+    the parameters held fixed and only ``interaction_freq`` asked for, the backward stops after the Regulation
+    transformer; asking for the features as well costs what the features alone cost, plus one small kernel."""
     bins = list(model.binsizes)
     t = _default_target(model, target)
     with _parameters_fixed(model):
-        out = _grads(model, _to_device(batch, model, bins), t, bins)
+        out = _grads(model, _to_device(batch, model, bins), t, bins, freq)
     return _relabel(out, batch, bins)
 
 
@@ -82,13 +96,16 @@ def _centre_rows(m, regions):
     return m.reshape(m.shape[0], regions, m.shape[-1])
 
 
-def integrated_gradients(model, batch, target=None, steps=32, baseline=None, chunk=4096):
-    """Integrated gradients over the features, midpoint rule: with alpha_k = (k + 1/2) / steps,
+def integrated_gradients(model, batch, target=None, steps=32, baseline=None, chunk=4096, freq=False):
+    """Integrated gradients, midpoint rule: with alpha_k = (k + 1/2) / steps,
         IG = (x - x0) * mean_k grad f(x0 + alpha_k (x - x0))
-    where f = logits[:, target] and the masks, interaction masks and interaction_freq stay those of ``batch``.
-    ``baseline`` (same layout as the result) defaults to zero features: ln(0 + 1), no reads.  The steps are stacked
-    along the batch dimension, at most ``chunk`` gene evaluations per forward / backward (a training workspace is
-    about 1.7 MB per gene); the pad masks are cut to their centre rows before they are replicated."""
+    where f = logits[:, target] and x is the features, or with ``freq=True`` the features and ``interaction_freq``
+    moving together along one path (the feature attributions are then those of that joint path, and completeness
+    holds over all of them: their sum approximates f(x) - f(x0)).  The masks and interaction masks, and without
+    ``freq`` interaction_freq, stay those of ``batch``.  ``baseline`` (same layout as the result) defaults to zero
+    features (ln(0 + 1), no reads) and zero interaction frequency.  The steps are stacked along the batch dimension, at
+    most ``chunk`` gene evaluations per forward / backward (a training workspace is about 1.7 MB per gene); the pad
+    masks are cut to their centre rows before they are replicated."""
     if steps < 1 or chunk < 1:
         raise ValueError("steps and chunk must be >= 1")
     bins = list(model.binsizes)
@@ -97,39 +114,70 @@ def integrated_gradients(model, batch, target=None, steps=32, baseline=None, chu
     I = int(dev_batch["pcre_feats"][bins[0]].shape[1])
     for key, regions in (("promoter_pad_masks", 1), ("pcre_pad_masks", I)):
         dev_batch[key] = {b: _centre_rows(m, regions) for b, m in dev_batch[key].items()}
-    x = {key: {b: dev_batch[key][b].float() for b in bins} for key in _FEATS}
+    # the inputs on the path, as (key, bin) with bin None for interaction_freq
+    path = [(key, b) for key in _FEATS for b in bins] + ([(_FREQ, None)] if freq else [])
+
+    def get(d, key, b):
+        return d[key] if b is None else d[key][b]
+
+    x = [get(dev_batch, key, b).float() for key, b in path]
     if baseline is None:
-        x0 = {key: {b: torch.zeros_like(x[key][b]) for b in bins} for key in _FEATS}
+        x0 = [torch.zeros_like(v) for v in x]
     else:
-        x0 = {key: {b: baseline[key][_key(baseline[key], b)].to(x[key][b]) for b in bins} for key in _FEATS}
-    delta = {key: {b: x[key][b] - x0[key][b] for b in bins} for key in _FEATS}
-    B = int(x["promoter_feats"][bins[0]].shape[0])
+        x0 = [(baseline[key] if b is None else baseline[key][_key(baseline[key], b)]).to(v)
+              for (key, b), v in zip(path, x)]
+    delta = [v - v0 for v, v0 in zip(x, x0)]
+    B = int(x[0].shape[0])
     alphas = [(k + 0.5) / steps for k in range(steps)]
     genes = min(B, chunk)                       # genes per evaluation
     per = max(1, chunk // genes)                # alpha steps per evaluation
     fixed = ("promoter_pad_masks", "pcre_pad_masks", "interaction_masks")
-    out = {key: {b: torch.empty_like(x[key][b]) for b in bins} for key in _FEATS}
+    out = [torch.empty_like(v) for v in x]
     with _parameters_fixed(model):
         for g0 in range(0, B, genes):
             g1 = min(B, g0 + genes)
-            acc = {key: {b: torch.zeros_like(x[key][b][g0:g1]) for b in bins} for key in _FEATS}
+            acc = [torch.zeros_like(v[g0:g1]) for v in x]
             for k0 in range(0, steps, per):
                 ks = alphas[k0:k0 + per]
-                sub = {key: {b: torch.cat([x0[key][b][g0:g1] + a * delta[key][b][g0:g1] for a in ks]) for b in bins}
-                       for key in _FEATS}
+                sub = {key: {} for key in _FEATS}
+                for (key, b), v0, d in zip(path, x0, delta):
+                    v = torch.cat([v0[g0:g1] + a * d[g0:g1] for a in ks])
+                    if b is None:
+                        sub[key] = v
+                    else:
+                        sub[key][b] = v
                 for key in fixed:
                     sub[key] = {b: dev_batch[key][b][g0:g1].repeat((len(ks),) + (1,) * (dev_batch[key][b].dim() - 1))
                                 for b in bins}
-                sub["interaction_freq"] = dev_batch["interaction_freq"][g0:g1].repeat(len(ks), 1, 1)
-                grads = _grads(model, sub, t, bins)
+                if not freq:
+                    sub[_FREQ] = dev_batch[_FREQ][g0:g1].repeat(len(ks), 1, 1)
+                grads = _grads(model, sub, t, bins, freq)
                 n = g1 - g0
-                for key in _FEATS:
-                    for b in bins:
-                        for i in range(len(ks)):        # the steps in order, whatever the chunking
-                            acc[key][b] += grads[key][b][i * n:(i + 1) * n]
-            for key in _FEATS:
-                for b in bins:
-                    out[key][b][g0:g1] = delta[key][b][g0:g1] * (acc[key][b] / steps)
-    dtype = {key: {b: dev_batch[key][b].dtype for b in bins} for key in _FEATS}
-    out = {key: {b: out[key][b].to(dtype[key][b]) for b in bins} for key in _FEATS}
-    return _relabel(out, batch, bins)
+                for j, (key, b) in enumerate(path):
+                    g = get(grads, key, b)
+                    for i in range(len(ks)):        # the steps in order, whatever the chunking
+                        acc[j] += g[i * n:(i + 1) * n]
+            for j in range(len(path)):
+                out[j][g0:g1] = delta[j][g0:g1] * (acc[j] / steps)
+    res = {key: {} for key in _FEATS}
+    for (key, b), v in zip(path, out):
+        v = v.to(get(dev_batch, key, b).dtype)
+        if b is None:
+            res[key] = v
+        else:
+            res[key][b] = v
+    return _relabel(res, batch, bins)
+
+
+def pcre_scores(attr):
+    """One score per pCRE slot, [B, I], from a result of ``input_gradients`` / ``integrated_gradients``: the sum of the
+    slot's ``pcre_feats`` attribution over resolutions, bins and marks, plus, when the result has it, the
+    ``interaction_freq`` attribution of its contact with the promoter, [b, 0, i + 1].  Dummy slots score exactly 0."""
+    score = None
+    for v in attr["pcre_feats"].values():
+        s = v.float().sum(dim=(2, 3))
+        score = s if score is None else score + s
+    if _FREQ in attr:
+        f = attr[_FREQ].float()
+        score = score + f.reshape(f.shape[0], f.shape[-2], f.shape[-1])[:, 0, 1:]
+    return score

@@ -140,8 +140,23 @@ __global__ void head_residual_kernel(float* g, long long g_z, const float* dz, i
     g[z * g_z + (long long)b * S * D + d] += dz[(long long)b * n_res * D + z * D + d];
 }
 
+// dfreq[b, i, j] = sum_r sum_k part_r[(b*K + k), i, j]: the Regulation backward's partials of d interaction_freq (K = 1
+// from the gene kernel, K = H per-head slices from the warp kernel), summed in a fixed order; every element is written.
+__global__ void freq_grad_sum_kernel(float* dfreq, const float* part, long long part_z, int NR, int K, int B, int SS) {
+    CHROMO_PDL_ENTER();
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= (long long)B * SS) return;
+    const long long b = i / SS, e = i % SS;
+    float t = 0.f;
+    for (int r = 0; r < NR; ++r)
+        for (int k = 0; k < K; ++k) t += part[r * part_z + (b * K + k) * SS + e];
+    dfreq[i] = t;
+}
+
 // Backward of reg_attention_kernel.  One warp per (gene, head), lane = channel.
-template <int SMAX>
+// FREQ: also gamma_f[h] dS[i, j] (=|+=) into this head's own [S,S] slice of the dfreq partial ([B,H,S,S] per resolution;
+// freq_grad_sum_kernel sums the heads), lane j storing column j - no atomics.
+template <int SMAX, bool FREQ>
 __global__ void __launch_bounds__(256) reg_attention_bwd_kernel(RegAttnBwdArgs a) {
     CHROMO_PDL_ENTER();
     const int warp_in_block = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -167,6 +182,8 @@ __global__ void __launch_bounds__(256) reg_attention_bwd_kernel(RegAttnBwdArgs a
         dk[i] = 0.f; dv[i] = 0.f;
     }
     float dgam = 0.f;
+    const float gam = FREQ ? a.gamma_f[z * a.dgamma_z + h] : 0.f;
+    float* dfq = FREQ ? a.dfreq + z * a.dfreq_z + gw * S * S : nullptr;
 #pragma unroll
     for (int i = 0; i < SMAX; ++i) {
         if (i >= S) break;
@@ -199,6 +216,7 @@ __global__ void __launch_bounds__(256) reg_attention_bwd_kernel(RegAttnBwdArgs a
             if (j >= S) continue;
             const float ds = mask[i * S + j] ? 0.f : p[j] * (dp[j] - dot);
             dgam = fmaf(ds, freq[i * S + j], dgam);
+            if (FREQ && lane == j) dfq[i * S + j] = a.dfreq_add ? fmaf(gam, ds, dfq[i * S + j]) : gam * ds;
             dq = fmaf(ds, k[j], dq);
             dk[j] = fmaf(ds, q[i], dk[j]);
         }
@@ -218,8 +236,10 @@ __global__ void __launch_bounds__(256) reg_attention_bwd_kernel(RegAttnBwdArgs a
 // staged once in shared memory; four lanes (eight channels each) per (head, query) for dgate, dq and the score
 // gradients - two shuffles per key instead of a 32-lane reduction - then, after a barrier, per (head, key) for dk and dv
 // from the staged dS / P / dA.  (The kernel above spends its time in 81 warp-wide reductions per (gene, head).)
+// FREQ: also sum_h gamma_f[h] dS[h, i, j] (=|+=) into the gene's [S,S] of the dfreq partial ([B,S,S] per resolution),
+// one thread per (i, j) (the block has H*S*4 >= S*S threads), the heads summed in a fixed order.
 constexpr int RAB_PAD = 4;
-template <int SMAX>
+template <int SMAX, bool FREQ>
 __global__ void __launch_bounds__(SMAX * 32) reg_attention_gene_bwd_kernel(RegAttnBwdArgs a) {
     CHROMO_PDL_ENTER();
     extern __shared__ __align__(16) float rab_sm[];
@@ -313,6 +333,13 @@ __global__ void __launch_bounds__(SMAX * 32) reg_attention_gene_bwd_kernel(RegAt
         float t = 0.f;
         for (int q = 0; q < S; ++q) t += sm_gam[tid * S + q];
         atomicAdd(a.dgamma_f + z * a.dgamma_z + tid, t);
+    }
+    if (FREQ && tid < S * S) {
+        const float* gam = a.gamma_f + z * a.dgamma_z;
+        float t = 0.f;
+        for (int hh = 0; hh < H; ++hh) t = fmaf(gam[hh], sm_ds[hh * S * S + tid], t);
+        float* d = a.dfreq + z * a.dfreq_z + (long long)b * S * S + tid;
+        *d = a.dfreq_add ? *d + t : t;
     }
     {   // phase 2: (head, key j = i): dk[j] = scale sum_i dS[i, j] q[i],  dv[j] = sum_i P[i, j] dA[i]
         const int j = i;
@@ -696,10 +723,11 @@ int input_grad(cudaStream_t st, const SqaBwd& s, const float* dhc, float* dx, bo
 }  // namespace
 
 // G == nullptr: no parameter gradient (no weight / bias contraction, no LayerNorm or gamma_f reduction); dx: feature
-// gradients to write (nullptr or NULL entries: none) - chromo_backward passes (G, nullptr).
+// gradients to write (nullptr or NULL entries: none); dfreq: d interaction_freq [B,S,S] to write (nullptr: none) -
+// chromo_backward passes (G, nullptr, nullptr).
 static int backward_impl(const chromo_config_t* c, const float* P, const chromo_batch_t* in, const float* dlogits,
                          float* G, float* ws, const WsLayout& w, cudaStream_t st, bool tc, bool part1, bool part2,
-                         const chromo_input_grads_t* dx = nullptr) {
+                         const chromo_input_grads_t* dx = nullptr, float* dfreq = nullptr) {
     const ParamLayout& L = get_layout(c);
     const int B = w.B, I = w.I, S = w.S, R = w.R, T = w.T, D = w.D, F = c->n_feats, NR = c->n_res;
     const long long RS = w.res_stride;
@@ -721,6 +749,10 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
         o_gCr[l] = take((int64_t)T * D); o_dProj[l] = take((int64_t)T * 4 * dmr);
     }
     const int64_t o_tR0 = take((int64_t)T * D), o_tR1 = take((int64_t)T * D), o_dAtt = take((int64_t)T * dmr);
+    // The rest of each resolution's block (the Pairwise and Embedding gradient scratch, from o_gAp[0] on) is idle until
+    // the Pairwise stage: it holds that resolution's partial of d interaction_freq during the Regulation stage,
+    // [B,S,S] (gene kernel) or [B,Hr,S,S] (warp kernel: one slice per head).
+    const int64_t o_fq = cur;
     int64_t o_gAp[CHROMO_MAX_LAYERS], o_dFp[CHROMO_MAX_LAYERS], o_gCp[CHROMO_MAX_LAYERS], o_dAvp[CHROMO_MAX_LAYERS],
         o_dQp[CHROMO_MAX_LAYERS], o_dCbP[CHROMO_MAX_LAYERS], o_dQKp[CHROMO_MAX_LAYERS], o_dU8p[CHROMO_MAX_LAYERS];
     for (int l = 0; l < c->pw_layers; ++l) {
@@ -734,6 +766,12 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
                   o_dQKe = take((int64_t)B * He * D), o_dU8e = take((int64_t)B * He * 8),
                   o_tE0 = take((int64_t)B * D), o_tE1 = take((int64_t)B * D), o_dHc = take((int64_t)B * D);
     const long long GS = cur - blk0;
+    const bool gene_bwd = Hr == 8 && S <= 17;          // reg_attention_gene_bwd_kernel, else reg_attention_bwd_kernel
+    const int fq_k = gene_bwd ? 1 : Hr;                // dfreq partials per (resolution, gene)
+    if (dfreq && (int64_t)B * fq_k * S * S > blk0 + GS - o_fq) {
+        set_error("internal: interaction_freq gradient partials exceed the idle Pairwise scratch");
+        return CHROMO_ENOMEM;
+    }
     cur = blk0 + GS * NR;
     int64_t o_dSp[CHROMO_MAX_RES], o_dSe[CHROMO_MAX_RES];
     for (int r = 0; r < NR; ++r) {
@@ -785,20 +823,29 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
             a.freq = in->freq;
             for (int r = 0; r < NR; ++r) a.imask[r] = in->imask[r];
             a.dgamma_f = wgrad ? G + ra.gamma_f : nullptr; a.dgamma_z = L.reg_stride;
+            a.gamma_f = P + ra.gamma_f;
+            a.dfreq = dfreq ? ws + o_fq : nullptr; a.dfreq_z = GS;
+            a.dfreq_add = l != c->reg_layers - 1;       // the layers run in order on st
             dim3 grid((unsigned)(((long long)B * Hr + 7) / 8), NR);
-            if (Hr == 8 && S <= 17) {       // one CTA per gene, rows staged in shared memory
+            if (gene_bwd) {       // one CTA per gene, rows staged in shared memory
                 const size_t smem = ((size_t)S * (4 * dmr + RAB_PAD) + (size_t)S * dmr + 2 * (size_t)Hr * S * S + Hr * S) * sizeof(float);
                 static bool configured = false;
                 if (!configured) {
                     const int mx = (17 * (4 * 256 + RAB_PAD) + 17 * 256 + 2 * 8 * 17 * 17 + 8 * 17) * (int)sizeof(float);
-                    cudaFuncSetAttribute(reg_attention_gene_bwd_kernel<9>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
-                    cudaFuncSetAttribute(reg_attention_gene_bwd_kernel<17>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
+                    cudaFuncSetAttribute(reg_attention_gene_bwd_kernel<9, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
+                    cudaFuncSetAttribute(reg_attention_gene_bwd_kernel<17, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
+                    cudaFuncSetAttribute(reg_attention_gene_bwd_kernel<9, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
+                    cudaFuncSetAttribute(reg_attention_gene_bwd_kernel<17, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, mx);
                     configured = true;
                 }
-                if (S <= 9) launch_pdl(reg_attention_gene_bwd_kernel<9>, dim3(B, NR), dim3(Hr * S * 4), smem, st, a);
-                else launch_pdl(reg_attention_gene_bwd_kernel<17>, dim3(B, NR), dim3(Hr * S * 4), smem, st, a);
-            } else if (S <= 9) launch_pdl(reg_attention_bwd_kernel<9>, dim3(grid), dim3(256), 0, st, a);
-            else launch_pdl(reg_attention_bwd_kernel<17>, dim3(grid), dim3(256), 0, st, a);
+                auto k = S <= 9 ? (dfreq ? reg_attention_gene_bwd_kernel<9, true> : reg_attention_gene_bwd_kernel<9, false>)
+                                : (dfreq ? reg_attention_gene_bwd_kernel<17, true> : reg_attention_gene_bwd_kernel<17, false>);
+                launch_pdl(k, dim3(B, NR), dim3(Hr * S * 4), smem, st, a);
+            } else {
+                auto k = S <= 9 ? (dfreq ? reg_attention_bwd_kernel<9, true> : reg_attention_bwd_kernel<9, false>)
+                                : (dfreq ? reg_attention_bwd_kernel<17, true> : reg_attention_bwd_kernel<17, false>);
+                launch_pdl(k, dim3(grid), dim3(256), 0, st, a);
+            }
             CHROMO_CHECK_LAUNCH("reg_attention_bwd");
         }
         CHROMO_TRY(bwd_weight(cx, dProj, 4 * dmr, GS, xin, D, 1, RS, G + ra.att, D, L.reg_stride, T, 4 * dmr, D, NR));
@@ -815,6 +862,11 @@ static int backward_impl(const chromo_config_t* c, const float* P, const chromo_
     // thirds of the SMs, under the Pairwise / Embedding backward; the rest follows at the end.
     launch_pdl(head_residual_kernel, dim3(dim3((B * D + 255) / 256, NR)), dim3(256), 0, st, gcur, GS, ws + o_dz, B, S, D, NR);
     CHROMO_CHECK_LAUNCH("head_residual");
+    if (dfreq) {      // before the Pairwise stage reuses the partials' scratch on st
+        launch_pdl(freq_grad_sum_kernel, dim3((unsigned)(((long long)B * S * S + 255) / 256)), dim3(256), 0, st, dfreq,
+                   (const float*)(ws + o_fq), GS, NR, fq_k, B, S * S);
+        CHROMO_CHECK_LAUNCH("freq_grad_sum");
+    }
     }   // part1
     float* gR = gcur;                   // dX_in incl. the residual of net.py:378 (the Regulation loop ends in the buffer it began in)
     if (!part2) {
@@ -982,6 +1034,15 @@ extern "C" int chromo_backward_inputs(const chromo_config_t* cfg, const float* p
         set_error("chromo_backward_inputs runs the whole pass: CHROMO_F_BWD_HEAD_REG / CHROMO_F_BWD_REST are not accepted");
         return CHROMO_EINVAL;
     }
+    float* dfreq = nullptr;             // (dx->freq exists only for callers that set the flag)
+    if (flags & CHROMO_F_FREQ_GRAD) {
+        if (!dx->freq) { set_error("chromo_backward_inputs: CHROMO_F_FREQ_GRAD with dx->freq == NULL"); return CHROMO_EINVAL; }
+        dfreq = dx->freq;
+    }
+    // Only parameter and feature gradients need the Pairwise / Embedding stages: d interaction_freq alone stops after
+    // the Regulation stage.
+    bool feats = false;
+    for (int r = 0; r < cfg->n_res; ++r) feats |= dx->x_p[r] != nullptr || dx->x_pcre[r] != nullptr;
     return backward_impl(cfg, params, in, dlogits, grads, workspace, w, (cudaStream_t)stream,
-                         (flags & CHROMO_F_BF16) != 0, true, true, dx);
+                         (flags & CHROMO_F_BF16) != 0, true, grads != nullptr || feats, dx, dfreq);
 }

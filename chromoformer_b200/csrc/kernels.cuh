@@ -56,6 +56,11 @@ struct RegAttnBwdArgs {
     const float* freq;
     const uint8_t* imask[CHROMO_MAX_RES];
     float* dgamma_f; long long dgamma_z;
+    // d interaction_freq (chromo_backward_inputs with CHROMO_F_FREQ_GRAD): the kernels' FREQ instantiation adds
+    // gamma_f[h] * dS into a per-resolution partial (stride dfreq_z); gamma_f has the stride dgamma_z of dgamma_f
+    const float* gamma_f;
+    float* dfreq; long long dfreq_z;
+    int dfreq_add;        // 0: write (top Regulation layer), 1: add (the layers below it)
 };
 
 struct AttnRowsBwdArgs {

@@ -175,15 +175,16 @@ class RegulationTransformer(nn.Module):
 # --------------------------------------------------------------------------------------
 class _ChromoFunction(torch.autograd.Function):
     """loss.backward() support for the unchanged training loop (train.py:182-196), and gradients with respect to the
-    histone-mark features (``promoter_feats`` / ``pcre_feats``, passed as ``feats``: every x_p, then every x_pcre).
+    inputs: the histone-mark features (``promoter_feats`` / ``pcre_feats``) and ``interaction_freq``, passed as
+    ``inputs``: every x_p, then every x_pcre, then interaction_freq.
 
     Limits (by design: the backward kernels write straight into the flat gradient buffer): parameter gradients
     arrive as a side effect on ``p.grad`` (``torch.autograd.grad(loss, params)`` sees only the zero anchor), the
-    masks and ``interaction_freq`` get no gradient, and a forward's activations are released by its first
-    backward (no ``retain_graph``)."""
+    masks and position tables get no gradient, and a forward's activations are released by its first backward
+    (no ``retain_graph``)."""
 
     @staticmethod
-    def forward(ctx, anchor, model, io, *feats):
+    def forward(ctx, anchor, model, io, *inputs):
         logits, ws = model._launch_forward(io, _lib.F_TRAINING | model._precision_flag())
         ctx.model, ctx.io, ctx.ws = model, io, ws
         return logits
@@ -267,6 +268,7 @@ class _BatchIO:
         if fq.numel() != B * S * S:
             raise ValueError(f"interaction_freq has shape {tuple(fq.shape)}, expected [{B},{S},{S}]")
         st.freq = fq.data_ptr()
+        self.freq = fq                            # (and its gradient this shape)
         self.struct = st
 
 
@@ -431,9 +433,10 @@ class _ChromoformerCore(nn.Module):
         return logits, ws
 
     def _launch_backward(self, io, ws, dlogits, want_dx=None):
-        """Parameter gradients into ``p.grad`` (chromo_backward).  ``want_dx``: one flag per feature tensor (every x_p,
-        then every x_pcre); the pass then also returns those features' gradients (chromo_backward_inputs), and leaves
-        the parameter gradients out entirely when no active parameter requires grad."""
+        """Parameter gradients into ``p.grad`` (chromo_backward).  ``want_dx``: one flag per input tensor (every x_p,
+        then every x_pcre, then interaction_freq); the pass then also returns those inputs' gradients
+        (chromo_backward_inputs), and leaves the parameter gradients out entirely when no active parameter requires
+        grad."""
         lib = _lib.load()
         flat = self._flat
         active = self.active_parameters()
@@ -442,11 +445,14 @@ class _ChromoformerCore(nn.Module):
         dx, dx_struct = None, None
         if want_dx is not None:
             nr = len(io.x_p)
-            dx = [torch.empty_like(t) if w else None for t, w in zip(io.x_p + io.x_pcre, want_dx)]
+            dx = [torch.empty_like(t) if w else None for t, w in zip(io.x_p + io.x_pcre + [io.freq], want_dx)]
             dx_struct = _lib.InputGrads()
             for r in range(nr):
                 dx_struct.x_p[r] = dx[r].data_ptr() if dx[r] is not None else None
                 dx_struct.x_pcre[r] = dx[nr + r].data_ptr() if dx[nr + r] is not None else None
+            if dx[-1] is not None:
+                dx_struct.freq = dx[-1].data_ptr()
+                flags |= _lib.F_FREQ_GRAD
             if not any(p.requires_grad for p in active):
                 _lib.check(lib.chromo_backward_inputs(ctypes.byref(io.cfg), flat.data_ptr(), ctypes.byref(io.struct),
                                                       dlogits.data_ptr(), None, ctypes.byref(dx_struct), ws.data_ptr(),
@@ -512,10 +518,10 @@ class _ChromoformerCore(nn.Module):
 
     def _run(self, x_p, mask_p, x_pcre, mask_pcre, imask, freq, dense=False):
         io = _BatchIO(self, x_p, mask_p, x_pcre, mask_pcre, imask, freq)
-        feats = list(x_p) + list(x_pcre)
+        inputs = list(x_p) + list(x_pcre) + [freq]
         if torch.is_grad_enabled() and (any(p.requires_grad for p in self.parameters()) or
-                                        any(t.requires_grad for t in feats)):
-            return _ChromoFunction.apply(self._anchor, self, io, *feats)
+                                        any(t.requires_grad for t in inputs)):
+            return _ChromoFunction.apply(self._anchor, self, io, *inputs)
         logits, _ = self._launch_forward(io, self._precision_flag() | (_lib.F_DENSE if dense else 0))
         return logits
 

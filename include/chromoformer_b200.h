@@ -53,6 +53,7 @@ extern "C" {
                                  path - dummy slots of data.py:175-203 leave the Pairwise and
                                  Regulation stages, padded bins of data.py:86-97 leave the attention
                                  windows - is not built.  Results do not depend on the hint.     */
+#define CHROMO_F_FREQ_GRAD 128 /* chromo_backward_inputs: also write d interaction_freq to dx->freq */
 
 /* Hyper-parameters: the config.yaml schema of chromoformer/configs/default.yaml:11-32
  * plus the number of bins per resolution (w_max // binsize, data.py:140).     */
@@ -166,16 +167,20 @@ int chromo_backward(const chromo_config_t* cfg, const float* params, const chrom
                     const float* dlogits /* [B,n_out] */, float* grads, float* workspace,
                     int64_t workspace_floats, int32_t flags, void* stream);
 
-/* ---- gradients with respect to the input features (saliency, integrated gradients) --------------------------
+/* ---- gradients with respect to the inputs (saliency, integrated gradients) ------------------------------------
  * The same pass as chromo_backward (same CHROMO_F_TRAINING workspace of the same batch, CHROMO_F_BF16 honoured)
  * that also WRITES (=) the gradient of the histone-mark features of every resolution whose pointer is non-NULL:
- * every element, zeros on padded bins and dummy pCRE slots included.  grads == NULL: no parameter gradient at all
- * (no weight / bias contraction runs), otherwise grads is accumulated into exactly as by chromo_backward.  The
- * masks, interaction_freq and the position tables get no gradient.  CHROMO_F_BWD_HEAD_REG / CHROMO_F_BWD_REST are
- * rejected (CHROMO_EINVAL).                                                                                   */
+ * every element, zeros on padded bins and dummy pCRE slots included.  With CHROMO_F_FREQ_GRAD in flags it also
+ * WRITES (=) the gradient of interaction_freq to dx->freq (non-NULL then), every element, zeros wherever the
+ * interaction mask of every resolution is set; without the flag dx->freq is never read, so callers built against
+ * the struct without that member keep working.  grads == NULL: no parameter gradient at all (no weight / bias
+ * contraction runs), otherwise grads is accumulated into exactly as by chromo_backward; with grads == NULL and no
+ * feature pointer the pass ends after the Regulation transformer.  The masks and the position tables get no
+ * gradient.  CHROMO_F_BWD_HEAD_REG / CHROMO_F_BWD_REST are rejected (CHROMO_EINVAL).                           */
 typedef struct chromo_input_grads {
     float* x_p[CHROMO_MAX_RES];       /* [B,1,n_r,F], written (=) when non-NULL */
     float* x_pcre[CHROMO_MAX_RES];    /* [B,I,n_r,F], written (=) when non-NULL */
+    float* freq;                      /* [B,S,S], written (=) with CHROMO_F_FREQ_GRAD; read only then */
 } chromo_input_grads_t;
 int chromo_backward_inputs(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
                            const float* dlogits /* [B,n_out] */, float* grads /* NULL: no parameter gradient */,
