@@ -84,6 +84,9 @@ EXPORTS = {
     "chromo_workspace_floats": (c_int64, [POINTER(Config), c_int32, c_int32]),
     "chromo_forward": (c_int32, [POINTER(Config), c_void_p, POINTER(Batch), c_void_p, c_void_p, c_int64,
                                  c_int32, c_void_p]),
+    "chromo_pcre_deletion_workspace_floats": (c_int64, [POINTER(Config), c_int32, c_int32]),
+    "chromo_pcre_deletion": (c_int32, [POINTER(Config), c_void_p, POINTER(Batch), c_void_p, c_void_p, c_void_p, c_void_p,
+                                       c_int64, c_int32, c_void_p]),
     "chromo_regulation_layer": (c_int32, [POINTER(Config), c_void_p, c_int32, c_void_p, c_void_p, c_int64,
                                           POINTER(c_void_p), c_void_p, c_int32, c_void_p, c_int64, c_int32, c_void_p]),
     "chromo_linear": (c_int32, [c_void_p, c_void_p, c_void_p, c_void_p, c_int32, c_int32, c_int32, c_int32, c_int32,

@@ -7,13 +7,17 @@ as ``synthetic.make_batch`` or the reference's DataLoader produce them) and retu
 ``freq=True`` also ``"interaction_freq"`` ([B,S,S], S = I + 1).  Without it ``interaction_freq`` is held fixed, not
 attributed.  The gradients come from the sm_100a backward (``chromo_backward_inputs``); the parameters are held fixed:
 they do not require grad during the call, and nothing is written to ``p.grad``.  The masks are inputs held fixed.
-``pcre_scores`` folds a result into one score per pCRE slot.
+``pcre_scores`` folds a result into one score per pCRE slot.  These are local (gradient) or path (integrated gradients)
+approximations; ``pcre_deletion`` gives the exact counterfactual per pCRE: the prediction with that pCRE removed.
 """
 import contextlib
 
 import torch
 
-__all__ = ["input_gradients", "integrated_gradients", "pcre_scores"]
+from . import _lib
+from .model import _BatchIO
+
+__all__ = ["input_gradients", "integrated_gradients", "pcre_scores", "pcre_deletion"]
 
 _FEATS = ("promoter_feats", "pcre_feats")
 _MASKS = ("promoter_pad_masks", "pcre_pad_masks")
@@ -181,3 +185,38 @@ def pcre_scores(attr):
         f = attr[_FREQ].float()
         score = score + f.reshape(f.shape[0], f.shape[-2], f.shape[-1])[:, 0, 1:]
     return score
+
+
+def pcre_deletion(model, batch, target=None, chunk=4096, dense=False):
+    """In-silico deletion of every pCRE of every gene (``chromo_pcre_deletion``): the exact logits of each gene
+    reassembled without each of its pCREs, from one Embedding / Pairwise pass per gene and a batched replay of the
+    Regulation transformer and the head.  Returns
+
+        "logits"         [B, n_out]     the ordinary forward (bit-identical to ``forward_batch`` with the same ``dense``)
+        "without"        [B, I, n_out]  the logits without pCRE i; on a dummy slot the logits themselves
+        "promoter_only"  [B, n_out]     the logits without any pCRE
+        "effect"         [B, I]         logits[:, target] - without[:, :, target]: > 0 when the pCRE raises the target
+                                        logit; exactly 0.0 on dummy slots
+
+    A slot counts as a pCRE when its token is unmasked in row 0 of some resolution's interaction mask; deleting it means
+    setting row and column i + 1 of every resolution's interaction mask.  ``target`` defaults to column 1 for the
+    classifier and 0 for the regressor.  At most ``chunk`` genes go to one library call (its workspace holds I + 1
+    variants per gene).  ``dense`` is the hint of ``forward_batch``.  Nothing requires grad, nothing touches ``p.grad``."""
+    if chunk < 1:
+        raise ValueError("chunk must be >= 1")
+    bins = list(model.binsizes)
+    t = _default_target(model, target)
+    dev_batch = _to_device(batch, model, bins)
+    B = int(dev_batch["interaction_freq"].shape[0])
+    flags = model._precision_flag() | (_lib.F_DENSE if dense else 0)
+    parts = []
+    with torch.no_grad():
+        for g0 in range(0, B, chunk):
+            g1 = min(B, g0 + chunk)
+            lists = [[dev_batch[key][b][g0:g1] for b in bins]
+                     for key in ("promoter_feats", "promoter_pad_masks", "pcre_feats", "pcre_pad_masks", "interaction_masks")]
+            io = _BatchIO(model, *lists, dev_batch[_FREQ][g0:g1])
+            parts.append(model._launch_deletion(io, flags))
+    logits, without, promoter_only = (torch.cat(p) for p in zip(*parts))
+    return {"logits": logits, "without": without, "promoter_only": promoter_only,
+            "effect": logits[:, t:t + 1] - without[:, :, t]}

@@ -748,6 +748,9 @@ static int pack_all_weights(const chromo_config_t* c, const ParamLayout& L, cons
 }
 
 struct RegOnly { int layer; const float* x; float* y; long long xy_stride; };
+// The Regulation transformer and the head alone, over the X_in rows already in the workspace (the variants of
+// chromo_pcre_deletion); the fused Regulation kernel runs under the token classes of `plan` when it is set.
+struct RegReplay { const RaggedPlan* plan; };
 
 // The side stream of aux_fork: joined back into `st` by join(), or on leaving the scope when an error return comes first
 // (a fork left open invalidates a stream capture).
@@ -758,14 +761,18 @@ struct AuxStream {
 };
 
 static int forward_impl(const chromo_config_t* c, const float* P, const chromo_batch_t* in, float* logits,
-                        float* ws, const WsLayout& w, int flags, cudaStream_t st, const RegOnly* only = nullptr) {
+                        float* ws, const WsLayout& w, int flags, cudaStream_t st, const RegOnly* only = nullptr,
+                        const RegReplay* replay = nullptr) {
     const ParamLayout& L = get_layout(c);
     const int B = w.B, I = w.I, S = w.S, R = w.R, T = w.T, D = w.D, F = c->n_feats;
     const int NR = c->n_res;
     const bool train = w.training;
     const long long RS = w.res_stride;
     const bool bf16 = (flags & CHROMO_F_BF16) != 0;
-    const bool proj_bf16 = bf16 && !train && T >= 64;
+    // a replay over the S variants of each gene picks every path by the gene pass's row count (rows / S), so a gene's
+    // variants are computed the way the gene itself is
+    const int m_div = replay ? S : 1;
+    const bool proj_bf16 = bf16 && !train && T / m_div >= 64;
     const bool fold = bf16 && !train;           // folded single-query attention weights (see pack_all_weights)      // q|k|v|gate handed to the attention kernel in BF16
     __nv_bfloat16* packed = bf16 ? reinterpret_cast<__nv_bfloat16*>(ws + w.bf_params) : nullptr;
     // Dense projection: tcgen05 BF16 engine when requested and the shape qualifies, FP32 SIMT otherwise.
@@ -774,7 +781,7 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
             // training: parameters change every step, so nothing is packed: FP32 weights are converted while staged
             return gemm_auto(g, true, true, nz, st, true);
         }
-        if (bf16 && g.M >= 64 && g.B >= P && g.B < P + L.total && umma_supported(g))
+        if (bf16 && g.M / m_div >= 64 && g.B >= P && g.B < P + L.total && umma_supported(g))
             return umma_launch(g, packed + (g.B - P), nz, st);
         if (fold && g.B >= ws + w.fold_f32 && g.B < ws + w.fold_f32 + w.fold_total && umma_supported(g))
             return umma_launch(g, reinterpret_cast<const __nv_bfloat16*>(ws + w.fold_bf) + (g.B - (ws + w.fold_f32)), nz, st);
@@ -789,7 +796,7 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
 
     RaggedPlan plan;                            // (ragged.cu; built next to the Embedding stage when the fused kernels run)
     bool ragged = false, reg_plan = false, reg_y_att = false;
-    if (!only) {
+    if (!only && !replay) {
     // ---------------- Embedding transformer, centre query (net.py:31-59) ----
     {
         CentreEmbedArgs a;
@@ -1096,10 +1103,11 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
         }
     }
 
-    }   // !only
+    }   // !only && !replay
     // ---------------- Regulation transformer (net.py:152-153) ---------------
     const int dmr = c->reg_d_model, Hr = c->reg_heads;
     const bool pb16 = proj_bf16 && !reg_fp32;
+    const RaggedPlan* rgp = ragged ? &plan : replay ? replay->plan : nullptr;
     auto rlin = [&](const GemmArgs& g, int nz) -> int { return reg_fp32 ? lin_fp32(g, nz) : lin(g, nz); };
     for (int l = 0; l < c->reg_layers; ++l) {
         if (only && only->layer >= 0 && l != only->layer) continue;
@@ -1117,9 +1125,9 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
             if (all && l > 0) continue;
             RegFusedArgs a;
             a.B = B; a.S = S; a.G = 128 / S; a.n_tiles = (B + a.G - 1) / a.G;
-            if (ragged && all) {
+            if (rgp && all) {
                 // token classes of the plan: a tile holds genes of one class with their live tokens only
-                a.plan_tiles = plan.reg_tiles; a.plan_rows = plan.reg_rows; a.n_tiles = plan.reg_tiles_max;
+                a.plan_tiles = rgp->reg_tiles; a.plan_rows = rgp->reg_rows; a.n_tiles = rgp->reg_tiles_max;
                 reg_plan = true;
             }
             a.x = xin; a.x_z = x_z; a.y = xout; a.y_z = y_z;
@@ -1234,9 +1242,8 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
 
 using namespace chromo;
 
-extern "C" int chromo_forward(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
-                              float* logits, float* workspace, int64_t workspace_floats, int32_t flags,
-                              void* stream) {
+static int check_forward_args(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                              const float* logits, const float* workspace) {
     CHROMO_TRY(validate_config(cfg));
     if (!params || !in || !logits || !workspace) { set_error("null pointer argument"); return CHROMO_EINVAL; }
     if (in->batch < 1) { set_error("batch must be >= 1"); return CHROMO_EINVAL; }
@@ -1248,12 +1255,121 @@ extern "C" int chromo_forward(const chromo_config_t* cfg, const float* params, c
         }
     }
     if (!in->freq) { set_error("null interaction_freq"); return CHROMO_EINVAL; }
+    return CHROMO_OK;
+}
+
+extern "C" int chromo_forward(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                              float* logits, float* workspace, int64_t workspace_floats, int32_t flags,
+                              void* stream) {
+    CHROMO_TRY(check_forward_args(cfg, params, in, logits, workspace));
     WsLayout w = make_ws_layout(cfg, in->batch, flags);
     if (workspace_floats < w.total) {
         set_error("workspace too small: need %lld floats, got %lld", (long long)w.total, (long long)workspace_floats);
         return CHROMO_ENOMEM;
     }
     return forward_impl(cfg, params, in, logits, workspace, w, flags, (cudaStream_t)stream);
+}
+
+// ---- in-silico pCRE deletion (deletion.cu) ----
+// Workspace: the variant pass's own layout [0, wv.total) (its batch-independent front holds the packed BF16 weights both
+// passes read; the gene pass's layout fits inside it), then the gene X_in rows, the variants' freq and masks, their
+// logits and the Regulation plan of the variants.
+namespace {
+struct DeletionWs {
+    WsLayout wb, wv;
+    int64_t xin_b, freq_v, imask_v, logits_v, plan, total;
+    bool plan_on;
+};
+int deletion_ws(const chromo_config_t* c, int batch, int flags, DeletionWs* d) {
+    const int S = c->i_max + 1;
+    if ((int64_t)batch * S * S > INT32_MAX) { set_error("chromo_pcre_deletion: batch * (i_max + 1)^2 must fit in int32"); return CHROMO_EINVAL; }
+    const int V = batch * S;
+    d->wb = make_ws_layout(c, batch, flags);
+    d->wv = make_ws_layout(c, V, flags);
+    int64_t cur = d->wv.total;
+    auto take = [&](int64_t n) { int64_t o = cur; cur = align4(cur + n); return o; };
+    d->xin_b = take((int64_t)c->n_res * batch * S * c->d_emb);
+    d->freq_v = take((int64_t)V * S * S);
+    d->imask_v = take(((int64_t)V * S * S + 3) / 4 * c->n_res);
+    d->logits_v = take((int64_t)V * c->n_out);
+    d->plan_on = (flags & CHROMO_F_BF16) && d->wv.reg_fused;
+    d->plan = d->plan_on ? take(reg_plan_floats(V, c->i_max)) : 0;
+    d->total = cur;
+    return CHROMO_OK;
+}
+}  // namespace
+
+extern "C" int64_t chromo_pcre_deletion_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t flags) {
+    if (validate_config(cfg) != CHROMO_OK) return CHROMO_EINVAL;
+    if (batch < 1) { set_error("batch must be >= 1"); return CHROMO_EINVAL; }
+    DeletionWs d;
+    CHROMO_TRY(deletion_ws(cfg, batch, flags, &d));
+    return d.total;
+}
+
+extern "C" int chromo_pcre_deletion(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                                    float* logits, float* without, float* promoter_only, float* workspace,
+                                    int64_t workspace_floats, int32_t flags, void* stream) {
+    CHROMO_TRY(check_forward_args(cfg, params, in, logits, workspace));
+    if (!without || !promoter_only) { set_error("chromo_pcre_deletion: null output"); return CHROMO_EINVAL; }
+    if (flags & (CHROMO_F_TRAINING | CHROMO_F_REGONLY | CHROMO_F_BWD_HEAD_REG | CHROMO_F_BWD_REST | CHROMO_F_FREQ_GRAD)) {
+        set_error("chromo_pcre_deletion: inference only (flags CHROMO_F_BF16, CHROMO_F_PACKED, CHROMO_F_DENSE)");
+        return CHROMO_EINVAL;
+    }
+    DeletionWs d;
+    CHROMO_TRY(deletion_ws(cfg, in->batch, flags, &d));
+    if (workspace_floats < d.total) {
+        set_error("chromo_pcre_deletion: workspace too small: need %lld floats, got %lld", (long long)d.total,
+                  (long long)workspace_floats);
+        return CHROMO_ENOMEM;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    float* ws = workspace;
+    const int B = in->batch, I = cfg->i_max, S = I + 1, V = B * S, NR = cfg->n_res, D = cfg->d_emb;
+    // the genes: the ordinary forward (it packs the BF16 weights unless CHROMO_F_PACKED), X_in left in the workspace
+    CHROMO_TRY(forward_impl(cfg, params, in, logits, ws, d.wb, flags, st));
+    // their X_in rows out of the way of the variant layout, which overlaps the gene layout
+    const size_t row_bytes = (size_t)B * S * D * sizeof(float);
+    if (cudaMemcpy2DAsync(ws + d.xin_b, row_bytes, ws + d.wb.r_xin, (size_t)d.wb.res_stride * sizeof(float), row_bytes, NR,
+                          cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
+        set_error("chromo_pcre_deletion: X_in copy failed");
+        return CHROMO_ECUDA;
+    }
+    chromo_batch_t vin;
+    memset(&vin, 0, sizeof(vin));
+    vin.batch = V; vin.freq = ws + d.freq_v;
+    {
+        DeletionExpandArgs a;
+        a.B = B; a.I = I; a.n_res = NR;
+        a.xin = ws + d.xin_b; a.xin_z = (long long)B * S * D;
+        a.freq = in->freq;
+        a.xin_v = ws + d.wv.r_xin; a.xin_v_z = d.wv.res_stride;
+        a.freq_v = ws + d.freq_v;
+        for (int r = 0; r < NR; ++r) {
+            a.imask[r] = in->imask[r];
+            a.imask_v[r] = reinterpret_cast<uint8_t*>(ws + d.imask_v) + (long long)r * V * S * S;
+            vin.imask[r] = a.imask_v[r];
+        }
+        CHROMO_TRY(launch_deletion_expand(a, st));
+    }
+    RaggedPlan plan;
+    if (d.plan_on) {
+        RaggedArgs ra;
+        memset(&ra, 0, sizeof(ra));
+        ra.B = V; ra.I = I; ra.n_res = NR;
+        for (int r = 0; r < NR; ++r) ra.imask[r] = vin.imask[r];
+        CHROMO_TRY(build_reg_plan(ra, ws + d.plan, &plan, st));
+    }
+    // the variants: Regulation transformer + head, with the weights the gene pass packed
+    const RegReplay replay{d.plan_on ? &plan : nullptr};
+    const int vflags = (flags & ~CHROMO_F_DENSE) | ((flags & CHROMO_F_BF16) ? CHROMO_F_PACKED : 0);
+    CHROMO_TRY(forward_impl(cfg, params, &vin, ws + d.logits_v, ws, d.wv, vflags, st, nullptr, &replay));
+    DeletionScatterArgs s;
+    s.B = B; s.I = I; s.n_res = NR; s.n_out = cfg->n_out;
+    for (int r = 0; r < NR; ++r) s.imask[r] = in->imask[r];
+    s.logits = logits; s.logits_v = ws + d.logits_v;
+    s.without = without; s.promoter_only = promoter_only;
+    return launch_deletion_scatter(s, st);
 }
 
 extern "C" int chromo_regulation_layer(const chromo_config_t* cfg, const float* params, int32_t layer, const float* x,

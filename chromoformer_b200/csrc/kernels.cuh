@@ -92,6 +92,25 @@ struct SqaArgs {
     const __nv_bfloat16* pet_pk = nullptr;  //                   PE^T packed as a [D,n] weight
 };
 
+// in-silico pCRE deletion (deletion.cu): B genes -> V = B * (I + 1) variants of the Regulation stage
+struct DeletionExpandArgs {
+    int B, I, n_res;
+    const float* xin; long long xin_z;              // X_in of the genes [B*S, 128] per resolution
+    const uint8_t* imask[CHROMO_MAX_RES];           // [B,S,S]
+    const float* freq;                              // [B,S,S]
+    float* xin_v; long long xin_v_z;                // X_in of the variants [V*S, 128] per resolution
+    uint8_t* imask_v[CHROMO_MAX_RES];               // [V,S,S]
+    float* freq_v;                                  // [V,S,S]
+};
+struct DeletionScatterArgs {
+    int B, I, n_res, n_out;
+    const uint8_t* imask[CHROMO_MAX_RES];           // the genes' masks (which slots are live)
+    const float* logits; const float* logits_v;     // [B, n_out], [V, n_out]
+    float* without; float* promoter_only;           // [B, I, n_out], [B, n_out]
+};
+int launch_deletion_expand(const DeletionExpandArgs& a, cudaStream_t st);
+int launch_deletion_scatter(const DeletionScatterArgs& a, cudaStream_t st);
+
 int launch_reg_attention(const RegAttnArgs& a, int nz, cudaStream_t st);
 int launch_attn_rows(const AttnRowsArgs& a, cudaStream_t st);
 int single_query_attention(const SqaArgs& s, cudaStream_t st);

@@ -281,6 +281,20 @@ Carve carve(const RaggedArgs& a, float* ws, RaggedPlan* p) {
     return c;
 }
 
+// token classes of the Regulation stage from the interaction masks: the counts per (run, class), then the gene list, the
+// tiles and their row map
+int launch_reg_classes(const RaggedArgs& a, int* k_gene, int* cls_cnt, RaggedPlan* plan, cudaStream_t st) {
+    const int n_blk = (a.B + 1023) / 1024;
+    if (cudaMemsetAsync(cls_cnt, 0, (size_t)n_blk * NCLS * sizeof(int), st) != cudaSuccess) { set_error("ragged plan: memset failed"); return CHROMO_ECUDA; }
+    ragged_gene_kernel<<<(unsigned)(((long long)a.B * 32 + 255) / 256), 256, 0, st>>>(a, k_gene, cls_cnt);
+    CHROMO_CHECK_LAUNCH("ragged_gene");
+    ragged_class_kernel<<<n_blk, 1024, 0, st>>>(a.B, a.I, k_gene, cls_cnt, *plan);
+    CHROMO_CHECK_LAUNCH("ragged_class");
+    ragged_rows_kernel<<<plan->reg_tiles_max, 128, 0, st>>>(a.I, *plan);
+    CHROMO_CHECK_LAUNCH("ragged_rows");
+    return CHROMO_OK;
+}
+
 }  // namespace
 
 int ragged_reg_tiles_max(int B, int I) {
@@ -300,14 +314,7 @@ int build_ragged_plan(const RaggedArgs& a, float* ws, RaggedPlan* plan, cudaStre
     for (int r = 1; r < a.n_res; ++r)
         if (a.n[r] > a.n[r_fine]) r_fine = r;
     if (a.n[r_fine] > 512) { set_error("ragged plan: more than 512 bins per region"); return CHROMO_EINVAL; }
-    const int n_blk = (a.B + 1023) / 1024;
-    if (cudaMemsetAsync(c.cls_cnt, 0, (size_t)n_blk * NCLS * sizeof(int), st) != cudaSuccess) { set_error("ragged plan: memset failed"); return CHROMO_ECUDA; }
-    ragged_gene_kernel<<<(unsigned)(((long long)a.B * 32 + 255) / 256), 256, 0, st>>>(a, c.k_gene, c.cls_cnt);
-    CHROMO_CHECK_LAUNCH("ragged_gene");
-    ragged_class_kernel<<<n_blk, 1024, 0, st>>>(a.B, a.I, c.k_gene, c.cls_cnt, *plan);
-    CHROMO_CHECK_LAUNCH("ragged_class");
-    ragged_rows_kernel<<<plan->reg_tiles_max, 128, 0, st>>>(a.I, *plan);
-    CHROMO_CHECK_LAUNCH("ragged_rows");
+    CHROMO_TRY(launch_reg_classes(a, c.k_gene, c.cls_cnt, plan, st));
     ragged_span_kernel<<<(unsigned)(((long long)(R + SPAN_RPW - 1) / SPAN_RPW * 32 + 255) / 256), 256, 0, st>>>(a, c.k_gene, c.keys_in, c.vals_in, c, r_fine);
     CHROMO_CHECK_LAUNCH("ragged_span");
     size_t need = 0;
@@ -323,6 +330,25 @@ int build_ragged_plan(const RaggedArgs& a, float* ws, RaggedPlan* plan, cudaStre
     ragged_tile_kernel<<<(tiles * 32 + 255) / 256, 256, 0, st>>>(a, c, *plan);
     CHROMO_CHECK_LAUNCH("ragged_tile");
     return CHROMO_OK;
+}
+
+// class counts, n_partners per gene, gene list, tile count, tiles, row map
+long long reg_plan_floats(int B, int I) {
+    return a4((long long)((B + 1023) / 1024) * NCLS) + 2 * a4(B) + 4 + 132LL * ragged_reg_tiles_max(B, I);
+}
+
+int build_reg_plan(const RaggedArgs& a, float* ws, RaggedPlan* plan, cudaStream_t st) {
+    int* cur = reinterpret_cast<int*>(ws);
+    auto take = [&](long long n) { int* o = cur; cur += a4(n); return o; };
+    *plan = RaggedPlan();
+    int* cls_cnt = take((long long)((a.B + 1023) / 1024) * NCLS);
+    int* k_gene = take(a.B);
+    plan->gene_list = take(a.B);
+    plan->reg_n = take(4);
+    plan->reg_tiles_max = ragged_reg_tiles_max(a.B, a.I);
+    plan->reg_tiles = reinterpret_cast<int4*>(take(4LL * plan->reg_tiles_max));
+    plan->reg_rows = take(128LL * plan->reg_tiles_max);
+    return launch_reg_classes(a, k_gene, cls_cnt, plan, st);
 }
 
 }  // namespace chromo

@@ -34,5 +34,9 @@ long long ragged_plan_floats(int B, int I, int n_res);            // workspace t
 int ragged_reg_tiles_max(int B, int I);                           // upper bound of the Regulation tiles of a plan
 // carves the plan out of `ws` (ragged_plan_floats floats, 16-byte aligned) and builds it on `st`
 int build_ragged_plan(const RaggedArgs& a, float* ws, RaggedPlan* plan, cudaStream_t st);
+// The Regulation part of a plan alone (gene_list, reg_tiles, reg_rows, reg_n), from the interaction masks of `a` (B, I,
+// n_res, imask; nothing else is read): reg_plan_floats floats of `ws`, 16-byte aligned
+long long reg_plan_floats(int B, int I);
+int build_reg_plan(const RaggedArgs& a, float* ws, RaggedPlan* plan, cudaStream_t st);
 
 }  // namespace chromo

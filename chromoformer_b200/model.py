@@ -301,6 +301,7 @@ class _ChromoformerCore(nn.Module):
         object.__setattr__(self, "_anchor", None)
         object.__setattr__(self, "_table", None)
         object.__setattr__(self, "_packed_key", None)
+        object.__setattr__(self, "_deletion_packed_key", None)
         object.__setattr__(self, "_param_epoch", 0)
         self._rebuild_flat()
 
@@ -357,6 +358,7 @@ class _ChromoformerCore(nn.Module):
         BF16 weight packs are rebuilt on the next forward.  In-place torch ops are tracked automatically."""
         object.__setattr__(self, "_param_epoch", self._param_epoch + 1)
         object.__setattr__(self, "_packed_key", None)
+        object.__setattr__(self, "_deletion_packed_key", None)
 
     def _flat_is_current(self):
         base = self._flat.data_ptr()
@@ -396,12 +398,14 @@ class _ChromoformerCore(nn.Module):
             self._pe_cache[key] = t
         return t
 
-    def _workspace(self, cfg, batch, flags, cached):
+    def _workspace(self, cfg, batch, flags, cached, entry="chromo_workspace_floats"):
         lib = _lib.load()
-        n = _lib.check(lib.chromo_workspace_floats(ctypes.byref(cfg), batch, flags), "chromo_workspace_floats")
+        n = _lib.check(getattr(lib, entry)(ctypes.byref(cfg), batch, flags), entry)
         if not cached:
             return torch.empty(n, dtype=torch.float32, device=self._flat.device)
         key = (str(self._flat.device), flags & ~_lib.F_DENSE)      # (the hint does not change the layout)
+        if entry != "chromo_workspace_floats":
+            key = (entry,) + key
         ws = self._ws_cache.get(key)
         if ws is None or ws.numel() < n:
             ws = torch.empty(n, dtype=torch.float32, device=self._flat.device)
@@ -414,15 +418,9 @@ class _ChromoformerCore(nn.Module):
             self._rebuild_flat()
         training = bool(flags & _lib.F_TRAINING)
         ws = self._workspace(io.cfg, io.batch, flags, cached=not training)
-        packed_key = None
-        if (flags & _lib.F_BF16) and not training:
-            # the packed BF16 weights live at the (batch-independent) front of the cached workspace:
-            # reuse them while neither the buffer nor the parameters changed
-            # (p.data = view keeps each parameter's own version counter, so sum them)
-            packed_key = (ws.data_ptr(), sum(p._version for (_, p, _, _) in self._slots), self._param_epoch,
-                          int(io.cfg.i_max), tuple(io.cfg.n_bins[r] for r in range(io.cfg.n_res)))
-            if packed_key == self._packed_key:
-                flags |= _lib.F_PACKED
+        packed_key = self._packed_key_of(ws, io, flags) if not training else None
+        if packed_key is not None and packed_key == self._packed_key:
+            flags |= _lib.F_PACKED
         logits = torch.empty(io.batch, int(self._cfg.n_out), dtype=torch.float32, device=self._flat.device)
         stream = torch.cuda.current_stream(self._flat.device).cuda_stream
         _lib.check(lib.chromo_forward(ctypes.byref(io.cfg), self._flat.data_ptr(), ctypes.byref(io.struct),
@@ -431,6 +429,37 @@ class _ChromoformerCore(nn.Module):
         if packed_key is not None:
             object.__setattr__(self, "_packed_key", packed_key)
         return logits, ws
+
+    def _packed_key_of(self, ws, io, flags):
+        """The packed BF16 weights live at the (batch-independent) front of a cached inference workspace: they can be
+        reused while neither the buffer nor the parameters changed (p.data = view keeps each parameter's own version
+        counter, so sum them).  None: nothing is packed (FP32)."""
+        if not flags & _lib.F_BF16:
+            return None
+        return (ws.data_ptr(), sum(p._version for (_, p, _, _) in self._slots), self._param_epoch,
+                int(io.cfg.i_max), tuple(io.cfg.n_bins[r] for r in range(io.cfg.n_res)))
+
+    def _launch_deletion(self, io, flags):
+        """chromo_pcre_deletion: (logits [B, n_out], without [B, I, n_out], promoter_only [B, n_out]).  Its workspace
+        and packed BF16 weights are cached apart from the forward's, so the two never invalidate each other."""
+        lib = _lib.load()
+        if not self._flat_is_current():
+            self._rebuild_flat()
+        ws = self._workspace(io.cfg, io.batch, flags, cached=True, entry="chromo_pcre_deletion_workspace_floats")
+        packed_key = self._packed_key_of(ws, io, flags)
+        if packed_key is not None and packed_key == self._deletion_packed_key:
+            flags |= _lib.F_PACKED
+        dev, n_out, I = self._flat.device, int(self._cfg.n_out), int(io.cfg.i_max)
+        logits = torch.empty(io.batch, n_out, dtype=torch.float32, device=dev)
+        without = torch.empty(io.batch, I, n_out, dtype=torch.float32, device=dev)
+        promoter_only = torch.empty(io.batch, n_out, dtype=torch.float32, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(lib.chromo_pcre_deletion(ctypes.byref(io.cfg), self._flat.data_ptr(), ctypes.byref(io.struct),
+                                            logits.data_ptr(), without.data_ptr(), promoter_only.data_ptr(),
+                                            ws.data_ptr(), ws.numel(), flags, stream), "chromo_pcre_deletion")
+        if packed_key is not None:
+            object.__setattr__(self, "_deletion_packed_key", packed_key)
+        return logits, without, promoter_only
 
     def _launch_backward(self, io, ws, dlogits, want_dx=None):
         """Parameter gradients into ``p.grad`` (chromo_backward).  ``want_dx``: one flag per input tensor (every x_p,

@@ -114,6 +114,27 @@ int chromo_forward(const chromo_config_t* cfg, const float* params, const chromo
                    float* logits /* [B,n_out] */, float* workspace, int64_t workspace_floats,
                    int32_t flags, void* stream);
 
+/* ---- in-silico pCRE deletion: the exact effect of removing each pCRE of each gene -------------------------------
+ * For B genes with I = i_max slots (S = I + 1 tokens).  Slot i of gene g is LIVE when token i + 1 is unmasked in row 0
+ * of at least one resolution's interaction mask, DEAD otherwise (the dummy slots of data.py:175-203).
+ *   logits[g]          the ordinary forward, bit-identical to chromo_forward with the same flags;
+ *   without[g, i]      live slot: the logits with row and column i + 1 of every resolution's interaction mask set, which
+ *                      is the gene reassembled without pCRE i; dead slot: logits[g], bit for bit;
+ *   promoter_only[g]   the logits with tokens 1..I masked in every resolution (the gene with no pCRE at all).
+ * One Embedding + Pairwise pass serves every deletion of a gene (slot i's Pairwise output depends on the promoter and
+ * pCRE i only); the Regulation transformer and the head then run over V = B * (I + 1) variants whose live tokens come
+ * first, so that the BF16 path's ragged plan packs them into the token class below the gene's.  Every output element is
+ * written; no atomics on the floating-point path; identical inputs give identical outputs; no host synchronisation
+ * (legal inside a stream capture).  Flags: CHROMO_F_BF16, CHROMO_F_PACKED (as for chromo_forward) and the
+ * CHROMO_F_DENSE hint (the gene pass only); any other flag, or a NULL output, is CHROMO_EINVAL.  The workspace must hold
+ * chromo_pcre_deletion_workspace_floats floats (CHROMO_ENOMEM otherwise); it is not interchangeable with a
+ * chromo_forward workspace, except that it too keeps the packed BF16 weights at its front.                        */
+int64_t chromo_pcre_deletion_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t flags);
+int chromo_pcre_deletion(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                         float* logits /* [B,n_out] */, float* without /* [B,I,n_out] */,
+                         float* promoter_only /* [B,n_out] */, float* workspace, int64_t workspace_floats,
+                         int32_t flags, void* stream);
+
 /* ---- one Regulation-transformer layer: AttentionBlock with gate (modules.py:104-111 as used by
  * net.py:152-153), for every resolution at once: y[r] = layer(x[r]), x/y = [n_res][B*(i_max+1), d_emb] FP32
  * with `xy_stride` floats between resolutions.  With CHROMO_F_BF16 and the default geometry this is ONE
