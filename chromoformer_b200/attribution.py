@@ -9,15 +9,20 @@ attributed.  The gradients come from the sm_100a backward (``chromo_backward_inp
 they do not require grad during the call, and nothing is written to ``p.grad``.  The masks are inputs held fixed.
 ``pcre_scores`` folds a result into one score per pCRE slot.  These are local (gradient) or path (integrated gradients)
 approximations; ``pcre_deletion`` gives the exact counterfactual per pCRE: the prediction with that pCRE removed.
+``pcre_subsets`` gives the prediction without any set of pCREs, and on top of it ``pcre_shapley`` (credit per pCRE that
+sums to logits - promoter only) and ``pcre_interactions`` (the synergy of every pair of pCREs).
 """
 import contextlib
+import math
 
+import numpy as np
 import torch
 
 from . import _lib
 from .model import _BatchIO
 
-__all__ = ["input_gradients", "integrated_gradients", "pcre_scores", "pcre_deletion"]
+__all__ = ["input_gradients", "integrated_gradients", "pcre_scores", "pcre_deletion", "pcre_subsets", "pcre_shapley",
+           "pcre_interactions"]
 
 _FEATS = ("promoter_feats", "pcre_feats")
 _MASKS = ("promoter_pad_masks", "pcre_pad_masks")
@@ -220,3 +225,257 @@ def pcre_deletion(model, batch, target=None, chunk=4096, dense=False):
     logits, without, promoter_only = (torch.cat(p) for p in zip(*parts))
     return {"logits": logits, "without": without, "promoter_only": promoter_only,
             "effect": logits[:, t:t + 1] - without[:, :, t]}
+
+
+# ---- pCRE subsets (chromo_pcre_subsets) ----------------------------------------------------------------------------
+_GENE_KEYS = ("promoter_feats", "promoter_pad_masks", "pcre_feats", "pcre_pad_masks", "interaction_masks")
+_SUBSET_CHUNK = 65536           # variants per library call: about 3.8 GB of workspace in BF16, 33 GB in FP32
+
+
+def _live(dev_batch, bins):
+    """[B, I] bool on the device: slot i is a pCRE when token i + 1 is unmasked in row 0 of some resolution's
+    interaction mask (the definition of ``pcre_deletion``)."""
+    shape = dev_batch[_FREQ].shape
+    im = torch.stack([dev_batch["interaction_masks"][b].reshape(shape).bool() for b in bins])
+    return (~im[:, :, 0, 1:]).any(0)
+
+
+def _replay(model, dev_batch, bins, var_gene, var_drop, chunk, dense):
+    """logits [B, n_out] and var_logits [V, n_out] on the device for variant descriptors given as numpy int64 arrays:
+    var_gene non-decreasing, every gene with at least one variant.  One library call covers whole genes, at most ``chunk``
+    variants (a gene with more gets a call of its own), so every gene's Embedding / Pairwise pass runs once."""
+    if chunk < 1:
+        raise ValueError("chunk must be >= 1")
+    B = int(dev_batch[_FREQ].shape[0])
+    counts = np.bincount(var_gene, minlength=B)
+    if len(counts) != B or (counts == 0).any():
+        raise ValueError("every gene needs at least one variant, and var_gene must lie in [0, B)")
+    starts = np.concatenate([[0], np.cumsum(counts)])
+    flags = model._precision_flag() | (_lib.F_DENSE if dense else 0)
+    dev = model.flat_params.device
+    logits, var_logits = [], []
+    with torch.no_grad():
+        g0 = 0
+        while g0 < B:
+            g1 = int(np.searchsorted(starts, starts[g0] + chunk, side="right")) - 1
+            g1 = min(B, max(g1, g0 + 1))
+            v0, v1 = int(starts[g0]), int(starts[g1])
+            io = _BatchIO(model, *[[dev_batch[key][b][g0:g1] for b in bins] for key in _GENE_KEYS],
+                          dev_batch[_FREQ][g0:g1])
+            vg = torch.from_numpy((var_gene[v0:v1] - g0).astype(np.int32)).to(dev)
+            vd = torch.from_numpy(var_drop[v0:v1].astype(np.int32)).to(dev)
+            lg, vl = model._launch_subsets(io, vg, vd, flags)
+            logits.append(lg)
+            var_logits.append(vl)
+            g0 = g1
+    return torch.cat(logits), torch.cat(var_logits)
+
+
+def pcre_subsets(model, batch, drop, target=None, chunk=_SUBSET_CHUNK, dense=False):
+    """The exact logits of every gene without any set of its pCREs (``chromo_pcre_subsets``), from one Embedding /
+    Pairwise pass per gene and a batched replay of the Regulation transformer and the head over the variants.
+
+    ``drop`` is bool, [V, I] (the same V sets for every gene) or [B, V, I]: variant v of gene g is the gene without the
+    pCREs of slots ``drop[g, v]``.  Dropping a dummy slot (no pCRE, see ``pcre_deletion``) changes nothing; an empty set
+    gives the gene itself, the set of every pCRE the promoter alone.  Returns
+
+        "logits"    [B, n_out]      the ordinary forward (bit-identical to ``forward_batch`` with the same ``dense``)
+        "variants"  [B, V, n_out]   the logits of each variant
+        "value"     [B, V]          variants[..., target], only when ``target`` is given
+
+    At most ``chunk`` variants go to one library call, whole genes at a time (a gene with more variants than ``chunk``
+    gets a call of its own).  The replay needs about 58 kB of workspace per variant in BF16 with the default
+    configuration (X_in, the last Regulation layer's rows and the fused kernel's parking rows; no Embedding / Pairwise
+    buffers) and about 0.5 MB in FP32.  A variant's logits do not depend on the other variants or on ``chunk`` (as for a
+    forward, for chunks whose gene counts are on the same side of the 64-row threshold).  Nothing requires grad."""
+    bins = list(model.binsizes)
+    dev_batch = _to_device(batch, model, bins)
+    B, I = (int(n) for n in dev_batch[_FREQ].shape[:2])
+    I -= 1
+    drop = torch.as_tensor(drop)
+    if drop.dtype != torch.bool:
+        raise ValueError("drop must be a bool tensor")
+    if drop.dim() == 2:
+        drop = drop.unsqueeze(0).expand(B, -1, -1)
+    if drop.dim() != 3 or drop.shape[0] != B or drop.shape[2] != I or drop.shape[1] < 1:
+        raise ValueError(f"drop must be [V, {I}] or [{B}, V, {I}] with V >= 1, got {tuple(drop.shape)}")
+    V = int(drop.shape[1])
+    bits = (drop.cpu().long() << torch.arange(I)).sum(-1).reshape(-1).numpy()
+    logits, var_logits = _replay(model, dev_batch, bins, np.repeat(np.arange(B), V), bits, chunk, dense)
+    out = {"logits": logits, "variants": var_logits.view(B, V, -1)}
+    if target is not None:
+        out["value"] = out["variants"][..., _default_target(model, target)]
+    return out
+
+
+def _shapley_exact(v, k):
+    """Exact Shapley values of k players from v [G, 2^k] (float64; column s = the value of the coalition whose bit j
+    is set for player j): phi_j = sum over s without j of |s|! (k - |s| - 1)! / k! (v[s + j] - v[s]), accumulated over
+    s in increasing order.  [G, k]."""
+    w = [math.factorial(n) * math.factorial(k - n - 1) / math.factorial(k) for n in range(k)]
+    phi = torch.zeros(v.shape[0], k, dtype=torch.float64)
+    for s in range(1 << k):
+        js = [j for j in range(k) if not (s >> j) & 1]
+        if js:
+            phi[:, js] += w[bin(s).count("1")] * (v[:, [s | (1 << j) for j in js]] - v[:, s:s + 1])
+    return phi
+
+
+def _shapley_from_orders(v, order, k):
+    """The permutation (Monte-Carlo) estimate of Shapley values from P orders per gene: v [G, P, I + 1] float64, the
+    values of the prefixes of each order (entry j: the first j players of the order; entries past k[g] are not read),
+    order [G, P, I] the slots in order (the k[g] players first), k [G].  Player order[g, p, j - 1] gets
+    v[g, p, j] - v[g, p, j - 1]; the orders are added in turn and averaged, so per order the credits telescope to
+    v(all) - v(none).  Slots that are no player get exactly 0.  [G, I]."""
+    G, P, I = order.shape
+    valid = torch.arange(1, I + 1).view(1, I) <= k.view(G, 1)
+    phi = torch.zeros(G, I, dtype=torch.float64)
+    for p in range(P):
+        d = torch.where(valid, v[:, p, 1:] - v[:, p, :-1], torch.zeros((), dtype=torch.float64))
+        phi.scatter_add_(1, order[:, p, :], d)
+    return phi / P
+
+
+def _first_variants(var_gene):
+    """The index of each gene's first variant (var_gene non-decreasing, every gene present)."""
+    return np.concatenate([[0], np.cumsum(np.bincount(var_gene))[:-1]])
+
+
+def _shapley_descriptors(live):
+    """The variants of exact Shapley values: for each gene (in order) the 2^k subsets T of its k pCREs, variant s keeping
+    the pCREs whose bit is set in s (bit j: the j-th pCRE of the gene).  Returns var_gene, var_drop (numpy int64) and,
+    per pCRE count k, (k, the genes [G], their pCRE slots [G, k], the variant index of each (gene, s) [G, 2^k])."""
+    B, I = live.shape
+    k = live.sum(1)
+    live_bits = (live.long() << torch.arange(I)).sum(1).numpy()
+    pos = torch.argsort((~live).to(torch.int8), dim=1, stable=True)          # the pCREs of each gene first, ascending
+    n_var = (1 << k).numpy()
+    starts = np.concatenate([[0], np.cumsum(n_var)])
+    var_drop = np.zeros(int(starts[-1]), dtype=np.int64)
+    groups = []
+    for kk in sorted(set(k.tolist())):
+        genes = torch.nonzero(k == kk).view(-1)
+        sub = np.arange(1 << kk)
+        s_bits = (sub.reshape(-1, 1) >> np.arange(kk)) & 1                     # [2^k, k]
+        slots = pos[genes, :kk]
+        kept = (1 << slots.numpy().astype(np.int64)) @ s_bits.T                # [G, 2^k]
+        idx = starts[genes.numpy()].reshape(-1, 1) + sub.reshape(1, -1)
+        var_drop[idx] = live_bits[genes.numpy()].reshape(-1, 1) & ~kept
+        groups.append((kk, genes, slots, idx))
+    return np.repeat(np.arange(B), n_var), var_drop, groups
+
+
+def _interaction_descriptors(live):
+    """The variants of pairwise interactions: for each gene (in order) the candidates () (the gene itself), (i,) and
+    (i, j), i < j, whose slots are all pCREs.  Returns var_gene, var_drop (numpy int64), valid [B, n_cand] and the
+    pairs in candidate order."""
+    B, I = live.shape
+    pairs = [(i, j) for i in range(I) for j in range(i + 1, I)]
+    cand = [()] + [(i,) for i in range(I)] + pairs
+    bits = torch.tensor([sum(1 << i for i in c) for c in cand])
+    valid = torch.stack([live[:, list(c)].all(1) if c else torch.ones(B, dtype=torch.bool) for c in cand], 1)
+    gene = torch.arange(B).view(B, 1).expand(B, len(cand))
+    return gene[valid].numpy(), bits.view(1, -1).expand(B, -1)[valid].numpy(), valid, pairs
+
+
+def pcre_shapley(model, batch, target=None, permutations=None, seed=0, chunk=_SUBSET_CHUNK, dense=False):
+    """Shapley values of the pCREs of every gene: the players are the gene's pCREs (its live slots, as for
+    ``pcre_deletion``), the value of a set T is ``logits[target]`` of the gene with only the pCREs of T kept (from
+    ``pcre_subsets``).  A pCRE's value is its average marginal contribution over every order in which the pCREs could be
+    added, so redundant pCREs share their credit and cooperating pCREs are not credited twice, and the values of a gene
+    sum to v(all) - v(none) = logits[target] - promoter_only[target] (up to the rounding of the FP64 combination).
+
+    Exact by default: every subset of each gene's k pCREs, 2^k variants per gene; a gene with more than 12 pCREs is a
+    ValueError (use ``permutations=``).  With ``permutations=P``: the estimate over P random orders per gene (seeded by
+    ``seed``), k + 1 prefix variants per order; per order the credits sum exactly to v(all) - v(none).  The values are
+    combined in FP64 in a fixed order.  Returns
+
+        "shapley"        [B, I] float64   exactly 0.0 on dummy slots
+        "logits"         [B, n_out]       the ordinary forward
+        "promoter_only"  [B, n_out]       the logits without any pCRE
+
+    ``target`` defaults to column 1 for the classifier and 0 for the regressor; ``chunk`` and ``dense`` are those of
+    ``pcre_subsets``.  Cost: one Embedding / Pairwise pass per gene and the Regulation transformer over the variants; a
+    variant keeping m pCREs costs m + 1 tokens on the BF16 path (DESIGN.md 3.5)."""
+    bins = list(model.binsizes)
+    t = _default_target(model, target)
+    dev_batch = _to_device(batch, model, bins)
+    live = _live(dev_batch, bins).cpu()                      # (the one host read of the call)
+    B, I = live.shape
+    k = live.sum(1)
+    live_bits = (live.long() << torch.arange(I)).sum(1)
+    # the slots of each gene, its pCREs first (ascending)
+    shapley = torch.zeros(B, I, dtype=torch.float64)
+    if permutations is None:
+        if int(k.max()) > 12:
+            g = int(torch.argmax(k))
+            raise ValueError(f"gene {g} has {int(k[g])} pCREs: exact Shapley values need 2^k variants per gene; "
+                             "pass permutations= for the sampling estimate")
+        var_gene, var_drop, groups = _shapley_descriptors(live)
+        logits, var_logits = _replay(model, dev_batch, bins, var_gene, var_drop, chunk, dense)
+        v = var_logits[:, t].double().cpu().numpy()
+        for kk, genes, slots, idx in groups:
+            if kk:
+                shapley[genes.view(-1, 1), slots] = _shapley_exact(torch.from_numpy(v[idx]), kk)
+        promoter_only = var_logits[torch.from_numpy(_first_variants(var_gene)).to(var_logits.device)]   # the empty coalition
+    else:
+        P = int(permutations)
+        if P < 1:
+            raise ValueError("permutations must be >= 1")
+        gen = torch.Generator().manual_seed(int(seed))
+        r = torch.rand(B, P, I, generator=gen, dtype=torch.float64)
+        order = torch.argsort(torch.where(live.view(B, 1, I), r, torch.full((), 2.0, dtype=torch.float64)), dim=2)
+        kept = torch.cat([torch.zeros(B, P, 1, dtype=torch.long), torch.cumsum(1 << order, dim=2)], 2)   # [B, P, I + 1]
+        valid = (torch.arange(I + 1).view(1, 1, I + 1) <= k.view(B, 1, 1)).expand(B, P, I + 1)
+        drop = live_bits.view(B, 1, 1) & ~kept
+        gene = torch.arange(B).view(B, 1, 1).expand(B, P, I + 1)
+        logits, var_logits = _replay(model, dev_batch, bins, gene[valid].numpy(), drop[valid].numpy(), chunk, dense)
+        v = torch.zeros(B, P, I + 1, dtype=torch.float64)
+        v[valid] = var_logits[:, t].double().cpu()
+        shapley = _shapley_from_orders(v, order, k)
+        first = torch.nonzero(valid.reshape(-1)).view(-1)      # prefix 0 of order 0 is each gene's first variant
+        promoter_only = var_logits[torch.searchsorted(first, torch.arange(B) * P * (I + 1)).to(var_logits.device)]
+    dev = logits.device
+    return {"shapley": shapley.to(dev), "logits": logits, "promoter_only": promoter_only}
+
+
+def _interactions(f0, fi, fij, pairs, live):
+    """Delta_ij = f(N) - f(N without i) - f(N without j) + f(N without i, j) for the live pairs: f0 [G], fi [G, I],
+    fij [G, n_pairs] float64 for the pairs (i, j), i < j.  Returns (interaction [G, I, I], exactly symmetric, 0.0 on
+    the diagonal and on dead rows / columns; effect [G, I] = f0 - fi, 0.0 on dead slots)."""
+    G, I = live.shape
+    zero = torch.zeros((), dtype=torch.float64)
+    inter = torch.zeros(G, I, I, dtype=torch.float64)
+    for c, (i, j) in enumerate(pairs):
+        d = torch.where(live[:, i] & live[:, j], f0 - fi[:, i] - fi[:, j] + fij[:, c], zero)
+        inter[:, i, j] = d
+        inter[:, j, i] = d
+    return inter, torch.where(live, f0.view(G, 1) - fi, zero)
+
+
+def pcre_interactions(model, batch, target=None, chunk=_SUBSET_CHUNK, dense=False):
+    """Pairwise interaction effects of the pCREs of every gene, from the 1 + k + k (k - 1) / 2 variants of a gene with
+    k pCREs (``pcre_subsets``): with f = logits[target] and N the gene's pCREs,
+
+        Delta_ij = f(N) - f(N without i) - f(N without j) + f(N without i and j)
+
+    the extra effect of removing both over removing each alone: 0 when the two act independently, < 0 when each covers
+    for the other (redundant), > 0 when each needs the other (synergy).  Returns
+
+        "interaction"  [B, I, I] float64   exactly symmetric; exactly 0.0 on the diagonal and on dummy slots
+        "effect"       [B, I] float64      f(N) - f(N without i) (as ``pcre_deletion``'s); 0.0 on dummy slots
+        "logits"       [B, n_out]          the ordinary forward
+
+    f(N) is the replayed gene itself.  ``target``, ``chunk`` and ``dense`` as for ``pcre_shapley``."""
+    bins = list(model.binsizes)
+    t = _default_target(model, target)
+    dev_batch = _to_device(batch, model, bins)
+    live = _live(dev_batch, bins).cpu()
+    B, I = live.shape
+    var_gene, var_drop, valid, pairs = _interaction_descriptors(live)
+    logits, var_logits = _replay(model, dev_batch, bins, var_gene, var_drop, chunk, dense)
+    v = torch.zeros(B, valid.shape[1], dtype=torch.float64)
+    v[valid] = var_logits[:, t].double().cpu()
+    inter, effect = _interactions(v[:, 0], v[:, 1:1 + I], v[:, 1 + I:], pairs, live)
+    dev = logits.device
+    return {"interaction": inter.to(dev), "effect": effect.to(dev), "logits": logits}

@@ -122,6 +122,7 @@ struct WsLayout {
     int64_t tail_stream;    // packed weight streams of the fused Embedding/Pairwise tails (float offset)
     int tail_fused;         // 1 when the fused row-tail kernel applies
     int reg_fused;          // 1 when the fused Regulation-layer kernel applies to this configuration
+    int reg_compact;        // replay layout of the fused path: r_xin, r_att and the r_out parking slots only
     int64_t rg_plan;        // ragged plan of the batch (ragged.cu; float offset, 0 = none)
     // backward scratch (training only)
     int64_t g_base;
@@ -130,7 +131,10 @@ struct WsLayout {
     inline int pslot(int l) const { return training ? l : (l & 1); }
     inline int rslot(int l) const { return training ? l : (l & 1); }
 };
-WsLayout make_ws_layout(const chromo_config_t* cfg, int batch, int flags);
+// replay: the layout of a Regulation + head replay over `batch` variants (chromo_pcre_subsets): the same batch-independent
+// front (the packed BF16 weights), X_in, the Regulation buffers and the head, no Embedding or Pairwise block.  On the fused
+// BF16 path the Regulation buffers are the parking rows r_out and the last-layer rows r_att alone.
+WsLayout make_ws_layout(const chromo_config_t* cfg, int batch, int flags, bool replay = false);
 
 static inline int64_t align4(int64_t x) { return (x + 3) & ~int64_t(3); }
 

@@ -16,6 +16,8 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <algorithm>
+
 #include "common.cuh"
 #include "gemm_simt.cuh"
 #include "kernels.cuh"
@@ -749,8 +751,10 @@ static int pack_all_weights(const chromo_config_t* c, const ParamLayout& L, cons
 
 struct RegOnly { int layer; const float* x; float* y; long long xy_stride; };
 // The Regulation transformer and the head alone, over the X_in rows already in the workspace (the variants of
-// chromo_pcre_deletion); the fused Regulation kernel runs under the token classes of `plan` when it is set.
-struct RegReplay { const RaggedPlan* plan; };
+// chromo_pcre_deletion and chromo_pcre_subsets); the fused Regulation kernel runs under the token classes of `plan` when
+// it is set.  gene_batch: the row count of the gene pass the variants come from; every GEMM takes the path (tcgen05 or
+// FP32) the gene pass takes, so a variant is computed the way its gene is, whatever the number of variants.
+struct RegReplay { const RaggedPlan* plan; int gene_batch; };
 
 // The side stream of aux_fork: joined back into `st` by join(), or on leaving the scope when an error return comes first
 // (a fork left open invalidates a stream capture).
@@ -769,10 +773,10 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
     const bool train = w.training;
     const long long RS = w.res_stride;
     const bool bf16 = (flags & CHROMO_F_BF16) != 0;
-    // a replay over the S variants of each gene picks every path by the gene pass's row count (rows / S), so a gene's
-    // variants are computed the way the gene itself is
-    const int m_div = replay ? S : 1;
-    const bool proj_bf16 = bf16 && !train && T / m_div >= 64;
+    // a replay picks every path by the gene pass's row count (the rows of a variant GEMM are B or T = B * S, those of
+    // the gene pass's gene_batch or gene_batch * S), so the variants are computed the way their genes are
+    auto gene_rows = [&](long long M) -> long long { return replay ? M / B * replay->gene_batch : M; };
+    const bool proj_bf16 = bf16 && !train && gene_rows(T) >= 64;
     const bool fold = bf16 && !train;           // folded single-query attention weights (see pack_all_weights)      // q|k|v|gate handed to the attention kernel in BF16
     __nv_bfloat16* packed = bf16 ? reinterpret_cast<__nv_bfloat16*>(ws + w.bf_params) : nullptr;
     // Dense projection: tcgen05 BF16 engine when requested and the shape qualifies, FP32 SIMT otherwise.
@@ -781,7 +785,7 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
             // training: parameters change every step, so nothing is packed: FP32 weights are converted while staged
             return gemm_auto(g, true, true, nz, st, true);
         }
-        if (bf16 && g.M / m_div >= 64 && g.B >= P && g.B < P + L.total && umma_supported(g))
+        if (bf16 && gene_rows(g.M) >= 64 && g.B >= P && g.B < P + L.total && umma_supported(g))
             return umma_launch(g, packed + (g.B - P), nz, st);
         if (fold && g.B >= ws + w.fold_f32 && g.B < ws + w.fold_f32 + w.fold_total && umma_supported(g))
             return umma_launch(g, reinterpret_cast<const __nv_bfloat16*>(ws + w.fold_bf) + (g.B - (ws + w.fold_f32)), nz, st);
@@ -793,6 +797,7 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
     // precision diagnostics (tools/precision_stress.py): keep one stage's contractions on the FP32 CUDA-core GEMM
     const bool reg_fp32 = getenv("CHROMO_REG_FP32") != nullptr, head_fp32 = getenv("CHROMO_HEAD_FP32") != nullptr;
     auto lin_fp32 = [&](const GemmArgs& g, int nz) -> int { return gemm_launch(g, true, true, nz, st); };
+    if (w.reg_compact && reg_fp32) { set_error("CHROMO_REG_FP32 set after the replay workspace was sized"); return CHROMO_EINVAL; }
 
     RaggedPlan plan;                            // (ragged.cu; built next to the Embedding stage when the fused kernels run)
     bool ragged = false, reg_plan = false, reg_y_att = false;
@@ -1361,7 +1366,7 @@ extern "C" int chromo_pcre_deletion(const chromo_config_t* cfg, const float* par
         CHROMO_TRY(build_reg_plan(ra, ws + d.plan, &plan, st));
     }
     // the variants: Regulation transformer + head, with the weights the gene pass packed
-    const RegReplay replay{d.plan_on ? &plan : nullptr};
+    const RegReplay replay{d.plan_on ? &plan : nullptr, B};
     const int vflags = (flags & ~CHROMO_F_DENSE) | ((flags & CHROMO_F_BF16) ? CHROMO_F_PACKED : 0);
     CHROMO_TRY(forward_impl(cfg, params, &vin, ws + d.logits_v, ws, d.wv, vflags, st, nullptr, &replay));
     DeletionScatterArgs s;
@@ -1370,6 +1375,113 @@ extern "C" int chromo_pcre_deletion(const chromo_config_t* cfg, const float* par
     s.logits = logits; s.logits_v = ws + d.logits_v;
     s.without = without; s.promoter_only = promoter_only;
     return launch_deletion_scatter(s, st);
+}
+
+// ---- pCRE subsets (subsets.cu) ----
+// Workspace: the larger of the gene pass's layout and the replay layout of the V variants [0, front) (both start with
+// the same batch-independent front, the packed BF16 weights; the replay layout has no Embedding or Pairwise block), then
+// the gene X_in rows, the variants' freq and masks and the Regulation plan of the variants.
+namespace {
+struct SubsetsWs {
+    WsLayout wb, wv;
+    int64_t xin_b, freq_v, imask_v, plan, total;
+    bool plan_on;
+};
+int subsets_ws(const chromo_config_t* c, int batch, int variants, int flags, SubsetsWs* d) {
+    const int S = c->i_max + 1;
+    const int64_t row = std::max<int64_t>((int64_t)S * S, (int64_t)c->n_res * c->d_emb);
+    if ((int64_t)batch * row > INT32_MAX || (int64_t)variants * row > INT32_MAX) {
+        set_error("chromo_pcre_subsets: batch and variants times max((i_max + 1)^2, n_res * d_emb) must fit in int32");
+        return CHROMO_EINVAL;
+    }
+    const int V = variants;
+    d->wb = make_ws_layout(c, batch, flags);
+    d->wv = make_ws_layout(c, V, flags, true);
+    int64_t cur = std::max(d->wb.total, d->wv.total);
+    auto take = [&](int64_t n) { int64_t o = cur; cur = align4(cur + n); return o; };
+    d->xin_b = take((int64_t)c->n_res * batch * S * c->d_emb);
+    d->freq_v = take((int64_t)V * S * S);
+    d->imask_v = take(((int64_t)V * S * S + 3) / 4 * c->n_res);
+    d->plan_on = (flags & CHROMO_F_BF16) && d->wv.reg_fused;
+    d->plan = d->plan_on ? take(reg_plan_floats(V, c->i_max)) : 0;
+    d->total = cur;
+    return CHROMO_OK;
+}
+}  // namespace
+
+extern "C" int64_t chromo_pcre_subsets_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t variants,
+                                                        int32_t flags) {
+    if (validate_config(cfg) != CHROMO_OK) return CHROMO_EINVAL;
+    if (batch < 1 || variants < 1) { set_error("batch and variants must be >= 1"); return CHROMO_EINVAL; }
+    SubsetsWs d;
+    CHROMO_TRY(subsets_ws(cfg, batch, variants, flags, &d));
+    return d.total;
+}
+
+extern "C" int chromo_pcre_subsets(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                                   const int32_t* var_gene, const uint32_t* var_drop, int32_t variants, float* logits,
+                                   float* var_logits, float* workspace, int64_t workspace_floats, int32_t flags,
+                                   void* stream) {
+    CHROMO_TRY(check_forward_args(cfg, params, in, logits, workspace));
+    if (!var_gene || !var_drop || !var_logits) { set_error("chromo_pcre_subsets: null variant descriptor or output"); return CHROMO_EINVAL; }
+    if (variants < 1) { set_error("chromo_pcre_subsets: variants must be >= 1"); return CHROMO_EINVAL; }
+    if (flags & ~(CHROMO_F_BF16 | CHROMO_F_PACKED | CHROMO_F_DENSE)) {
+        set_error("chromo_pcre_subsets: inference only (flags CHROMO_F_BF16, CHROMO_F_PACKED, CHROMO_F_DENSE)");
+        return CHROMO_EINVAL;
+    }
+    SubsetsWs d;
+    CHROMO_TRY(subsets_ws(cfg, in->batch, variants, flags, &d));
+    if (workspace_floats < d.total) {
+        set_error("chromo_pcre_subsets: workspace too small: need %lld floats, got %lld", (long long)d.total,
+                  (long long)workspace_floats);
+        return CHROMO_ENOMEM;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    float* ws = workspace;
+    const int B = in->batch, I = cfg->i_max, S = I + 1, V = variants, NR = cfg->n_res, D = cfg->d_emb;
+    // the genes: the ordinary forward (it packs the BF16 weights unless CHROMO_F_PACKED), X_in left in the workspace
+    CHROMO_TRY(forward_impl(cfg, params, in, logits, ws, d.wb, flags, st));
+    // their X_in rows out of the way of the replay layout, which overlaps the gene layout
+    const size_t row_bytes = (size_t)B * S * D * sizeof(float);
+    if (cudaMemcpy2DAsync(ws + d.xin_b, row_bytes, ws + d.wb.r_xin, (size_t)d.wb.res_stride * sizeof(float), row_bytes, NR,
+                          cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
+        set_error("chromo_pcre_subsets: X_in copy failed");
+        return CHROMO_ECUDA;
+    }
+    chromo_batch_t vin;
+    memset(&vin, 0, sizeof(vin));
+    vin.batch = V; vin.freq = ws + d.freq_v;
+    {
+        SubsetExpandArgs a;
+        a.B = B; a.I = I; a.n_res = NR; a.V = V;
+        a.var_gene = var_gene; a.var_drop = var_drop;
+        a.xin = ws + d.xin_b; a.xin_z = (long long)B * S * D;
+        a.freq = in->freq;
+        a.xin_v = ws + d.wv.r_xin; a.xin_v_z = d.wv.res_stride;
+        a.freq_v = ws + d.freq_v;
+        for (int r = 0; r < NR; ++r) {
+            a.imask[r] = in->imask[r];
+            a.imask_v[r] = reinterpret_cast<uint8_t*>(ws + d.imask_v) + (long long)r * V * S * S;
+            vin.imask[r] = a.imask_v[r];
+        }
+        CHROMO_TRY(launch_subset_expand(a, st));
+    }
+    RaggedPlan plan;
+    if (d.plan_on) {
+        RaggedArgs ra;
+        memset(&ra, 0, sizeof(ra));
+        ra.B = V; ra.I = I; ra.n_res = NR;
+        for (int r = 0; r < NR; ++r) ra.imask[r] = vin.imask[r];
+        CHROMO_TRY(build_reg_plan(ra, ws + d.plan, &plan, st));
+    }
+    // the variants: Regulation transformer + head, with the weights the gene pass packed, logits in variant order
+    const RegReplay replay{d.plan_on ? &plan : nullptr, B};
+    const int vflags = (flags & ~CHROMO_F_DENSE) | ((flags & CHROMO_F_BF16) ? CHROMO_F_PACKED : 0);
+    CHROMO_TRY(forward_impl(cfg, params, &vin, var_logits, ws, d.wv, vflags, st, nullptr, &replay));
+    SubsetGuardArgs gd;
+    gd.B = B; gd.I = I; gd.V = V; gd.n_out = cfg->n_out;
+    gd.var_gene = var_gene; gd.var_drop = var_drop; gd.logits_v = var_logits;
+    return launch_subset_guard(gd, st);
 }
 
 extern "C" int chromo_regulation_layer(const chromo_config_t* cfg, const float* params, int32_t layer, const float* x,

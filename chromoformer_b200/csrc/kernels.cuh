@@ -111,6 +111,26 @@ struct DeletionScatterArgs {
 int launch_deletion_expand(const DeletionExpandArgs& a, cudaStream_t st);
 int launch_deletion_scatter(const DeletionScatterArgs& a, cudaStream_t st);
 
+// pCRE subsets (subsets.cu): B genes -> V variants of the Regulation stage, variant v = gene var_gene[v] without the live
+// slots of var_drop[v]
+struct SubsetExpandArgs {
+    int B, I, n_res, V;
+    const int* var_gene; const uint32_t* var_drop;  // [V]
+    const float* xin; long long xin_z;              // X_in of the genes [B*S, 128] per resolution
+    const uint8_t* imask[CHROMO_MAX_RES];           // [B,S,S]
+    const float* freq;                              // [B,S,S]
+    float* xin_v; long long xin_v_z;                // X_in of the variants [V*S, 128] per resolution
+    uint8_t* imask_v[CHROMO_MAX_RES];               // [V,S,S]
+    float* freq_v;                                  // [V,S,S]
+};
+struct SubsetGuardArgs {
+    int B, I, V, n_out;
+    const int* var_gene; const uint32_t* var_drop;  // [V]
+    float* logits_v;                                // [V, n_out]: NaN rows for out-of-range descriptors
+};
+int launch_subset_expand(const SubsetExpandArgs& a, cudaStream_t st);
+int launch_subset_guard(const SubsetGuardArgs& a, cudaStream_t st);
+
 int launch_reg_attention(const RegAttnArgs& a, int nz, cudaStream_t st);
 int launch_attn_rows(const AttnRowsArgs& a, cudaStream_t st);
 int single_query_attention(const SqaArgs& s, cudaStream_t st);

@@ -182,7 +182,7 @@ const ParamLayout& get_layout(const chromo_config_t* c) {
     return *L;
 }
 
-WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags) {
+WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags, bool replay) {
     WsLayout w;
     memset(&w, 0, sizeof(w));
     const int B = batch, I = c->i_max, S = I + 1, D = c->d_emb;
@@ -230,6 +230,7 @@ WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags) {
     }
     // ---- per-resolution block
     const int64_t res_base = cur;
+    if (!replay) {
     w.e_hc = take((int64_t)B * D);
     w.e_q = take((int64_t)B * c->embed_d_model);
     w.e_qk = take((int64_t)B * He * D);
@@ -261,8 +262,17 @@ WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags) {
         w.p_preU += s0; w.p_u += s0; w.p_f += s0; w.p_preY += s0; w.p_out += s0;
         cur = s0 + w.p_slot * w.pslots;
     }
+    }   // !replay
     w.r_xin = take((int64_t)T * D);
-    {
+    // a replay on the fused path (CHROMO_REG_FP32 sends the Regulation stage down the layer-by-layer path instead) needs
+    // the last layer's rows (token 0 is what the head reads) and the parking slots of the plan's tiles
+    w.reg_compact = replay && w.reg_fused && getenv("CHROMO_REG_FP32") == nullptr;
+    if (w.reg_compact) {
+        w.r_att = take((int64_t)T * D);
+        w.r_out = cur;
+        w.r_slot = align4((int64_t)ragged_reg_tiles_max(B, I) * 128 * D);
+        cur += w.r_slot * w.rslots;
+    } else {
         int64_t s0 = cur;
         w.r_proj = take((int64_t)T * 4 * c->reg_d_model);
         w.r_att = take((int64_t)T * c->reg_d_model);
@@ -282,7 +292,7 @@ WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags) {
     w.res_stride = cur - res_base;
     cur = res_base + w.res_stride * c->n_res;
     // ---- resolution-dependent buffers
-    for (int r = 0; r < c->n_res; ++r) {
+    for (int r = 0; r < c->n_res && !replay; ++r) {
         // rows may be padded to a multiple of 16 bins (tensor path for short rows, see single_query_attention)
         const int64_t n16 = (c->n_bins[r] + 15) / 16 * 16;
         w.e_p[r] = take((int64_t)B * He * n16);
@@ -291,7 +301,7 @@ WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags) {
     }
     w.h_z = take((int64_t)B * c->n_res * D);
     w.h_h1 = take((int64_t)B * c->d_head);
-    if (w.tail_fused) w.rg_plan = take(ragged_plan_floats(B, I, c->n_res));
+    if (w.tail_fused && !replay) w.rg_plan = take(ragged_plan_floats(B, I, c->n_res));
     w.g_base = cur;
     if (w.training) {
         // backward scratch, carved up in backward.cu: every gradient tensor of every layer has its own buffer (the

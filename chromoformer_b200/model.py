@@ -302,6 +302,7 @@ class _ChromoformerCore(nn.Module):
         object.__setattr__(self, "_table", None)
         object.__setattr__(self, "_packed_key", None)
         object.__setattr__(self, "_deletion_packed_key", None)
+        object.__setattr__(self, "_subsets_packed_key", None)
         object.__setattr__(self, "_param_epoch", 0)
         self._rebuild_flat()
 
@@ -359,6 +360,7 @@ class _ChromoformerCore(nn.Module):
         object.__setattr__(self, "_param_epoch", self._param_epoch + 1)
         object.__setattr__(self, "_packed_key", None)
         object.__setattr__(self, "_deletion_packed_key", None)
+        object.__setattr__(self, "_subsets_packed_key", None)
 
     def _flat_is_current(self):
         base = self._flat.data_ptr()
@@ -398,9 +400,10 @@ class _ChromoformerCore(nn.Module):
             self._pe_cache[key] = t
         return t
 
-    def _workspace(self, cfg, batch, flags, cached, entry="chromo_workspace_floats"):
+    def _workspace(self, cfg, batch, flags, cached, entry="chromo_workspace_floats", variants=None):
         lib = _lib.load()
-        n = _lib.check(getattr(lib, entry)(ctypes.byref(cfg), batch, flags), entry)
+        sizes = (batch,) if variants is None else (batch, variants)
+        n = _lib.check(getattr(lib, entry)(ctypes.byref(cfg), *sizes, flags), entry)
         if not cached:
             return torch.empty(n, dtype=torch.float32, device=self._flat.device)
         key = (str(self._flat.device), flags & ~_lib.F_DENSE)      # (the hint does not change the layout)
@@ -460,6 +463,34 @@ class _ChromoformerCore(nn.Module):
         if packed_key is not None:
             object.__setattr__(self, "_deletion_packed_key", packed_key)
         return logits, without, promoter_only
+
+    def _launch_subsets(self, io, var_gene, var_drop, flags):
+        """chromo_pcre_subsets: (logits [B, n_out], var_logits [V, n_out]) for the variant descriptors ``var_gene``
+        (int32 [V]) and ``var_drop`` (int32 [V], the bit pattern of the uint32 drop sets), both on the model's device.
+        Its workspace and packed BF16 weights are cached apart from the forward's and the deletion's."""
+        lib = _lib.load()
+        if not self._flat_is_current():
+            self._rebuild_flat()
+        dev, n_out = self._flat.device, int(self._cfg.n_out)
+        V = int(var_gene.numel())
+        if var_drop.numel() != V or var_gene.dtype != torch.int32 or var_drop.dtype != torch.int32:
+            raise ValueError("var_gene and var_drop must be int32 tensors of the same length")
+        var_gene, var_drop = var_gene.to(dev).contiguous(), var_drop.to(dev).contiguous()
+        ws = self._workspace(io.cfg, io.batch, flags, cached=True, entry="chromo_pcre_subsets_workspace_floats",
+                             variants=V)
+        packed_key = self._packed_key_of(ws, io, flags)
+        if packed_key is not None and packed_key == self._subsets_packed_key:
+            flags |= _lib.F_PACKED
+        logits = torch.empty(io.batch, n_out, dtype=torch.float32, device=dev)
+        var_logits = torch.empty(V, n_out, dtype=torch.float32, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(lib.chromo_pcre_subsets(ctypes.byref(io.cfg), self._flat.data_ptr(), ctypes.byref(io.struct),
+                                           var_gene.data_ptr(), var_drop.data_ptr(), V, logits.data_ptr(),
+                                           var_logits.data_ptr(), ws.data_ptr(), ws.numel(), flags, stream),
+                   "chromo_pcre_subsets")
+        if packed_key is not None:
+            object.__setattr__(self, "_subsets_packed_key", packed_key)
+        return logits, var_logits
 
     def _launch_backward(self, io, ws, dlogits, want_dx=None):
         """Parameter gradients into ``p.grad`` (chromo_backward).  ``want_dx``: one flag per input tensor (every x_p,

@@ -135,6 +135,32 @@ int chromo_pcre_deletion(const chromo_config_t* cfg, const float* params, const 
                          float* promoter_only /* [B,n_out] */, float* workspace, int64_t workspace_floats,
                          int32_t flags, void* stream);
 
+/* ---- pCRE subsets: the logits of each gene without an arbitrary set of its pCREs --------------------------------
+ * For B genes with I = i_max slots (S = I + 1 tokens) and V variants.  Variant v is gene var_gene[v] without the pCREs
+ * of the bit set var_drop[v] (bit i: slot i; a dead slot, as defined for chromo_pcre_deletion, is no pCRE, so its bit
+ * changes nothing):
+ *   logits[g]          the ordinary forward, bit-identical to chromo_forward with the same flags;
+ *   var_logits[v]      the logits with row and column i + 1 of every resolution's interaction mask set for every live
+ *                      slot i of var_drop[v], which is the gene reassembled without those pCREs; an empty set gives the
+ *                      gene itself, the set of every live slot the promoter alone.
+ * One Embedding + Pairwise pass per gene serves all its variants; the Regulation transformer and the head then run over
+ * the V variants, each listing the tokens it keeps first, so that the BF16 path's ragged plan packs a variant that keeps
+ * m live pCREs into token class m + 1.  Every GEMM takes the path the gene pass takes for the same B genes, so a
+ * variant's logits do not depend on V or on the other variants.  The descriptors (device memory) are checked on the
+ * device: a variant with var_gene[v] outside [0, B) or a bit at or above I reads no gene and gets a NaN row in
+ * var_logits; the other rows are unaffected.  No atomics on the floating-point path; identical inputs give identical
+ * outputs; no host synchronisation (legal inside a stream capture).  Flags: CHROMO_F_BF16, CHROMO_F_PACKED (as for
+ * chromo_forward) and the CHROMO_F_DENSE hint (the gene pass only); any other flag, a NULL descriptor or output, or
+ * variants < 1 is CHROMO_EINVAL.  The workspace must hold chromo_pcre_subsets_workspace_floats floats (CHROMO_ENOMEM
+ * otherwise); it keeps the packed BF16 weights at its front, as a chromo_forward workspace does.  With CHROMO_F_BF16 and
+ * the default configuration it grows by about 58 kB per variant (the replay needs X_in, the last Regulation layer's
+ * rows and the fused kernel's parking rows, not the Embedding / Pairwise buffers); FP32 by about 0.5 MB.            */
+int64_t chromo_pcre_subsets_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t variants, int32_t flags);
+int chromo_pcre_subsets(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                        const int32_t* var_gene /* [V] device */, const uint32_t* var_drop /* [V] device */,
+                        int32_t variants, float* logits /* [B,n_out] */, float* var_logits /* [V,n_out] */,
+                        float* workspace, int64_t workspace_floats, int32_t flags, void* stream);
+
 /* ---- one Regulation-transformer layer: AttentionBlock with gate (modules.py:104-111 as used by
  * net.py:152-153), for every resolution at once: y[r] = layer(x[r]), x/y = [n_res][B*(i_max+1), d_emb] FP32
  * with `xy_stride` floats between resolutions.  With CHROMO_F_BF16 and the default geometry this is ONE
