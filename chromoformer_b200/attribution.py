@@ -10,7 +10,9 @@ they do not require grad during the call, and nothing is written to ``p.grad``. 
 ``pcre_scores`` folds a result into one score per pCRE slot.  These are local (gradient) or path (integrated gradients)
 approximations; ``pcre_deletion`` gives the exact counterfactual per pCRE: the prediction with that pCRE removed.
 ``pcre_subsets`` gives the prediction without any set of pCREs, and on top of it ``pcre_shapley`` (credit per pCRE that
-sums to logits - promoter only) and ``pcre_interactions`` (the synergy of every pair of pCREs).
+sums to logits - promoter only) and ``pcre_interactions`` (the synergy of every pair of pCREs).  ``pcre_occlusion`` and
+``occlusion_map`` give the exact counterpart of the saliency maps: the prediction with histone marks removed over a
+window of bins.
 """
 import contextlib
 import math
@@ -22,7 +24,7 @@ from . import _lib
 from .model import _BatchIO
 
 __all__ = ["input_gradients", "integrated_gradients", "pcre_scores", "pcre_deletion", "pcre_subsets", "pcre_shapley",
-           "pcre_interactions"]
+           "pcre_interactions", "pcre_occlusion", "occlusion_map"]
 
 _FEATS = ("promoter_feats", "pcre_feats")
 _MASKS = ("promoter_pad_masks", "pcre_pad_masks")
@@ -479,3 +481,220 @@ def pcre_interactions(model, batch, target=None, chunk=_SUBSET_CHUNK, dense=Fals
     inter, effect = _interactions(v[:, 0], v[:, 1:1 + I], v[:, 1 + I:], pairs, live)
     dev = logits.device
     return {"interaction": inter.to(dev), "effect": effect.to(dev), "logits": logits}
+
+
+# ---- histone-mark occlusion (chromo_pcre_occlusion) ----------------------------------------------------------------
+_OCCLUSION_CHUNK = 65536        # variants per library call: about 4.5 GB of workspace in BF16, 31 GB in FP32 (DESIGN.md 3.6)
+_FORWARD_CHUNK = 8192           # genes per forward_batch call of the promoter windows
+_INT32_MAX = 2 ** 31 - 1
+
+
+def _int32(a, bad):
+    """int64 numpy -> int32, every value outside int32 replaced by ``bad`` (so that it stays invalid on the device)."""
+    a = np.asarray(a, dtype=np.int64)
+    return np.where((a < -_INT32_MAX - 1) | (a > _INT32_MAX), bad, a).astype(np.int32)
+
+
+def _mark_bits(marks, V, F):
+    """Mark sets as uint32 bit patterns in int32 [V]: from bool [V, F] or from integers (bit m: mark m)."""
+    m = torch.as_tensor(marks)
+    if m.dtype == torch.bool:
+        if m.dim() != 2 or m.shape != (V, F):
+            raise ValueError(f"bool marks must be [{V}, {F}], got {tuple(m.shape)}")
+        bits = (m.cpu().long() << torch.arange(F)).sum(-1).numpy()
+    else:
+        bits = m.cpu().long().reshape(-1).numpy()
+        if bits.shape[0] != V:
+            raise ValueError(f"marks must hold {V} mark sets, got {bits.shape[0]}")
+        bits = np.where((bits < 0) | (bits > 0xFFFFFFFF), 0xFFFFFFFF, bits)     # (out of range: invalid on the device)
+    return bits.astype(np.uint32).view(np.int32)
+
+
+def _occlude(model, dev_batch, bins, gene, slot, var_bins, marks, chunk, dense):
+    """logits [B, n_out] and var_logits [V, n_out] (descriptor order) on the device from numpy descriptors (gene, slot
+    int64 [V], var_bins int64 [V, n_res, 2], marks int32 [V]).  One library call covers whole genes, at most ``chunk``
+    variants (a gene with more gets a call of its own), so every gene's Embedding / Pairwise pass runs once.  Descriptors
+    of a gene outside [0, B) stay invalid (NaN rows): they go to calls of their own, at most ``chunk`` per call, each over
+    gene 0 alone (whose logits there are discarded)."""
+    if chunk < 1:
+        raise ValueError("chunk must be >= 1")
+    B = int(dev_batch[_FREQ].shape[0])
+    V = int(gene.shape[0])
+    ok = (gene >= 0) & (gene < B)
+    bad = np.nonzero(~ok)[0]
+    good = np.nonzero(ok)[0]
+    order = good[np.argsort(gene[good], kind="stable")]       # the valid descriptors by gene, stable
+    starts = np.concatenate([[0], np.cumsum(np.bincount(gene[good], minlength=B))])
+    flags = model._precision_flag() | (_lib.F_DENSE if dense else 0)
+    dev = model.flat_params.device
+    n_out = int(model._cfg.n_out)
+    logits, var_logits = [], torch.empty(V, n_out, dtype=torch.float32, device=dev)
+
+    def call(g0, g1, idx, vg):
+        io = _BatchIO(model, *[[dev_batch[k][b][g0:g1] for b in bins] for k in _GENE_KEYS], dev_batch[_FREQ][g0:g1])
+        if idx.size:
+            vs, vb, vm = slot[idx], var_bins[idx], marks[idx]
+        else:                                                   # genes without variants: one invalid one, discarded
+            vg, vs = np.full(1, -1), np.zeros(1, dtype=np.int64)
+            vb, vm = np.zeros((1,) + var_bins.shape[1:], dtype=np.int64), np.zeros(1, dtype=np.int32)
+        desc = [torch.from_numpy(a).to(dev) for a in (_int32(vg, -1), _int32(vs, -1), _int32(vb, -1), vm)]
+        lg, vl = model._launch_occlusion(io, *desc, flags)
+        if idx.size:
+            var_logits[torch.from_numpy(idx).to(dev)] = vl
+        return lg
+
+    with torch.no_grad():
+        for v0 in range(0, len(bad), chunk):
+            idx = bad[v0:v0 + chunk]
+            call(0, 1, idx, np.full(len(idx), -1))
+        g0 = 0
+        while g0 < B:
+            g1 = int(np.searchsorted(starts, starts[g0] + chunk, side="right")) - 1
+            g1 = min(B, max(g1, g0 + 1))
+            idx = order[starts[g0]:starts[g1]]
+            logits.append(call(g0, g1, idx, gene[idx] - g0))
+            g0 = g1
+    return torch.cat(logits), var_logits
+
+
+def pcre_occlusion(model, batch, gene, slot, bins, marks, target=None, chunk=_OCCLUSION_CHUNK, dense=False):
+    """The exact logits of genes with histone marks removed over bin ranges of one pCRE (``chromo_pcre_occlusion``).
+    Variant v is gene ``gene[v]`` with
+
+        pcre_feats[r][gene[v], slot[v], bins[v, r, 0]:bins[v, r, 1], m] = 0     for every resolution r, every m in marks[v]
+
+    (r in the order of ``model.binsizes``); the masks and interaction_freq stay as they are.  Zero is what the input
+    path writes where no read fell (ln(0 + 1)), so a variant is the gene as if those marks had no reads there.  An empty
+    range leaves that resolution alone.  ``gene``, ``slot``: ints [V]; ``bins``: ints [V, n_res, 2]; ``marks``: bool
+    [V, n_feats] or integer bit sets [V] (bit m: mark m).  A dead slot (no pCRE, see ``pcre_deletion``) gives the gene's
+    logits exactly; an invalid descriptor (gene or slot out of range, a range with lo < 0, lo > hi or hi > n_r, a mark
+    at or above n_feats) gives a NaN row and leaves the others alone.  Returns
+
+        "logits"    [B, n_out]   the ordinary forward (bit-identical to ``forward_batch`` with the same ``dense``)
+        "variants"  [V, n_out]   the logits of each variant, in descriptor order
+        "value"     [V]          variants[:, target], only when ``target`` is given
+
+    One Embedding / Pairwise pass per gene, one Pairwise pass over the occluded region per variant, and the Regulation
+    transformer and the head over the variants.  At most ``chunk`` variants go to one library call, whole genes at a
+    time; descriptors of a gene out of range go to calls of their own.  A variant's logits do not depend on the other
+    variants of its call (every occluded region is computed on its own, on the GEMM paths of its gene's pass), nor on
+    ``chunk`` as long as every call's gene count B keeps B, B * I and B * (I + 1) on the same side of 64 and, in BF16
+    without ``dense``, B * I on the same side of the 897 rows (113 genes at I = 8) from which the gene pass builds its
+    ragged plan (a forward's results depend on the same thresholds).  With that plan the gene's own rows come from
+    shared key windows, so an empty occlusion matches ``logits`` to BF16 rounding, not bit for bit.  Nothing requires
+    grad, nothing touches ``p.grad``."""
+    binsizes = list(model.binsizes)
+    dev_batch = _to_device(batch, model, binsizes)
+    F, NR = int(model._cfg.n_feats), len(binsizes)
+    gene = np.asarray(torch.as_tensor(gene).cpu().long().reshape(-1).numpy())
+    V = int(gene.shape[0])
+    if V < 1:
+        raise ValueError("at least one variant is needed")
+    slot = torch.as_tensor(slot).cpu().long().reshape(-1).numpy()
+    var_bins = torch.as_tensor(bins).cpu().long().numpy()
+    if slot.shape[0] != V or var_bins.shape != (V, NR, 2):
+        raise ValueError(f"slot must be [{V}] and bins [{V}, {NR}, 2], got {slot.shape} and {var_bins.shape}")
+    logits, var_logits = _occlude(model, dev_batch, binsizes, gene, slot, var_bins, _mark_bits(marks, V, F), chunk, dense)
+    out = {"logits": logits, "variants": var_logits}
+    if target is not None:
+        out["value"] = var_logits[:, _default_target(model, target)]
+    return out
+
+
+def _mark_sets(marks, F):
+    """bool [M, F] mark sets from "all", "each" or a bool [M, F] list."""
+    if isinstance(marks, str):
+        if marks == "all":
+            return torch.ones(1, F, dtype=torch.bool)
+        if marks == "each":
+            return torch.eye(F, dtype=torch.bool)
+        raise ValueError('marks must be "all", "each" or a bool [M, n_feats] list of mark sets')
+    m = torch.as_tensor(marks)
+    if m.dtype != torch.bool or m.dim() != 2 or m.shape[1] != F or m.shape[0] < 1:
+        raise ValueError(f"mark sets must be bool [M, {F}], got {tuple(m.shape)} {m.dtype}")
+    return m.cpu()
+
+
+def occlusion_map(model, batch, window=1, stride=None, marks="all", target=None, chunk=_OCCLUSION_CHUNK, dense=False):
+    """Occlusion map of every region of every gene: the logits with the marks of each mark set removed over each genomic
+    window, for the promoter and for every pCRE slot.
+
+    Windows are ``[w0, w0 + window)`` for w0 = 0, stride, 2 stride, ... (``stride`` defaults to ``window``) in units of the
+    coarsest bin (n_0 bins per region, the smallest n_r); at resolution r the window covers the bins
+    ``[w0 n_r / n_0, (w0 + window) n_r / n_0)``, which needs n_0 to divide every n_r (20 / 80 / 400 for 2 kb / 500 bp /
+    100 bp bins).  For a region without centre padding that is exactly the gene with the reads of that genomic interval
+    removed before binning; for a padded region (shorter than the window of w_max, centred by data.py) it is a window in
+    bin space, and bins under the pad mask carry no information, so occluding only those changes nothing.
+    ``marks``: "all" (one set of every mark), "each" (one set per mark) or bool [M, n_feats].  Returns
+
+        "pcre"             [B, I, W, M, n_out]  logits with pCRE slot i occluded (``pcre_occlusion``); on a dummy slot
+                                                the logits themselves
+        "promoter"         [B, W, M, n_out]     logits with the promoter occluded
+        "effect_pcre"      [B, I, W, M]         logits[:, target] - pcre[..., target]; exactly 0.0 on dummy slots
+        "effect_promoter"  [B, W, M]            logits[:, target] - promoter[..., target]
+        "logits"           [B, n_out]           the ordinary forward
+        "windows"          [W, 2]               the windows, in coarsest-bin units
+
+    The pCRE variants replay one Pairwise region each plus the Regulation transformer (``pcre_occlusion``; dummy slots
+    are not replayed).  Promoter windows cannot take that route: the promoter's Embedding row is the query of every
+    Pairwise layer of its resolution, so occluding promoter bins changes every token of the gene, and such a variant is
+    a full forward: those genes are built on the device, occluded, and run through ``forward_batch``, a window and
+    mark set at a time.  Occlusion is not additive: the single-mark maps of "each" need not sum to the map of "all".
+    ``target`` defaults to column 1 for the classifier and 0 for the regressor.  Nothing requires grad."""
+    binsizes = list(model.binsizes)
+    t = _default_target(model, target)
+    dev_batch = _to_device(batch, model, binsizes)
+    F = int(model._cfg.n_feats)
+    n = [int(dev_batch["pcre_feats"][b].shape[2]) for b in binsizes]
+    n0 = min(n)
+    if any(nr % n0 for nr in n):
+        raise ValueError(f"the coarsest resolution's {n0} bins must divide every resolution's bins {n}")
+    window = int(window)
+    stride = window if stride is None else int(stride)
+    if window < 1 or stride < 1 or window > n0:
+        raise ValueError(f"window must be in [1, {n0}] and stride >= 1")
+    w0 = np.arange(0, n0 - window + 1, stride)
+    windows = np.stack([w0, w0 + window], 1)                             # [W, 2]
+    sets = _mark_sets(marks, F)                                         # [M, F]
+    W, M = len(w0), int(sets.shape[0])
+    bits = (sets.long() << torch.arange(F)).sum(-1).numpy()             # [M]
+    B, S = (int(x) for x in dev_batch[_FREQ].shape[:2])
+    I = S - 1
+    live = _live(dev_batch, binsizes).cpu().numpy()                     # (the host read of the call)
+    rb = np.stack([windows * (nr // n0) for nr in n], 1)                # [W, n_res, 2]
+    g, i = np.nonzero(live)                                             # live slots, gene-major
+    K = len(g)
+    gene = np.repeat(g, W * M)
+    slot = np.repeat(i, W * M)
+    var_bins = np.tile(np.repeat(rb, M, axis=0), (K, 1, 1))             # [(K W M), n_res, 2]
+    vmarks = np.tile(bits, K * W).astype(np.uint32).view(np.int32)
+    if K:
+        logits, vl = _occlude(model, dev_batch, binsizes, gene, slot, var_bins, vmarks, chunk, dense)
+    else:
+        logits, vl = _occlude(model, dev_batch, binsizes, np.full(1, -1), np.zeros(1, dtype=np.int64),
+                              np.zeros((1, len(n), 2), dtype=np.int64), np.zeros(1, dtype=np.int32), chunk, dense)
+        vl = vl[:0]
+    n_out = logits.shape[1]
+    pcre = logits.view(B, 1, 1, 1, n_out).expand(B, I, W, M, n_out).clone()
+    live_t = torch.from_numpy(live).to(logits.device)
+    pcre[live_t] = vl.view(K, W, M, n_out)
+    promoter = torch.empty(B, W, M, n_out, dtype=torch.float32, device=logits.device)
+    with torch.no_grad():
+        for w in range(W):
+            for m in range(M):
+                feats = {}
+                for r, b in enumerate(binsizes):
+                    x = dev_batch["promoter_feats"][b].clone()
+                    lo, hi = (int(v) for v in rb[w, r])
+                    x[..., lo:hi, sets[m].to(x.device)] = 0
+                    feats[b] = x
+                for g0 in range(0, B, _FORWARD_CHUNK):
+                    g1 = min(B, g0 + _FORWARD_CHUNK)
+                    sub = {k: {b: dev_batch[k][b][g0:g1] for b in binsizes} for k in _GENE_KEYS}
+                    sub["promoter_feats"] = {b: feats[b][g0:g1] for b in binsizes}
+                    sub[_FREQ] = dev_batch[_FREQ][g0:g1]
+                    promoter[g0:g1, w, m] = model.forward_batch(sub, dense=dense)
+    return {"pcre": pcre, "promoter": promoter,
+            "effect_pcre": logits[:, t].view(B, 1, 1, 1) - pcre[..., t],
+            "effect_promoter": logits[:, t].view(B, 1, 1) - promoter[..., t],
+            "logits": logits, "windows": torch.from_numpy(windows)}

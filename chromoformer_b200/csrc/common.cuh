@@ -134,7 +134,10 @@ struct WsLayout {
 // replay: the layout of a Regulation + head replay over `batch` variants (chromo_pcre_subsets): the same batch-independent
 // front (the packed BF16 weights), X_in, the Regulation buffers and the head, no Embedding or Pairwise block.  On the fused
 // BF16 path the Regulation buffers are the parking rows r_out and the last-layer rows r_att alone.
-WsLayout make_ws_layout(const chromo_config_t* cfg, int batch, int flags, bool replay = false);
+// pairwise: the layout of a Pairwise replay over `batch` pseudo-genes of ONE pCRE slot each (chromo_pcre_occlusion): the
+// same front, then the Pairwise buffers alone (no Embedding, X_in, Regulation or head block; the pass reads and writes
+// an X_in the caller places).  The front is that of `cfg` itself, so the packed weights of a gene pass stay valid.
+WsLayout make_ws_layout(const chromo_config_t* cfg, int batch, int flags, bool replay = false, bool pairwise = false);
 
 static inline int64_t align4(int64_t x) { return (x + 3) & ~int64_t(3); }
 

@@ -592,7 +592,8 @@ int single_query_attention(const SqaArgs& s, cudaStream_t st) {
     // Short rows (n <= 32).  BF16 inference: pad the row to 32 bins (the packed position tables carry zero rows /
     // columns there) so that both position-table GEMMs run on the tensor pipe; otherwise the rows kernel does
     // them itself (attn_rows_reg_kernel<.., FUSE_PE>).
-    const bool pad32 = s.pe_pk && s.folded && s.n <= 32 && s.rows * s.H >= 64;
+    const long long path_rows = (s.path_rows ? s.path_rows : s.rows) * s.H;     // the row count that picks the paths
+    const bool pad32 = s.pe_pk && s.folded && s.n <= 32 && path_rows >= 64;
     const int np = pad32 ? 32 : s.n;                       // row stride / GEMM extent of the P buffer
     const bool fuse_pe = !pad32 && s.H == 2 && s.F == 7 && D == 128 && s.n <= 32;
     // Spe[(row,h), j] = QK[(row,h), :] . PE[j, :]                          (NT GEMM vs the table)
@@ -602,7 +603,7 @@ int single_query_attention(const SqaArgs& s, cudaStream_t st) {
         g.B = s.pe; g.ldb = D;
         g.C = s.P; g.ldc = np;
         g.M = s.rows * s.H; g.N = np; g.K = D;
-        if (s.pe_pk && g.M >= 64 && np % 16 == 0 && umma_supported(g)) CHROMO_TRY(umma_launch(g, s.pe_pk, 1, st));
+        if (s.pe_pk && path_rows >= 64 && np % 16 == 0 && umma_supported(g)) CHROMO_TRY(umma_launch(g, s.pe_pk, 1, st));
         else if (pad32) { set_error("internal: padded short-row path needs the tensor engine"); return CHROMO_EINVAL; }
         else CHROMO_TRY(gemm_auto(g, true, true, 1, st, s.tc));
     }
@@ -622,7 +623,7 @@ int single_query_attention(const SqaArgs& s, cudaStream_t st) {
         g.B = s.pe; g.ldb = D;
         g.C = s.cbar; g.ldc = D; g.accumulate = 1;
         g.M = s.rows * s.H; g.N = D; g.K = np;
-        if (s.pet_pk && g.M >= 64 && np % 16 == 0 && umma_supported(g)) CHROMO_TRY(umma_launch(g, s.pet_pk, 1, st));
+        if (s.pet_pk && path_rows >= 64 && np % 16 == 0 && umma_supported(g)) CHROMO_TRY(umma_launch(g, s.pet_pk, 1, st));
         else if (pad32) { set_error("internal: padded short-row path needs the tensor engine"); return CHROMO_EINVAL; }
         else CHROMO_TRY(gemm_auto(g, true, false, 1, st, s.tc));   // (no split-K here: the forward stays deterministic)
     }
@@ -755,6 +756,15 @@ struct RegOnly { int layer; const float* x; float* y; long long xy_stride; };
 // it is set.  gene_batch: the row count of the gene pass the variants come from; every GEMM takes the path (tcgen05 or
 // FP32) the gene pass takes, so a variant is computed the way its gene is, whatever the number of variants.
 struct RegReplay { const RaggedPlan* plan; int gene_batch; };
+// The Pairwise stage alone over pseudo-genes of one pCRE slot each (the occluded regions of chromo_pcre_occlusion), on a
+// make_ws_layout(..., pairwise = true) layout: the PP GEMM reads token 0 of the X_in at `xin` (resolution stride xin_z,
+// [B * 2, 128]) and the last layer writes token 1 there; no Embedding, Regulation or head.  Every GEMM takes the path
+// the gene pass of gene_batch genes with gene_slots slots takes (its PP GEMM has gene_batch rows, its Pairwise GEMMs
+// gene_batch * gene_slots), so an occluded region takes the GEMM paths its gene's region took, whatever the number of
+// pseudo-genes.  (The path choice, not the bits: a gene pass under the ragged plan computed its regions over key windows
+// shared by a tile.)  No ragged plan here: every region walks the whole position table, so its rows do not depend on
+// the others.
+struct PwReplay { int gene_batch, gene_slots; float* xin; long long xin_z; };
 
 // The side stream of aux_fork: joined back into `st` by join(), or on leaving the scope when an error return comes first
 // (a fork left open invalidates a stream capture).
@@ -766,7 +776,7 @@ struct AuxStream {
 
 static int forward_impl(const chromo_config_t* c, const float* P, const chromo_batch_t* in, float* logits,
                         float* ws, const WsLayout& w, int flags, cudaStream_t st, const RegOnly* only = nullptr,
-                        const RegReplay* replay = nullptr) {
+                        const RegReplay* replay = nullptr, const PwReplay* pw = nullptr) {
     const ParamLayout& L = get_layout(c);
     const int B = w.B, I = w.I, S = w.S, R = w.R, T = w.T, D = w.D, F = c->n_feats;
     const int NR = c->n_res;
@@ -775,17 +785,20 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
     const bool bf16 = (flags & CHROMO_F_BF16) != 0;
     // a replay picks every path by the gene pass's row count (the rows of a variant GEMM are B or T = B * S, those of
     // the gene pass's gene_batch or gene_batch * S), so the variants are computed the way their genes are
-    auto gene_rows = [&](long long M) -> long long { return replay ? M / B * replay->gene_batch : M; };
+    auto gene_rows = [&](long long M) -> long long {
+        return replay ? M / B * replay->gene_batch : pw ? M / B * pw->gene_batch * pw->gene_slots : M;
+    };
     const bool proj_bf16 = bf16 && !train && gene_rows(T) >= 64;
     const bool fold = bf16 && !train;           // folded single-query attention weights (see pack_all_weights)      // q|k|v|gate handed to the attention kernel in BF16
     __nv_bfloat16* packed = bf16 ? reinterpret_cast<__nv_bfloat16*>(ws + w.bf_params) : nullptr;
     // Dense projection: tcgen05 BF16 engine when requested and the shape qualifies, FP32 SIMT otherwise.
-    auto lin = [&](const GemmArgs& g, int nz) -> int {
+    // (path_rows: the gene pass's row count when gene_rows cannot tell it from g.M)
+    auto lin = [&](const GemmArgs& g, int nz, long long path_rows = -1) -> int {
         if (bf16 && train) {
             // training: parameters change every step, so nothing is packed: FP32 weights are converted while staged
             return gemm_auto(g, true, true, nz, st, true);
         }
-        if (bf16 && gene_rows(g.M) >= 64 && g.B >= P && g.B < P + L.total && umma_supported(g))
+        if (bf16 && (path_rows >= 0 ? path_rows : gene_rows(g.M)) >= 64 && g.B >= P && g.B < P + L.total && umma_supported(g))
             return umma_launch(g, packed + (g.B - P), nz, st);
         if (fold && g.B >= ws + w.fold_f32 && g.B < ws + w.fold_f32 + w.fold_total && umma_supported(g))
             return umma_launch(g, reinterpret_cast<const __nv_bfloat16*>(ws + w.fold_bf) + (g.B - (ws + w.fold_f32)), nz, st);
@@ -803,7 +816,7 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
     bool ragged = false, reg_plan = false, reg_y_att = false;
     if (!only && !replay) {
     // ---------------- Embedding transformer, centre query (net.py:31-59) ----
-    {
+    if (!pw) {
         CentreEmbedArgs a;
         a.B = B; a.D = D; a.F = F;
         for (int r = 0; r < NR; ++r) { a.x[r] = in->x_p[r]; a.pe[r] = in->pos_enc[r]; a.n[r] = c->n_bins[r]; }
@@ -895,6 +908,8 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
             ragged = true;
         }
     }
+    const long long tail_z = (long long)(1 + c->pw_layers) * TAIL_SLOT_ELEMS;
+    if (!pw) {      // (a Pairwise replay has its token 0 rows already)
     bool e_fused = false, e_tiles = false;
     CHROMO_TRY(sqa_fused(B, c->embed_heads, in->x_p, in->mask_p, in->mask_p_stride, in->mask_p_row_offset,
                          L.embed[0].lin_proj, L.embed_stride, 0, dme, ws + w.e_qk, ws + w.e_qkt, ws + w.e_cbar, cb16, true, false,
@@ -936,7 +951,6 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
         CHROMO_TRY(single_query_attention(s, ers.s[r]));
     }
     if (!e_fused) CHROMO_TRY(res_join(ers));
-    const long long tail_z = (long long)(1 + c->pw_layers) * TAIL_SLOT_ELEMS;
     if (tail) {   // out-projection + LN + FFN + LN in one launch (row_tail_fused.cu) -> X_in[b, 0, :]
         RowTailArgs t;
         t.M = B; t.dff = c->embed_d_ff;
@@ -987,16 +1001,19 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
         CHROMO_TRY(lin(g, NR));
     }
     }   // !tail
+    }   // !pw
 
     // ---------------- Pairwise Interaction transformer (net.py:105-139) -----
     const int dmp = c->pw_d_model, Hp = c->pw_heads;
+    float* const xin = pw ? pw->xin : ws + w.r_xin;       // token 0 in, the pCRE tokens out
+    const long long xin_z = pw ? pw->xin_z : RS;
     {   // PP = Y_c W_lpp^T   (identical for the I slots of a gene, net.py:114-118)
         GemmArgs g = gemm_args();
-        g.A = ws + w.r_xin; g.lda = S * D; g.sA1 = RS;
+        g.A = xin; g.lda = S * D; g.sA1 = xin_z;
         g.B = P + L.pw[0].lin_proj_p; g.ldb = D; g.sB1 = L.pw_stride;
         g.C = ws + w.p_pp; g.ldc = D; g.sC1 = RS;
         g.M = B; g.N = D; g.K = D;
-        CHROMO_TRY(lin(g, NR));
+        CHROMO_TRY(lin(g, NR, pw ? pw->gene_batch : -1));
     }
     if (ragged) {
         CHROMO_TRY(build_ragged_plan(ra, ws + w.rg_plan, &plan, plan_stream.aux));
@@ -1048,6 +1065,7 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
             s.P = ws + w.p_p[r] + (long long)w.pslot(l) * w.p_p_slot[r];
             s.xbar = ws + r * RS + w.p_xbar + so;
             s.cbar = ws + r * RS + w.p_cbar + so; s.av = ws + r * RS + w.p_av + so; s.folded = fold; s.tc = bf16 && train;
+            s.path_rows = gene_rows(R);
             CHROMO_TRY(single_query_attention(s, prs.s[r]));
         }
         if (!p_fused) CHROMO_TRY(res_join(prs));
@@ -1057,9 +1075,9 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
             t.a = ws + w.p_cbar + so; t.lda = Hp * D; t.a_z = RS;
             if (p_fused && cb16) t.a_bf16 = reinterpret_cast<const __nv_bfloat16*>(ws + w.p_cbar + so);
             t.res = pin; t.res_div = pin_div; t.res_z = RS;
-            if (last) { t.y = ws + w.r_xin; t.c_div = I; t.c_mul = S; t.c_add = 1; }
+            if (last) { t.y = xin; t.c_div = I; t.c_mul = S; t.c_add = 1; }
             else { t.y = ws + w.p_out + so; t.c_div = 1; t.c_mul = 1; t.c_add = 0; }
-            t.y_z = RS;
+            t.y_z = last ? xin_z : RS;
             t.wstream = reinterpret_cast<const __nv_bfloat16*>(ws + w.tail_stream) + (1 + l) * TAIL_SLOT_ELEMS; t.w_z = tail_z;
             t.bo = P + pa.ffb; t.ln1w = P + pa.lnw; t.ln1b = P + pa.lnb; t.b1 = P + pf.l1b; t.b2 = P + pf.l2b;
             t.ln2w = P + pf.lnw; t.ln2b = P + pf.lnb; t.p_z = L.pw_stride;
@@ -1096,9 +1114,9 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
             GemmArgs g = gemm_args();
             g.A = ws + w.p_f + so; g.lda = c->pw_d_ff; g.sA1 = RS;
             g.B = P + pf.l2w; g.ldb = c->pw_d_ff; g.sB1 = L.pw_stride;
-            if (last) { g.C = ws + w.r_xin; g.c_div = I; g.c_mul = S; g.c_add = 1; }
+            if (last) { g.C = xin; g.c_div = I; g.c_mul = S; g.c_add = 1; }
             else g.C = ws + w.p_out + so;
-            g.ldc = D; g.sC1 = RS;
+            g.ldc = D; g.sC1 = last ? xin_z : RS;
             g.M = R; g.N = D; g.K = c->pw_d_ff;
             g.epi = EPI_BIAS_RES_LN; g.bias = P + pf.l2b; g.sBias1 = L.pw_stride;
             g.res = ws + w.p_u + so; g.ldres = D; g.sRes1 = RS;
@@ -1108,6 +1126,7 @@ static int forward_impl(const chromo_config_t* c, const float* P, const chromo_b
         }
     }
 
+    if (pw) return CHROMO_OK;
     }   // !only && !replay
     // ---------------- Regulation transformer (net.py:152-153) ---------------
     const int dmr = c->reg_d_model, Hr = c->reg_heads;
@@ -1482,6 +1501,172 @@ extern "C" int chromo_pcre_subsets(const chromo_config_t* cfg, const float* para
     gd.B = B; gd.I = I; gd.V = V; gd.n_out = cfg->n_out;
     gd.var_gene = var_gene; gd.var_drop = var_drop; gd.logits_v = var_logits;
     return launch_subset_guard(gd, st);
+}
+
+// ---- histone-mark occlusion (occlusion.cu) ----
+// Workspace, three phases on one front (the packed BF16 weights the gene pass writes):
+//   [0, front)  the gene pass's layout; then the Pairwise replay's layout (make_ws_layout(..., pairwise = true)) with the
+//               variant regions and their pad-mask rows behind it; then the Regulation replay's layout
+//   after it    the gene X_in rows, the pseudo-genes' X_in (token 0 in, the occluded region's Pairwise row out), the
+//               variants' freq and masks, the empty drop sets of subset_expand_kernel and the Regulation plan.
+// The variant regions live only until the Pairwise replay has run, so they share room with the Regulation replay.
+namespace {
+struct OcclusionWs {
+    WsLayout wb, wp, wv;
+    int64_t x_v[CHROMO_MAX_RES], mask_v[CHROMO_MAX_RES];
+    int64_t xin_b, xin_p, freq_v, imask_v, drop0, plan, total;
+    bool plan_on;
+};
+int occlusion_ws(const chromo_config_t* c, int batch, int variants, int flags, OcclusionWs* d) {
+    const int S = c->i_max + 1, NR = c->n_res, V = variants;
+    int64_t row = std::max<int64_t>((int64_t)S * S, (int64_t)NR * c->d_emb * 2);
+    for (int r = 0; r < NR; ++r) row = std::max<int64_t>(row, (int64_t)c->n_bins[r] * c->n_feats);
+    if ((int64_t)batch * row > INT32_MAX || (int64_t)variants * row > INT32_MAX) {
+        set_error("chromo_pcre_occlusion: batch and variants times max((i_max + 1)^2, 2 * n_res * d_emb, n_bins * n_feats) "
+                  "must fit in int32");
+        return CHROMO_EINVAL;
+    }
+    d->wb = make_ws_layout(c, batch, flags);
+    d->wp = make_ws_layout(c, V, flags, false, true);
+    d->wv = make_ws_layout(c, V, flags, true);
+    int64_t cur = d->wp.total;
+    auto take = [&](int64_t n) { int64_t o = cur; cur = align4(cur + n); return o; };
+    for (int r = 0; r < NR; ++r) d->x_v[r] = take((int64_t)V * c->n_bins[r] * c->n_feats);
+    for (int r = 0; r < NR; ++r) d->mask_v[r] = take(((int64_t)V * c->n_bins[r] + 3) / 4);
+    cur = std::max({cur, d->wb.total, d->wv.total});
+    d->xin_b = take((int64_t)NR * batch * S * c->d_emb);
+    d->xin_p = take((int64_t)NR * V * 2 * c->d_emb);
+    d->freq_v = take((int64_t)V * S * S);
+    d->imask_v = take(((int64_t)V * S * S + 3) / 4 * NR);
+    d->drop0 = take(V);
+    d->plan_on = (flags & CHROMO_F_BF16) && d->wv.reg_fused;
+    d->plan = d->plan_on ? take(reg_plan_floats(V, c->i_max)) : 0;
+    d->total = cur;
+    return CHROMO_OK;
+}
+}  // namespace
+
+extern "C" int64_t chromo_pcre_occlusion_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t variants,
+                                                          int32_t flags) {
+    if (validate_config(cfg) != CHROMO_OK) return CHROMO_EINVAL;
+    if (batch < 1 || variants < 1) { set_error("batch and variants must be >= 1"); return CHROMO_EINVAL; }
+    OcclusionWs d;
+    CHROMO_TRY(occlusion_ws(cfg, batch, variants, flags, &d));
+    return d.total;
+}
+
+extern "C" int chromo_pcre_occlusion(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                                     int32_t variants, const int32_t* var_gene, const int32_t* var_slot,
+                                     const int32_t* var_bins, const uint32_t* var_marks, float* logits, float* var_logits,
+                                     float* workspace, int64_t workspace_floats, int32_t flags, void* stream) {
+    CHROMO_TRY(check_forward_args(cfg, params, in, logits, workspace));
+    if (!var_gene || !var_slot || !var_bins || !var_marks || !var_logits) {
+        set_error("chromo_pcre_occlusion: null variant descriptor or output");
+        return CHROMO_EINVAL;
+    }
+    if (variants < 1) { set_error("chromo_pcre_occlusion: variants must be >= 1"); return CHROMO_EINVAL; }
+    if (flags & ~(CHROMO_F_BF16 | CHROMO_F_PACKED | CHROMO_F_DENSE)) {
+        set_error("chromo_pcre_occlusion: inference only (flags CHROMO_F_BF16, CHROMO_F_PACKED, CHROMO_F_DENSE)");
+        return CHROMO_EINVAL;
+    }
+    OcclusionWs d;
+    CHROMO_TRY(occlusion_ws(cfg, in->batch, variants, flags, &d));
+    if (workspace_floats < d.total) {
+        set_error("chromo_pcre_occlusion: workspace too small: need %lld floats, got %lld", (long long)d.total,
+                  (long long)workspace_floats);
+        return CHROMO_ENOMEM;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    float* ws = workspace;
+    const int B = in->batch, I = cfg->i_max, S = I + 1, V = variants, NR = cfg->n_res, D = cfg->d_emb;
+    // 1. the genes: the ordinary forward (it packs the BF16 weights unless CHROMO_F_PACKED), X_in set aside
+    CHROMO_TRY(forward_impl(cfg, params, in, logits, ws, d.wb, flags, st));
+    const size_t row_bytes = (size_t)B * S * D * sizeof(float);
+    if (cudaMemcpy2DAsync(ws + d.xin_b, row_bytes, ws + d.wb.r_xin, (size_t)d.wb.res_stride * sizeof(float), row_bytes, NR,
+                          cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
+        set_error("chromo_pcre_occlusion: X_in copy failed");
+        return CHROMO_ECUDA;
+    }
+    OcclusionDesc desc;
+    desc.B = B; desc.I = I; desc.n_res = NR; desc.F = cfg->n_feats; desc.V = V;
+    desc.gene = var_gene; desc.slot = var_slot; desc.bins = var_bins; desc.marks = var_marks;
+    for (int r = 0; r < CHROMO_MAX_RES; ++r) {
+        desc.n[r] = r < NR ? cfg->n_bins[r] : 0;
+        desc.imask[r] = r < NR ? in->imask[r] : nullptr;
+    }
+    // 2. the variant regions as V pseudo-genes of one slot
+    chromo_batch_t pin;
+    memset(&pin, 0, sizeof(pin));
+    pin.batch = V; pin.freq = in->freq;
+    const long long xin_p_z = (long long)V * 2 * D;
+    {
+        OcclusionExpandArgs a;
+        a.d = desc;
+        a.xin = ws + d.xin_b; a.xin_z = (long long)B * S * D;
+        a.xin_p = ws + d.xin_p; a.xin_p_z = xin_p_z;
+        for (int r = 0; r < NR; ++r) {
+            a.x_pcre[r] = in->x_pcre[r];
+            a.mask_pcre[r] = in->mask_pcre[r]; a.mask_stride[r] = in->mask_pcre_stride[r];
+            a.mask_row_offset[r] = in->mask_pcre_row_offset[r];
+            a.x_v[r] = ws + d.x_v[r];
+            a.mask_v[r] = reinterpret_cast<uint8_t*>(ws + d.mask_v[r]);
+            pin.x_pcre[r] = a.x_v[r];
+            pin.mask_pcre[r] = a.mask_v[r]; pin.mask_pcre_stride[r] = cfg->n_bins[r]; pin.mask_pcre_row_offset[r] = 0;
+            pin.pos_enc[r] = in->pos_enc[r];
+            pin.imask[r] = in->imask[r];      // (not read: the replay builds no ragged plan and stops before the Regulation stage)
+        }
+        CHROMO_TRY(launch_occlusion_expand(a, st));
+    }
+    // 3. their Pairwise pass, on the paths of the gene pass, with the weights it packed
+    const int vflags = (flags & ~CHROMO_F_DENSE) | ((flags & CHROMO_F_BF16) ? CHROMO_F_PACKED : 0);
+    const PwReplay pw{B, I, ws + d.xin_p, xin_p_z};
+    CHROMO_TRY(forward_impl(cfg, params, &pin, nullptr, ws, d.wp, vflags, st, nullptr, nullptr, &pw));
+    // 4. the Regulation input: every variant's gene unchanged (empty drop sets), then the occluded region's row
+    chromo_batch_t vin;
+    memset(&vin, 0, sizeof(vin));
+    vin.batch = V; vin.freq = ws + d.freq_v;
+    if (cudaMemsetAsync(ws + d.drop0, 0, (size_t)V * sizeof(uint32_t), st) != cudaSuccess) {
+        set_error("chromo_pcre_occlusion: memset failed");
+        return CHROMO_ECUDA;
+    }
+    {
+        SubsetExpandArgs a;
+        a.B = B; a.I = I; a.n_res = NR; a.V = V;
+        a.var_gene = var_gene; a.var_drop = reinterpret_cast<const uint32_t*>(ws + d.drop0);
+        a.xin = ws + d.xin_b; a.xin_z = (long long)B * S * D;
+        a.freq = in->freq;
+        a.xin_v = ws + d.wv.r_xin; a.xin_v_z = d.wv.res_stride;
+        a.freq_v = ws + d.freq_v;
+        for (int r = 0; r < NR; ++r) {
+            a.imask[r] = in->imask[r];
+            a.imask_v[r] = reinterpret_cast<uint8_t*>(ws + d.imask_v) + (long long)r * V * S * S;
+            vin.imask[r] = a.imask_v[r];
+        }
+        CHROMO_TRY(launch_subset_expand(a, st));
+    }
+    {
+        OcclusionSpliceArgs a;
+        a.d = desc;
+        a.xin_p = ws + d.xin_p; a.xin_p_z = xin_p_z;
+        a.xin_v = ws + d.wv.r_xin; a.xin_v_z = d.wv.res_stride;
+        CHROMO_TRY(launch_occlusion_splice(a, st));
+    }
+    // 5. the Regulation replay and the head, logits in variant order
+    RaggedPlan plan;
+    if (d.plan_on) {
+        RaggedArgs ra;
+        memset(&ra, 0, sizeof(ra));
+        ra.B = V; ra.I = I; ra.n_res = NR;
+        for (int r = 0; r < NR; ++r) ra.imask[r] = vin.imask[r];
+        CHROMO_TRY(build_reg_plan(ra, ws + d.plan, &plan, st));
+    }
+    const RegReplay replay{d.plan_on ? &plan : nullptr, B};
+    CHROMO_TRY(forward_impl(cfg, params, &vin, var_logits, ws, d.wv, vflags, st, nullptr, &replay));
+    // 6. NaN rows for invalid descriptors, the gene's row for dead slots
+    OcclusionGuardArgs gd;
+    gd.d = desc; gd.n_out = cfg->n_out;
+    gd.logits = logits; gd.logits_v = var_logits;
+    return launch_occlusion_guard(gd, st);
 }
 
 extern "C" int chromo_regulation_layer(const chromo_config_t* cfg, const float* params, int32_t layer, const float* x,

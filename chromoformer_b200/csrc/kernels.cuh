@@ -90,6 +90,7 @@ struct SqaArgs {
     bool tc = false;                        // BF16 training: the four contractions on the staged tcgen05 GEMM
     const __nv_bfloat16* pe_pk = nullptr;   // BF16 tensor path: PE packed as a [n,D] weight
     const __nv_bfloat16* pet_pk = nullptr;  //                   PE^T packed as a [D,n] weight
+    long long path_rows = 0;                // the row count that picks the tensor or the FP32 paths (0 = rows)
 };
 
 // in-silico pCRE deletion (deletion.cu): B genes -> V = B * (I + 1) variants of the Regulation stage
@@ -130,6 +131,40 @@ struct SubsetGuardArgs {
 };
 int launch_subset_expand(const SubsetExpandArgs& a, cudaStream_t st);
 int launch_subset_guard(const SubsetGuardArgs& a, cudaStream_t st);
+
+// histone-mark occlusion (occlusion.cu): variant v = gene var_gene[v] with marks var_marks[v] zeroed over the bins
+// [var_bins[v, r, 0], var_bins[v, r, 1]) of pCRE slot var_slot[v] at every resolution r
+struct OcclusionDesc {
+    int B, I, n_res, F, V;
+    int n[CHROMO_MAX_RES];                          // bins per region
+    const int* gene; const int* slot;               // [V]
+    const int* bins;                                // [V, n_res, 2]
+    const uint32_t* marks;                          // [V]
+    const uint8_t* imask[CHROMO_MAX_RES];           // the genes' interaction masks [B,S,S] (which slots are live)
+};
+struct OcclusionExpandArgs {
+    OcclusionDesc d;
+    const float* x_pcre[CHROMO_MAX_RES];            // [B, I, n_r, F]
+    const uint8_t* mask_pcre[CHROMO_MAX_RES]; long long mask_stride[CHROMO_MAX_RES], mask_row_offset[CHROMO_MAX_RES];
+    const float* xin; long long xin_z;              // X_in of the genes [B*S, 128] per resolution
+    float* x_v[CHROMO_MAX_RES];                     // the variant regions [V, n_r, F]
+    uint8_t* mask_v[CHROMO_MAX_RES];                // their pad-mask centre rows [V, n_r]
+    float* xin_p; long long xin_p_z;                // X_in of the pseudo-genes [V*2, 128] per resolution (token 0 here)
+};
+struct OcclusionSpliceArgs {
+    OcclusionDesc d;
+    const float* xin_p; long long xin_p_z;          // the pseudo-genes' X_in: row 2v + 1 is the occluded region's row
+    float* xin_v; long long xin_v_z;                // X_in of the Regulation replay [V*S, 128] per resolution
+};
+struct OcclusionGuardArgs {
+    OcclusionDesc d;
+    int n_out;
+    const float* logits;                            // [B, n_out]
+    float* logits_v;                                // [V, n_out]: NaN rows for invalid descriptors, the gene's row on dead slots
+};
+int launch_occlusion_expand(const OcclusionExpandArgs& a, cudaStream_t st);
+int launch_occlusion_splice(const OcclusionSpliceArgs& a, cudaStream_t st);
+int launch_occlusion_guard(const OcclusionGuardArgs& a, cudaStream_t st);
 
 int launch_reg_attention(const RegAttnArgs& a, int nz, cudaStream_t st);
 int launch_attn_rows(const AttnRowsArgs& a, cudaStream_t st);

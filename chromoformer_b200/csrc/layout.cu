@@ -182,10 +182,10 @@ const ParamLayout& get_layout(const chromo_config_t* c) {
     return *L;
 }
 
-WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags, bool replay) {
+WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags, bool replay, bool pairwise) {
     WsLayout w;
     memset(&w, 0, sizeof(w));
-    const int B = batch, I = c->i_max, S = I + 1, D = c->d_emb;
+    const int B = batch, I = pairwise ? 1 : c->i_max, S = I + 1, D = c->d_emb;
     const int R = B * I, T = B * S;
     w.B = B; w.I = I; w.S = S; w.R = R; w.T = T; w.D = D;
     w.training = (flags & CHROMO_F_TRAINING) ? 1 : 0;
@@ -222,7 +222,7 @@ WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags, bool rep
             }
             // fused Regulation layer: default geometry only (8 heads x 32, d_ff 256), i_max 8 or 16 (kernel is
             // specialised on the exact token count)
-            if (c->reg_heads == 8 && c->reg_d_model == 256 && c->reg_d_ff == 256 && D == 128 && (S == 9 || S == 17)) {
+            if (c->reg_heads == 8 && c->reg_d_model == 256 && c->reg_d_ff == 256 && D == 128 && (c->i_max == 8 || c->i_max == 16)) {
                 w.reg_fused = 1;
                 w.reg_stream = take(((int64_t)c->n_res * c->reg_layers * 14 * 128 * 128 + 1) / 2 + 8);
             }
@@ -231,6 +231,7 @@ WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags, bool rep
     // ---- per-resolution block
     const int64_t res_base = cur;
     if (!replay) {
+    if (!pairwise) {
     w.e_hc = take((int64_t)B * D);
     w.e_q = take((int64_t)B * c->embed_d_model);
     w.e_qk = take((int64_t)B * He * D);
@@ -242,6 +243,7 @@ WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags, bool rep
     w.e_u = take((int64_t)B * D);
     w.e_f = take((int64_t)B * c->embed_d_ff);
     w.e_preY = take((int64_t)B * D);
+    }   // !pairwise
     w.p_pp = take((int64_t)B * D);
     {
         int64_t s0 = cur;
@@ -263,6 +265,7 @@ WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags, bool rep
         cur = s0 + w.p_slot * w.pslots;
     }
     }   // !replay
+    if (!pairwise) {
     w.r_xin = take((int64_t)T * D);
     // a replay on the fused path (CHROMO_REG_FP32 sends the Regulation stage down the layer-by-layer path instead) needs
     // the last layer's rows (token 0 is what the head reads) and the parking slots of the plan's tiles
@@ -289,19 +292,22 @@ WsLayout make_ws_layout(const chromo_config_t* c, int batch, int flags, bool rep
         w.r_slot = cur - s0;
         cur = s0 + w.r_slot * w.rslots;
     }
+    }   // !pairwise
     w.res_stride = cur - res_base;
     cur = res_base + w.res_stride * c->n_res;
     // ---- resolution-dependent buffers
     for (int r = 0; r < c->n_res && !replay; ++r) {
         // rows may be padded to a multiple of 16 bins (tensor path for short rows, see single_query_attention)
         const int64_t n16 = (c->n_bins[r] + 15) / 16 * 16;
-        w.e_p[r] = take((int64_t)B * He * n16);
+        if (!pairwise) w.e_p[r] = take((int64_t)B * He * n16);
         w.p_p_slot[r] = align4((int64_t)R * Hp * n16);
         w.p_p[r] = take(w.p_p_slot[r] * w.pslots);
     }
-    w.h_z = take((int64_t)B * c->n_res * D);
-    w.h_h1 = take((int64_t)B * c->d_head);
-    if (w.tail_fused && !replay) w.rg_plan = take(ragged_plan_floats(B, I, c->n_res));
+    if (!pairwise) {
+        w.h_z = take((int64_t)B * c->n_res * D);
+        w.h_h1 = take((int64_t)B * c->d_head);
+    }
+    if (w.tail_fused && !replay && !pairwise) w.rg_plan = take(ragged_plan_floats(B, I, c->n_res));
     w.g_base = cur;
     if (w.training) {
         // backward scratch, carved up in backward.cu: every gradient tensor of every layer has its own buffer (the

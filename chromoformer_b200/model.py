@@ -303,6 +303,7 @@ class _ChromoformerCore(nn.Module):
         object.__setattr__(self, "_packed_key", None)
         object.__setattr__(self, "_deletion_packed_key", None)
         object.__setattr__(self, "_subsets_packed_key", None)
+        object.__setattr__(self, "_occlusion_packed_key", None)
         object.__setattr__(self, "_param_epoch", 0)
         self._rebuild_flat()
 
@@ -361,6 +362,7 @@ class _ChromoformerCore(nn.Module):
         object.__setattr__(self, "_packed_key", None)
         object.__setattr__(self, "_deletion_packed_key", None)
         object.__setattr__(self, "_subsets_packed_key", None)
+        object.__setattr__(self, "_occlusion_packed_key", None)
 
     def _flat_is_current(self):
         base = self._flat.data_ptr()
@@ -490,6 +492,38 @@ class _ChromoformerCore(nn.Module):
                    "chromo_pcre_subsets")
         if packed_key is not None:
             object.__setattr__(self, "_subsets_packed_key", packed_key)
+        return logits, var_logits
+
+    def _launch_occlusion(self, io, var_gene, var_slot, var_bins, var_marks, flags):
+        """chromo_pcre_occlusion: (logits [B, n_out], var_logits [V, n_out]) for the variant descriptors ``var_gene``,
+        ``var_slot`` (int32 [V]), ``var_bins`` (int32 [V, n_res, 2]) and ``var_marks`` (int32 [V], the bit pattern of the
+        uint32 mark sets), all moved to the model's device.  Its workspace and packed BF16 weights are cached apart from
+        the other entry points'."""
+        lib = _lib.load()
+        if not self._flat_is_current():
+            self._rebuild_flat()
+        dev, n_out = self._flat.device, int(self._cfg.n_out)
+        V = int(var_gene.numel())
+        descs = (var_gene, var_slot, var_bins, var_marks)
+        if any(t.dtype != torch.int32 for t in descs) or var_slot.numel() != V or var_marks.numel() != V or \
+                var_bins.numel() != V * int(io.cfg.n_res) * 2:
+            raise ValueError("var_gene, var_slot, var_marks must be int32 [V] and var_bins int32 [V, n_res, 2]")
+        var_gene, var_slot, var_bins, var_marks = (t.to(dev).contiguous() for t in descs)
+        ws = self._workspace(io.cfg, io.batch, flags, cached=True, entry="chromo_pcre_occlusion_workspace_floats",
+                             variants=V)
+        packed_key = self._packed_key_of(ws, io, flags)
+        if packed_key is not None and packed_key == self._occlusion_packed_key:
+            flags |= _lib.F_PACKED
+        logits = torch.empty(io.batch, n_out, dtype=torch.float32, device=dev)
+        var_logits = torch.empty(V, n_out, dtype=torch.float32, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(lib.chromo_pcre_occlusion(ctypes.byref(io.cfg), self._flat.data_ptr(), ctypes.byref(io.struct), V,
+                                             var_gene.data_ptr(), var_slot.data_ptr(), var_bins.data_ptr(),
+                                             var_marks.data_ptr(), logits.data_ptr(), var_logits.data_ptr(),
+                                             ws.data_ptr(), ws.numel(), flags, stream),
+                   "chromo_pcre_occlusion")
+        if packed_key is not None:
+            object.__setattr__(self, "_occlusion_packed_key", packed_key)
         return logits, var_logits
 
     def _launch_backward(self, io, ws, dlogits, want_dx=None):

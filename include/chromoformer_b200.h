@@ -161,6 +161,35 @@ int chromo_pcre_subsets(const chromo_config_t* cfg, const float* params, const c
                         int32_t variants, float* logits /* [B,n_out] */, float* var_logits /* [V,n_out] */,
                         float* workspace, int64_t workspace_floats, int32_t flags, void* stream);
 
+/* ---- histone-mark occlusion: the logits with marks removed over bin windows of one pCRE --------------------------
+ * For B genes with I = i_max slots (S = I + 1 tokens), n_res resolutions of n_r bins and V variants.  Variant v is gene
+ * g = var_gene[v] with
+ *     pcre_feats[r][g, i, lo_r:hi_r, m] = 0     i = var_slot[v], [lo_r, hi_r) = var_bins[v, r, 0:2], m in var_marks[v]
+ * at every resolution r (bit m of var_marks: mark m); pad masks, interaction masks and freq stay as they are.  An empty
+ * range leaves that resolution alone.  Zero is what the input path writes where no read fell (ln(0 + 1)).
+ *   logits[g]          the ordinary forward, bit-identical to chromo_forward with the same flags;
+ *   var_logits[v]      the logits of the occluded gene, in variant order; on a dead slot (no pCRE, as defined for
+ *                      chromo_pcre_deletion) logits[g] bit for bit.
+ * One Embedding + Pairwise pass per gene; then ONE Pairwise pass per variant, over the occluded region alone (region i
+ * feeds only its own Pairwise row), and the Regulation transformer and the head over the V variants.  Every GEMM takes
+ * the path (tcgen05 or FP32) the gene pass takes for the same B genes, and a variant's region is computed apart from the
+ * others over the whole position table, so a variant's logits do not depend on V or on the other variants.  The path
+ * choice is shared, not the bits: where the BF16 gene pass builds its ragged plan, its own regions use key windows shared
+ * by a tile, and a variant without effect matches logits[g] to BF16 rounding.  The descriptors (device memory) are checked on the
+ * device: var_gene outside [0, B), var_slot outside [0, I), lo_r < 0, lo_r > hi_r, hi_r > n_r or a mark bit at or above
+ * n_feats reads no gene and gets a NaN row; the other rows are unaffected.  No atomics on the floating-point path;
+ * identical inputs give identical outputs; no host synchronisation (legal inside a stream capture).  Flags:
+ * CHROMO_F_BF16, CHROMO_F_PACKED and the CHROMO_F_DENSE hint (the gene pass only); any other flag, a NULL descriptor or
+ * output, or variants < 1 is CHROMO_EINVAL.  The workspace must hold chromo_pcre_occlusion_workspace_floats floats
+ * (CHROMO_ENOMEM otherwise) and keeps the packed BF16 weights at its front, as a chromo_forward workspace does.        */
+int64_t chromo_pcre_occlusion_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t variants,
+                                               int32_t flags);
+int chromo_pcre_occlusion(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in, int32_t variants,
+                          const int32_t* var_gene /* [V] device */, const int32_t* var_slot /* [V] device */,
+                          const int32_t* var_bins /* [V,n_res,2] device */, const uint32_t* var_marks /* [V] device */,
+                          float* logits /* [B,n_out] */, float* var_logits /* [V,n_out] */, float* workspace,
+                          int64_t workspace_floats, int32_t flags, void* stream);
+
 /* ---- one Regulation-transformer layer: AttentionBlock with gate (modules.py:104-111 as used by
  * net.py:152-153), for every resolution at once: y[r] = layer(x[r]), x/y = [n_res][B*(i_max+1), d_emb] FP32
  * with `xy_stride` floats between resolutions.  With CHROMO_F_BF16 and the default geometry this is ONE
