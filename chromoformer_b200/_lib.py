@@ -90,6 +90,9 @@ EXPORTS = {
     "chromo_pcre_subsets_workspace_floats": (c_int64, [POINTER(Config), c_int32, c_int32, c_int32]),
     "chromo_pcre_subsets": (c_int32, [POINTER(Config), c_void_p, POINTER(Batch), c_void_p, c_void_p, c_int32, c_void_p,
                                       c_void_p, c_void_p, c_int64, c_int32, c_void_p]),
+    "chromo_freq_edits_workspace_floats": (c_int64, [POINTER(Config), c_int32, c_int32, c_int32]),
+    "chromo_freq_edits": (c_int32, [POINTER(Config), c_void_p, POINTER(Batch), c_void_p, c_void_p, c_int32, c_void_p,
+                                    c_void_p, c_void_p, c_int64, c_int32, c_void_p]),
     "chromo_pcre_occlusion_workspace_floats": (c_int64, [POINTER(Config), c_int32, c_int32, c_int32]),
     "chromo_pcre_occlusion": (c_int32, [POINTER(Config), c_void_p, POINTER(Batch), c_int32, c_void_p, c_void_p, c_void_p,
                                         c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_int32, c_void_p]),

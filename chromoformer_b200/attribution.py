@@ -12,7 +12,10 @@ approximations; ``pcre_deletion`` gives the exact counterfactual per pCRE: the p
 ``pcre_subsets`` gives the prediction without any set of pCREs, and on top of it ``pcre_shapley`` (credit per pCRE that
 sums to logits - promoter only) and ``pcre_interactions`` (the synergy of every pair of pCREs).  ``pcre_occlusion`` and
 ``occlusion_map`` give the exact counterpart of the saliency maps: the prediction with histone marks removed over a
-window of bins.
+window of bins.  ``freq_edits`` gives the exact prediction with any interaction frequencies changed, and on top of it
+``contact_knockout`` (each pCRE's Hi-C contact set to 0, and every contact: the contact-blind prediction),
+``contact_response`` (the prediction against contact strength) and ``contact_shapley`` (credit per contact that sums to
+logits - blind): the exact counterparts of the ``freq=True`` attributions.
 """
 import contextlib
 import math
@@ -24,7 +27,8 @@ from . import _lib
 from .model import _BatchIO
 
 __all__ = ["input_gradients", "integrated_gradients", "pcre_scores", "pcre_deletion", "pcre_subsets", "pcre_shapley",
-           "pcre_interactions", "pcre_occlusion", "occlusion_map"]
+           "pcre_interactions", "pcre_occlusion", "occlusion_map", "freq_edits", "contact_knockout", "contact_response",
+           "contact_shapley"]
 
 _FEATS = ("promoter_feats", "pcre_feats")
 _MASKS = ("promoter_pad_masks", "pcre_pad_masks")
@@ -242,10 +246,12 @@ def _live(dev_batch, bins):
     return (~im[:, :, 0, 1:]).any(0)
 
 
-def _replay(model, dev_batch, bins, var_gene, var_drop, chunk, dense):
-    """logits [B, n_out] and var_logits [V, n_out] on the device for variant descriptors given as numpy int64 arrays:
-    var_gene non-decreasing, every gene with at least one variant.  One library call covers whole genes, at most ``chunk``
-    variants (a gene with more gets a call of its own), so every gene's Embedding / Pairwise pass runs once."""
+def _calls(model, dev_batch, bins, var_gene, chunk, dense, launch):
+    """logits [B, n_out] and var_logits [V, n_out] on the device for variants of the genes ``var_gene`` (numpy int64,
+    non-decreasing, every gene with at least one variant), by library calls ``launch(io, v0, v1, vg, flags)`` over the
+    variants [v0, v1), vg their genes as int32 on the device relative to the call's first gene.  One call covers whole
+    genes, at most ``chunk`` variants (a gene with more gets a call of its own), so every gene's Embedding / Pairwise
+    pass runs once."""
     if chunk < 1:
         raise ValueError("chunk must be >= 1")
     B = int(dev_batch[_FREQ].shape[0])
@@ -265,12 +271,20 @@ def _replay(model, dev_batch, bins, var_gene, var_drop, chunk, dense):
             io = _BatchIO(model, *[[dev_batch[key][b][g0:g1] for b in bins] for key in _GENE_KEYS],
                           dev_batch[_FREQ][g0:g1])
             vg = torch.from_numpy((var_gene[v0:v1] - g0).astype(np.int32)).to(dev)
-            vd = torch.from_numpy(var_drop[v0:v1].astype(np.int32)).to(dev)
-            lg, vl = model._launch_subsets(io, vg, vd, flags)
+            lg, vl = launch(io, v0, v1, vg, flags)
             logits.append(lg)
             var_logits.append(vl)
             g0 = g1
     return torch.cat(logits), torch.cat(var_logits)
+
+
+def _replay(model, dev_batch, bins, var_gene, var_drop, chunk, dense):
+    """``_calls`` over ``chromo_pcre_subsets``: variant v drops the pCREs of the bit set var_drop[v] (numpy int64)."""
+    dev = model.flat_params.device
+
+    def launch(io, v0, v1, vg, flags):
+        return model._launch_subsets(io, vg, torch.from_numpy(var_drop[v0:v1].astype(np.int32)).to(dev), flags)
+    return _calls(model, dev_batch, bins, var_gene, chunk, dense, launch)
 
 
 def pcre_subsets(model, batch, drop, target=None, chunk=_SUBSET_CHUNK, dense=False):
@@ -380,6 +394,51 @@ def _interaction_descriptors(live):
     return gene[valid].numpy(), bits.view(1, -1).expand(B, -1)[valid].numpy(), valid, pairs
 
 
+def _shapley(model, batch, target, permutations, seed, replay):
+    """Shapley values of each gene's live slots, the value of a coalition T being ``logits[target]`` of
+    ``replay(dev_batch, bins, var_gene, var_bits)`` (numpy int64 descriptors; bit i of var_bits: slot i is NOT in T).
+    Exact over the 2^k subsets, or with ``permutations=P`` the estimate over P seeded orders; combined in FP64 in a fixed
+    order.  Returns (shapley [B, I] float64 on the device, logits, the logits of the empty coalition)."""
+    bins = list(model.binsizes)
+    t = _default_target(model, target)
+    dev_batch = _to_device(batch, model, bins)
+    live = _live(dev_batch, bins).cpu()                      # (the one host read of the call)
+    B, I = live.shape
+    k = live.sum(1)
+    live_bits = (live.long() << torch.arange(I)).sum(1)
+    shapley = torch.zeros(B, I, dtype=torch.float64)
+    if permutations is None:
+        if int(k.max()) > 12:
+            g = int(torch.argmax(k))
+            raise ValueError(f"gene {g} has {int(k[g])} pCREs: exact Shapley values need 2^k variants per gene; "
+                             "pass permutations= for the sampling estimate")
+        var_gene, var_bits, groups = _shapley_descriptors(live)
+        logits, var_logits = replay(dev_batch, bins, var_gene, var_bits)
+        v = var_logits[:, t].double().cpu().numpy()
+        for kk, genes, slots, idx in groups:
+            if kk:
+                shapley[genes.view(-1, 1), slots] = _shapley_exact(torch.from_numpy(v[idx]), kk)
+        none = var_logits[torch.from_numpy(_first_variants(var_gene)).to(var_logits.device)]   # the empty coalition
+    else:
+        P = int(permutations)
+        if P < 1:
+            raise ValueError("permutations must be >= 1")
+        gen = torch.Generator().manual_seed(int(seed))
+        r = torch.rand(B, P, I, generator=gen, dtype=torch.float64)
+        order = torch.argsort(torch.where(live.view(B, 1, I), r, torch.full((), 2.0, dtype=torch.float64)), dim=2)
+        kept = torch.cat([torch.zeros(B, P, 1, dtype=torch.long), torch.cumsum(1 << order, dim=2)], 2)   # [B, P, I + 1]
+        valid = (torch.arange(I + 1).view(1, 1, I + 1) <= k.view(B, 1, 1)).expand(B, P, I + 1)
+        bits = live_bits.view(B, 1, 1) & ~kept
+        gene = torch.arange(B).view(B, 1, 1).expand(B, P, I + 1)
+        logits, var_logits = replay(dev_batch, bins, gene[valid].numpy(), bits[valid].numpy())
+        v = torch.zeros(B, P, I + 1, dtype=torch.float64)
+        v[valid] = var_logits[:, t].double().cpu()
+        shapley = _shapley_from_orders(v, order, k)
+        first = torch.nonzero(valid.reshape(-1)).view(-1)      # prefix 0 of order 0 is each gene's first variant
+        none = var_logits[torch.searchsorted(first, torch.arange(B) * P * (I + 1)).to(var_logits.device)]
+    return shapley.to(logits.device), logits, none
+
+
 def pcre_shapley(model, batch, target=None, permutations=None, seed=0, chunk=_SUBSET_CHUNK, dense=False):
     """Shapley values of the pCREs of every gene: the players are the gene's pCREs (its live slots, as for
     ``pcre_deletion``), the value of a set T is ``logits[target]`` of the gene with only the pCREs of T kept (from
@@ -399,46 +458,10 @@ def pcre_shapley(model, batch, target=None, permutations=None, seed=0, chunk=_SU
     ``target`` defaults to column 1 for the classifier and 0 for the regressor; ``chunk`` and ``dense`` are those of
     ``pcre_subsets``.  Cost: one Embedding / Pairwise pass per gene and the Regulation transformer over the variants; a
     variant keeping m pCREs costs m + 1 tokens on the BF16 path (DESIGN.md 3.5)."""
-    bins = list(model.binsizes)
-    t = _default_target(model, target)
-    dev_batch = _to_device(batch, model, bins)
-    live = _live(dev_batch, bins).cpu()                      # (the one host read of the call)
-    B, I = live.shape
-    k = live.sum(1)
-    live_bits = (live.long() << torch.arange(I)).sum(1)
-    # the slots of each gene, its pCREs first (ascending)
-    shapley = torch.zeros(B, I, dtype=torch.float64)
-    if permutations is None:
-        if int(k.max()) > 12:
-            g = int(torch.argmax(k))
-            raise ValueError(f"gene {g} has {int(k[g])} pCREs: exact Shapley values need 2^k variants per gene; "
-                             "pass permutations= for the sampling estimate")
-        var_gene, var_drop, groups = _shapley_descriptors(live)
-        logits, var_logits = _replay(model, dev_batch, bins, var_gene, var_drop, chunk, dense)
-        v = var_logits[:, t].double().cpu().numpy()
-        for kk, genes, slots, idx in groups:
-            if kk:
-                shapley[genes.view(-1, 1), slots] = _shapley_exact(torch.from_numpy(v[idx]), kk)
-        promoter_only = var_logits[torch.from_numpy(_first_variants(var_gene)).to(var_logits.device)]   # the empty coalition
-    else:
-        P = int(permutations)
-        if P < 1:
-            raise ValueError("permutations must be >= 1")
-        gen = torch.Generator().manual_seed(int(seed))
-        r = torch.rand(B, P, I, generator=gen, dtype=torch.float64)
-        order = torch.argsort(torch.where(live.view(B, 1, I), r, torch.full((), 2.0, dtype=torch.float64)), dim=2)
-        kept = torch.cat([torch.zeros(B, P, 1, dtype=torch.long), torch.cumsum(1 << order, dim=2)], 2)   # [B, P, I + 1]
-        valid = (torch.arange(I + 1).view(1, 1, I + 1) <= k.view(B, 1, 1)).expand(B, P, I + 1)
-        drop = live_bits.view(B, 1, 1) & ~kept
-        gene = torch.arange(B).view(B, 1, 1).expand(B, P, I + 1)
-        logits, var_logits = _replay(model, dev_batch, bins, gene[valid].numpy(), drop[valid].numpy(), chunk, dense)
-        v = torch.zeros(B, P, I + 1, dtype=torch.float64)
-        v[valid] = var_logits[:, t].double().cpu()
-        shapley = _shapley_from_orders(v, order, k)
-        first = torch.nonzero(valid.reshape(-1)).view(-1)      # prefix 0 of order 0 is each gene's first variant
-        promoter_only = var_logits[torch.searchsorted(first, torch.arange(B) * P * (I + 1)).to(var_logits.device)]
-    dev = logits.device
-    return {"shapley": shapley.to(dev), "logits": logits, "promoter_only": promoter_only}
+    def replay(dev_batch, bins, var_gene, var_drop):
+        return _replay(model, dev_batch, bins, var_gene, var_drop, chunk, dense)
+    shapley, logits, promoter_only = _shapley(model, batch, target, permutations, seed, replay)
+    return {"shapley": shapley, "logits": logits, "promoter_only": promoter_only}
 
 
 def _interactions(f0, fi, fij, pairs, live):
@@ -698,3 +721,172 @@ def occlusion_map(model, batch, window=1, stride=None, marks="all", target=None,
             "effect_pcre": logits[:, t].view(B, 1, 1, 1) - pcre[..., t],
             "effect_promoter": logits[:, t].view(B, 1, 1) - promoter[..., t],
             "logits": logits, "windows": torch.from_numpy(windows)}
+
+
+# ---- interaction-frequency edits (chromo_freq_edits) ---------------------------------------------------------------
+def _freq_replay(model, dev_batch, bins, var_gene, var_freq, chunk, dense):
+    """``_calls`` over ``chromo_freq_edits``: ``var_freq(v0, v1)`` gives the edits of variants [v0, v1) as float32
+    [v1 - v0, S, S] on the device (NaN = keep), built for that call only."""
+    def launch(io, v0, v1, vg, flags):
+        return model._launch_freq_edits(io, vg, var_freq(v0, v1), flags)
+    return _calls(model, dev_batch, bins, var_gene, chunk, dense, launch)
+
+
+def freq_edits(model, batch, freq, target=None, chunk=_SUBSET_CHUNK, dense=False):
+    """The exact logits of every gene with its pCRE-promoter interaction frequencies changed (``chromo_freq_edits``),
+    from one Embedding / Pairwise pass per gene and a batched replay of the Regulation transformer and the head over the
+    variants (interaction_freq enters only the Regulation attention, as the bias gamma_f * freq).
+
+    ``freq`` is float, [V, S, S] (the same V edits for every gene) or [B, V, S, S], S = I + 1: variant v of gene g is
+    the gene with ``interaction_freq[g]`` replaced entry by entry by the entries of ``freq[g, v]`` that are not NaN (NaN
+    keeps the gene's value, so an all-NaN edit gives the gene itself).  The contact of pCRE i with the promoter is entry
+    (0, i + 1); see ``contact_knockout``, ``contact_response`` and ``contact_shapley``.  An edit with a +-inf entry gives
+    a NaN row.  Returns
+
+        "logits"    [B, n_out]      the ordinary forward (bit-identical to ``forward_batch`` with the same ``dense``)
+        "variants"  [B, V, n_out]   the logits of each variant
+        "value"     [B, V]          variants[..., target], only when ``target`` is given
+
+    ``chunk`` and ``dense`` are those of ``pcre_subsets``; each call's edits are moved to the device for that call only.
+    Nothing requires grad."""
+    bins = list(model.binsizes)
+    dev_batch = _to_device(batch, model, bins)
+    B, S = (int(n) for n in dev_batch[_FREQ].shape[:2])
+    freq = torch.as_tensor(freq)
+    if not freq.is_floating_point():
+        raise ValueError("freq must be a float tensor")
+    if freq.dim() not in (3, 4) or tuple(freq.shape[-2:]) != (S, S) or freq.shape[-3] < 1 or \
+            (freq.dim() == 4 and freq.shape[0] != B):
+        raise ValueError(f"freq must be [V, {S}, {S}] or [{B}, V, {S}, {S}] with V >= 1, got {tuple(freq.shape)}")
+    V = int(freq.shape[-3])
+    dev = model.flat_params.device
+    if freq.dim() == 3:
+        shared = freq.to(device=dev, dtype=torch.float32)
+
+        def var_freq(v0, v1):
+            return shared[torch.arange(v0, v1, device=dev) % V]
+    else:
+        flat = freq.reshape(B * V, S, S)
+
+        def var_freq(v0, v1):
+            return flat[v0:v1].to(device=dev, dtype=torch.float32)
+    logits, var_logits = _freq_replay(model, dev_batch, bins, np.repeat(np.arange(B), V), var_freq, chunk, dense)
+    out = {"logits": logits, "variants": var_logits.view(B, V, -1)}
+    if target is not None:
+        out["value"] = out["variants"][..., _default_target(model, target)]
+    return out
+
+
+def _contact_replay(model, dev_batch, bins, var_gene, var_bits, var_value, chunk, dense, relative=False):
+    """``_freq_replay`` of contact edits: variant v sets the contact [0, i + 1] of every slot i of the bit set
+    var_bits[v] to var_value[v], or with ``relative`` to var_value[v] times the gene's own contact; nothing else
+    changes (numpy descriptors)."""
+    dev = model.flat_params.device
+    freq = dev_batch[_FREQ]
+    S = int(freq.shape[1])
+    slot_bits = torch.arange(S - 1, device=dev)
+    gene_t = torch.from_numpy(np.asarray(var_gene, dtype=np.int64)).to(dev)
+    bits_t = torch.from_numpy(np.asarray(var_bits, dtype=np.int64)).to(dev)
+    value_t = torch.from_numpy(np.asarray(var_value, dtype=np.float32)).to(dev)
+
+    def var_freq(v0, v1):
+        sel = ((bits_t[v0:v1].view(-1, 1) >> slot_bits) & 1).bool()
+        value = value_t[v0:v1].view(-1, 1)
+        contact = value * freq[gene_t[v0:v1], 0, 1:].float() if relative else value.expand(v1 - v0, S - 1)
+        out = torch.full((v1 - v0, S, S), float("nan"), dtype=torch.float32, device=dev)
+        out[:, 0, 1:] = torch.where(sel, contact, torch.full((), float("nan"), device=dev))
+        return out
+    return _freq_replay(model, dev_batch, bins, var_gene, var_freq, chunk, dense)
+
+
+def contact_knockout(model, batch, target=None, chunk=_SUBSET_CHUNK, dense=False):
+    """The exact logits of every gene with the Hi-C contact of each pCRE with the promoter (interaction_freq[g, 0, i + 1],
+    the only entry the dataset writes) set to 0, the pCRE's marks kept, and with every contact set to 0 ("contact-blind":
+    the prediction without the Hi-C information).  Returns
+
+        "without"       [B, I, n_out]  the logits with the contact of pCRE i set to 0; on a dummy slot the logits
+        "blind"         [B, n_out]     the logits with every contact set to 0
+        "effect"        [B, I]         logits[:, target] - without[:, :, target]; exactly 0.0 on dummy slots
+        "blind_effect"  [B]            logits[:, target] - blind[:, target]
+        "logits"        [B, n_out]     the ordinary forward
+
+    ``pcre_deletion``'s effect removes the marks and the contact together; the difference of the two effects is what
+    the pCRE contributes beyond its contact.  Dummy slots (no pCRE, see ``pcre_deletion``) run no variant.  ``target``
+    defaults to column 1 for the classifier and 0 for the regressor; ``chunk`` and ``dense`` as for ``pcre_subsets``."""
+    bins = list(model.binsizes)
+    t = _default_target(model, target)
+    dev_batch = _to_device(batch, model, bins)
+    live = _live(dev_batch, bins).cpu()
+    B, I = live.shape
+    g, i = (x.numpy() for x in torch.nonzero(live, as_tuple=True))
+    live_bits = (live.long() << torch.arange(I)).sum(1).numpy()
+    # per gene: one variant per pCRE (slot order), then the blind one
+    gene = np.concatenate([g, np.arange(B)])
+    bits = np.concatenate([np.int64(1) << i, live_bits])
+    blind_row = np.concatenate([np.zeros(len(g), dtype=bool), np.ones(B, dtype=bool)])
+    order = np.argsort(gene, kind="stable")
+    gene, bits, blind_row = gene[order], bits[order], blind_row[order]
+    logits, var_logits = _contact_replay(model, dev_batch, bins, gene, bits, np.zeros(len(gene)), chunk, dense)
+    n_out = logits.shape[1]
+    blind_t = torch.from_numpy(blind_row).to(logits.device)
+    without = logits.view(B, 1, n_out).expand(B, I, n_out).clone()
+    without[live.to(logits.device)] = var_logits[~blind_t]
+    blind = var_logits[blind_t]
+    return {"without": without, "blind": blind, "effect": logits[:, t:t + 1] - without[:, :, t],
+            "blind_effect": logits[:, t] - blind[:, t], "logits": logits}
+
+
+def contact_response(model, batch, values, relative=False, target=None, chunk=_SUBSET_CHUNK, dense=False):
+    """Response curves of the prediction against contact strength: for every pCRE i of every gene and every grid value
+    ``values[j]``, the exact logits with the contact interaction_freq[g, 0, i + 1] set to ``values[j]``, or with
+    ``relative=True`` to ``values[j]`` times the gene's own contact (1.0 gives the gene itself); everything else
+    unchanged.  Returns
+
+        "response"  [B, I, G, n_out]   on a dummy slot the logits themselves (no variant is run for it)
+        "value"     [B, I, G]          response[..., target]
+        "logits"    [B, n_out]         the ordinary forward
+
+    ``target`` defaults to column 1 for the classifier and 0 for the regressor; ``chunk`` and ``dense`` as for
+    ``pcre_subsets``."""
+    bins = list(model.binsizes)
+    t = _default_target(model, target)
+    dev_batch = _to_device(batch, model, bins)
+    values = np.asarray(torch.as_tensor(values, dtype=torch.float32).reshape(-1).numpy())
+    G = len(values)
+    if G < 1:
+        raise ValueError("values must hold at least one value")
+    live = _live(dev_batch, bins).cpu()
+    B, I = live.shape
+    g, i = (x.numpy() for x in torch.nonzero(live, as_tuple=True))
+    # genes without a pCRE get one empty variant (the gene itself, discarded): every gene needs one
+    empty = np.nonzero(~live.any(1).numpy())[0]
+    gene = np.concatenate([np.repeat(g, G), empty])
+    bits = np.concatenate([np.repeat(np.int64(1) << i, G), np.zeros(len(empty), dtype=np.int64)])
+    value = np.concatenate([np.tile(values, len(g)), np.zeros(len(empty), dtype=np.float32)])
+    order = np.argsort(gene, kind="stable")
+    gene, bits, value = gene[order], bits[order], value[order]
+    logits, var_logits = _contact_replay(model, dev_batch, bins, gene, bits, value, chunk, dense, relative)
+    n_out = logits.shape[1]
+    response = logits.view(B, 1, 1, n_out).expand(B, I, G, n_out).clone()
+    response[live.to(logits.device)] = var_logits[torch.from_numpy(bits != 0).to(logits.device)].view(len(g), G, n_out)
+    return {"response": response, "value": response[..., t], "logits": logits}
+
+
+def contact_shapley(model, batch, target=None, permutations=None, seed=0, chunk=_SUBSET_CHUNK, dense=False):
+    """Shapley values of the Hi-C contacts of every gene: the players are the contacts interaction_freq[g, 0, i + 1] of
+    the gene's pCREs (its live slots, as for ``pcre_deletion``), and the value of a set T is ``logits[target]`` with the
+    contacts outside T set to 0 (the marks of every pCRE kept).  The values of a gene sum to
+    v(all) - v(none) = logits[target] - blind[target] (``contact_knockout``), up to the rounding of the FP64 combination:
+    the exact counterpart of ``integrated_gradients(freq=True)`` restricted to the contacts.  Exact by default (2^k
+    variants per gene; more than 12 pCREs is a ValueError); ``permutations=P`` gives the seeded estimate over P orders
+    per gene, as for ``pcre_shapley``.  Returns
+
+        "shapley"  [B, I] float64   exactly 0.0 on dummy slots
+        "logits"   [B, n_out]       the ordinary forward
+        "blind"    [B, n_out]       the logits with every contact set to 0
+
+    ``target``, ``chunk`` and ``dense`` as for ``pcre_shapley``."""
+    def replay(dev_batch, bins, var_gene, var_bits):
+        return _contact_replay(model, dev_batch, bins, var_gene, var_bits, np.zeros(len(var_gene)), chunk, dense)
+    shapley, logits, blind = _shapley(model, batch, target, permutations, seed, replay)
+    return {"shapley": shapley, "logits": logits, "blind": blind}

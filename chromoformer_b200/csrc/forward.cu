@@ -1396,21 +1396,22 @@ extern "C" int chromo_pcre_deletion(const chromo_config_t* cfg, const float* par
     return launch_deletion_scatter(s, st);
 }
 
-// ---- pCRE subsets (subsets.cu) ----
+// ---- pCRE subsets (subsets.cu) and interaction-frequency edits (freq_edits.cu) ----
 // Workspace: the larger of the gene pass's layout and the replay layout of the V variants [0, front) (both start with
 // the same batch-independent front, the packed BF16 weights; the replay layout has no Embedding or Pairwise block), then
-// the gene X_in rows, the variants' freq and masks and the Regulation plan of the variants.
+// the gene X_in rows, the variants' freq and masks and the Regulation plan of the variants.  chromo_freq_edits adds the
+// V empty drop sets of subset_expand_kernel behind it.
 namespace {
 struct SubsetsWs {
     WsLayout wb, wv;
     int64_t xin_b, freq_v, imask_v, plan, total;
     bool plan_on;
 };
-int subsets_ws(const chromo_config_t* c, int batch, int variants, int flags, SubsetsWs* d) {
+int subsets_ws(const chromo_config_t* c, int batch, int variants, int flags, SubsetsWs* d, const char* fn) {
     const int S = c->i_max + 1;
     const int64_t row = std::max<int64_t>((int64_t)S * S, (int64_t)c->n_res * c->d_emb);
     if ((int64_t)batch * row > INT32_MAX || (int64_t)variants * row > INT32_MAX) {
-        set_error("chromo_pcre_subsets: batch and variants times max((i_max + 1)^2, n_res * d_emb) must fit in int32");
+        set_error("%s: batch and variants times max((i_max + 1)^2, n_res * d_emb) must fit in int32", fn);
         return CHROMO_EINVAL;
     }
     const int V = variants;
@@ -1426,45 +1427,37 @@ int subsets_ws(const chromo_config_t* c, int batch, int variants, int flags, Sub
     d->total = cur;
     return CHROMO_OK;
 }
-}  // namespace
 
-extern "C" int64_t chromo_pcre_subsets_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t variants,
-                                                        int32_t flags) {
-    if (validate_config(cfg) != CHROMO_OK) return CHROMO_EINVAL;
-    if (batch < 1 || variants < 1) { set_error("batch and variants must be >= 1"); return CHROMO_EINVAL; }
-    SubsetsWs d;
-    CHROMO_TRY(subsets_ws(cfg, batch, variants, flags, &d));
-    return d.total;
-}
+// chromo_freq_edits: the subsets layout, then the V drop words at d.total
+int64_t freq_edits_total(const SubsetsWs& d, int variants) { return align4(d.total + variants); }
 
-extern "C" int chromo_pcre_subsets(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
-                                   const int32_t* var_gene, const uint32_t* var_drop, int32_t variants, float* logits,
-                                   float* var_logits, float* workspace, int64_t workspace_floats, int32_t flags,
-                                   void* stream) {
+int check_subsets_args(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in, const void* var_gene,
+                       const void* var_desc, int variants, const float* logits, const float* var_logits,
+                       const float* workspace, int flags, const char* fn) {
     CHROMO_TRY(check_forward_args(cfg, params, in, logits, workspace));
-    if (!var_gene || !var_drop || !var_logits) { set_error("chromo_pcre_subsets: null variant descriptor or output"); return CHROMO_EINVAL; }
-    if (variants < 1) { set_error("chromo_pcre_subsets: variants must be >= 1"); return CHROMO_EINVAL; }
+    if (!var_gene || !var_desc || !var_logits) { set_error("%s: null variant descriptor or output", fn); return CHROMO_EINVAL; }
+    if (variants < 1) { set_error("%s: variants must be >= 1", fn); return CHROMO_EINVAL; }
     if (flags & ~(CHROMO_F_BF16 | CHROMO_F_PACKED | CHROMO_F_DENSE)) {
-        set_error("chromo_pcre_subsets: inference only (flags CHROMO_F_BF16, CHROMO_F_PACKED, CHROMO_F_DENSE)");
+        set_error("%s: inference only (flags CHROMO_F_BF16, CHROMO_F_PACKED, CHROMO_F_DENSE)", fn);
         return CHROMO_EINVAL;
     }
-    SubsetsWs d;
-    CHROMO_TRY(subsets_ws(cfg, in->batch, variants, flags, &d));
-    if (workspace_floats < d.total) {
-        set_error("chromo_pcre_subsets: workspace too small: need %lld floats, got %lld", (long long)d.total,
-                  (long long)workspace_floats);
-        return CHROMO_ENOMEM;
-    }
-    cudaStream_t st = (cudaStream_t)stream;
-    float* ws = workspace;
-    const int B = in->batch, I = cfg->i_max, S = I + 1, V = variants, NR = cfg->n_res, D = cfg->d_emb;
+    return CHROMO_OK;
+}
+
+// The sequence both entry points run: the gene pass, its X_in set aside, subset_expand_kernel, the splice of the freq
+// edits (`splice`, chromo_freq_edits only: its B, I, V and freq_v are filled in here), the variants' Regulation plan,
+// the replay of the Regulation transformer and the head, and subset_guard_kernel.
+int subsets_run(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in, const int32_t* var_gene,
+                const uint32_t* var_drop, int V, float* logits, float* var_logits, float* ws, const SubsetsWs& d,
+                int flags, cudaStream_t st, FreqSpliceArgs* splice, const char* fn) {
+    const int B = in->batch, I = cfg->i_max, S = I + 1, NR = cfg->n_res, D = cfg->d_emb;
     // the genes: the ordinary forward (it packs the BF16 weights unless CHROMO_F_PACKED), X_in left in the workspace
     CHROMO_TRY(forward_impl(cfg, params, in, logits, ws, d.wb, flags, st));
     // their X_in rows out of the way of the replay layout, which overlaps the gene layout
     const size_t row_bytes = (size_t)B * S * D * sizeof(float);
     if (cudaMemcpy2DAsync(ws + d.xin_b, row_bytes, ws + d.wb.r_xin, (size_t)d.wb.res_stride * sizeof(float), row_bytes, NR,
                           cudaMemcpyDeviceToDevice, st) != cudaSuccess) {
-        set_error("chromo_pcre_subsets: X_in copy failed");
+        set_error("%s: X_in copy failed", fn);
         return CHROMO_ECUDA;
     }
     chromo_batch_t vin;
@@ -1485,6 +1478,11 @@ extern "C" int chromo_pcre_subsets(const chromo_config_t* cfg, const float* para
         }
         CHROMO_TRY(launch_subset_expand(a, st));
     }
+    if (splice) {
+        splice->B = B; splice->I = I; splice->V = V;
+        splice->freq_v = ws + d.freq_v;
+        CHROMO_TRY(launch_freq_splice(*splice, st));
+    }
     RaggedPlan plan;
     if (d.plan_on) {
         RaggedArgs ra;
@@ -1501,6 +1499,66 @@ extern "C" int chromo_pcre_subsets(const chromo_config_t* cfg, const float* para
     gd.B = B; gd.I = I; gd.V = V; gd.n_out = cfg->n_out;
     gd.var_gene = var_gene; gd.var_drop = var_drop; gd.logits_v = var_logits;
     return launch_subset_guard(gd, st);
+}
+}  // namespace
+
+extern "C" int64_t chromo_pcre_subsets_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t variants,
+                                                        int32_t flags) {
+    if (validate_config(cfg) != CHROMO_OK) return CHROMO_EINVAL;
+    if (batch < 1 || variants < 1) { set_error("batch and variants must be >= 1"); return CHROMO_EINVAL; }
+    SubsetsWs d;
+    CHROMO_TRY(subsets_ws(cfg, batch, variants, flags, &d, "chromo_pcre_subsets"));
+    return d.total;
+}
+
+extern "C" int chromo_pcre_subsets(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                                   const int32_t* var_gene, const uint32_t* var_drop, int32_t variants, float* logits,
+                                   float* var_logits, float* workspace, int64_t workspace_floats, int32_t flags,
+                                   void* stream) {
+    const char* fn = "chromo_pcre_subsets";
+    CHROMO_TRY(check_subsets_args(cfg, params, in, var_gene, var_drop, variants, logits, var_logits, workspace, flags, fn));
+    SubsetsWs d;
+    CHROMO_TRY(subsets_ws(cfg, in->batch, variants, flags, &d, fn));
+    if (workspace_floats < d.total) {
+        set_error("%s: workspace too small: need %lld floats, got %lld", fn, (long long)d.total,
+                  (long long)workspace_floats);
+        return CHROMO_ENOMEM;
+    }
+    return subsets_run(cfg, params, in, var_gene, var_drop, variants, logits, var_logits, workspace, d, flags,
+                       (cudaStream_t)stream, nullptr, fn);
+}
+
+extern "C" int64_t chromo_freq_edits_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t variants,
+                                                      int32_t flags) {
+    if (validate_config(cfg) != CHROMO_OK) return CHROMO_EINVAL;
+    if (batch < 1 || variants < 1) { set_error("batch and variants must be >= 1"); return CHROMO_EINVAL; }
+    SubsetsWs d;
+    CHROMO_TRY(subsets_ws(cfg, batch, variants, flags, &d, "chromo_freq_edits"));
+    return freq_edits_total(d, variants);
+}
+
+extern "C" int chromo_freq_edits(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                                 const int32_t* var_gene, const float* var_freq, int32_t variants, float* logits,
+                                 float* var_logits, float* workspace, int64_t workspace_floats, int32_t flags,
+                                 void* stream) {
+    const char* fn = "chromo_freq_edits";
+    CHROMO_TRY(check_subsets_args(cfg, params, in, var_gene, var_freq, variants, logits, var_logits, workspace, flags, fn));
+    SubsetsWs d;
+    CHROMO_TRY(subsets_ws(cfg, in->batch, variants, flags, &d, fn));
+    const int64_t total = freq_edits_total(d, variants);
+    if (workspace_floats < total) {
+        set_error("%s: workspace too small: need %lld floats, got %lld", fn, (long long)total, (long long)workspace_floats);
+        return CHROMO_ENOMEM;
+    }
+    cudaStream_t st = (cudaStream_t)stream;
+    uint32_t* drop = reinterpret_cast<uint32_t*>(workspace + d.total);
+    if (cudaMemsetAsync(drop, 0, (size_t)variants * sizeof(uint32_t), st) != cudaSuccess) {
+        set_error("%s: memset failed", fn);
+        return CHROMO_ECUDA;
+    }
+    FreqSpliceArgs splice;
+    splice.var_gene = var_gene; splice.var_freq = var_freq; splice.var_drop = drop;
+    return subsets_run(cfg, params, in, var_gene, drop, variants, logits, var_logits, workspace, d, flags, st, &splice, fn);
 }
 
 // ---- histone-mark occlusion (occlusion.cu) ----

@@ -132,6 +132,18 @@ struct SubsetGuardArgs {
 int launch_subset_expand(const SubsetExpandArgs& a, cudaStream_t st);
 int launch_subset_guard(const SubsetGuardArgs& a, cudaStream_t st);
 
+// interaction-frequency edits (freq_edits.cu): after subset_expand_kernel with empty drop sets, variant v's freq takes
+// the non-NaN entries of var_freq[v]; an invalid variant (gene out of range, a +-inf entry) keeps its freq and gets the
+// drop word 0xffffffff, which subset_guard_kernel turns into a NaN logits row
+struct FreqSpliceArgs {
+    int B, I, V;
+    const int* var_gene;                            // [V]
+    const float* var_freq;                          // [V,S,S], NaN = keep
+    float* freq_v;                                  // [V,S,S] the replay's freq
+    uint32_t* var_drop;                             // [V] the (empty) drop sets of subset_expand_kernel
+};
+int launch_freq_splice(const FreqSpliceArgs& a, cudaStream_t st);
+
 // histone-mark occlusion (occlusion.cu): variant v = gene var_gene[v] with marks var_marks[v] zeroed over the bins
 // [var_bins[v, r, 0], var_bins[v, r, 1]) of pCRE slot var_slot[v] at every resolution r
 struct OcclusionDesc {

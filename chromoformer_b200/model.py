@@ -303,6 +303,7 @@ class _ChromoformerCore(nn.Module):
         object.__setattr__(self, "_packed_key", None)
         object.__setattr__(self, "_deletion_packed_key", None)
         object.__setattr__(self, "_subsets_packed_key", None)
+        object.__setattr__(self, "_freq_edits_packed_key", None)
         object.__setattr__(self, "_occlusion_packed_key", None)
         object.__setattr__(self, "_param_epoch", 0)
         self._rebuild_flat()
@@ -362,6 +363,7 @@ class _ChromoformerCore(nn.Module):
         object.__setattr__(self, "_packed_key", None)
         object.__setattr__(self, "_deletion_packed_key", None)
         object.__setattr__(self, "_subsets_packed_key", None)
+        object.__setattr__(self, "_freq_edits_packed_key", None)
         object.__setattr__(self, "_occlusion_packed_key", None)
 
     def _flat_is_current(self):
@@ -492,6 +494,34 @@ class _ChromoformerCore(nn.Module):
                    "chromo_pcre_subsets")
         if packed_key is not None:
             object.__setattr__(self, "_subsets_packed_key", packed_key)
+        return logits, var_logits
+
+    def _launch_freq_edits(self, io, var_gene, var_freq, flags):
+        """chromo_freq_edits: (logits [B, n_out], var_logits [V, n_out]) for the variant descriptors ``var_gene``
+        (int32 [V]) and ``var_freq`` (float32 [V, S, S], NaN = keep the gene's entry), both moved to the model's device.
+        Its workspace and packed BF16 weights are cached apart from the other entry points'."""
+        lib = _lib.load()
+        if not self._flat_is_current():
+            self._rebuild_flat()
+        dev, n_out = self._flat.device, int(self._cfg.n_out)
+        V, S = int(var_gene.numel()), int(io.cfg.i_max) + 1
+        if var_gene.dtype != torch.int32 or var_freq.dtype != torch.float32 or tuple(var_freq.shape) != (V, S, S):
+            raise ValueError(f"var_gene must be int32 [V] and var_freq float32 [V, {S}, {S}]")
+        var_gene, var_freq = var_gene.to(dev).contiguous(), var_freq.to(dev).contiguous()
+        ws = self._workspace(io.cfg, io.batch, flags, cached=True, entry="chromo_freq_edits_workspace_floats",
+                             variants=V)
+        packed_key = self._packed_key_of(ws, io, flags)
+        if packed_key is not None and packed_key == self._freq_edits_packed_key:
+            flags |= _lib.F_PACKED
+        logits = torch.empty(io.batch, n_out, dtype=torch.float32, device=dev)
+        var_logits = torch.empty(V, n_out, dtype=torch.float32, device=dev)
+        stream = torch.cuda.current_stream(dev).cuda_stream
+        _lib.check(lib.chromo_freq_edits(ctypes.byref(io.cfg), self._flat.data_ptr(), ctypes.byref(io.struct),
+                                         var_gene.data_ptr(), var_freq.data_ptr(), V, logits.data_ptr(),
+                                         var_logits.data_ptr(), ws.data_ptr(), ws.numel(), flags, stream),
+                   "chromo_freq_edits")
+        if packed_key is not None:
+            object.__setattr__(self, "_freq_edits_packed_key", packed_key)
         return logits, var_logits
 
     def _launch_occlusion(self, io, var_gene, var_slot, var_bins, var_marks, flags):

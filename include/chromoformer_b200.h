@@ -161,6 +161,30 @@ int chromo_pcre_subsets(const chromo_config_t* cfg, const float* params, const c
                         int32_t variants, float* logits /* [B,n_out] */, float* var_logits /* [V,n_out] */,
                         float* workspace, int64_t workspace_floats, int32_t flags, void* stream);
 
+/* ---- interaction-frequency edits: the logits with pCRE-promoter contact frequencies changed -----------------------
+ * For B genes with I = i_max slots (S = I + 1 tokens) and V variants.  Variant v is gene g = var_gene[v] with
+ *     interaction_freq[g, e] = var_freq[v, e]     for every e < S * S where var_freq[v, e] is not NaN
+ * (NaN: keep the gene's value); features and masks stay as they are.  The contact of pCRE i with the promoter is entry
+ * (0, i + 1), the only one the dataset writes; an entry of a pair masked at every resolution changes nothing.
+ *   logits[g]          the ordinary forward, bit-identical to chromo_forward with the same flags;
+ *   var_logits[v]      the logits of the edited gene, in variant order.
+ * interaction_freq is read only by the Regulation attention (the bias gamma_f * freq), so one Embedding + Pairwise pass
+ * per gene serves all its variants; the Regulation transformer and the head then run over the V variants, on the replay
+ * of chromo_pcre_subsets with empty drop sets and the edited freq spliced in.  Every GEMM takes the path the gene pass
+ * takes for the same B genes, so a variant's logits do not depend on V or on the other variants, and a variant that edits
+ * nothing gives the bits of chromo_pcre_subsets' empty drop set.  The descriptors (device memory) are checked on the
+ * device: var_gene outside [0, B) or a +-inf entry in var_freq[v] gets a NaN row in var_logits; the other rows are
+ * unaffected.  No atomics on the floating-point path; identical inputs give identical outputs; no host synchronisation
+ * (legal inside a stream capture).  Flags: CHROMO_F_BF16, CHROMO_F_PACKED and the CHROMO_F_DENSE hint (the gene pass
+ * only); any other flag, a NULL descriptor or output, or variants < 1 is CHROMO_EINVAL.  The workspace must hold
+ * chromo_freq_edits_workspace_floats floats (CHROMO_ENOMEM otherwise): the chromo_pcre_subsets bound plus V drop words
+ * (rounded up to 4); it keeps the packed BF16 weights at its front, as a chromo_forward workspace does.              */
+int64_t chromo_freq_edits_workspace_floats(const chromo_config_t* cfg, int32_t batch, int32_t variants, int32_t flags);
+int chromo_freq_edits(const chromo_config_t* cfg, const float* params, const chromo_batch_t* in,
+                      const int32_t* var_gene /* [V] device */, const float* var_freq /* [V,S,S] device, NaN = keep */,
+                      int32_t variants, float* logits /* [B,n_out] */, float* var_logits /* [V,n_out] */,
+                      float* workspace, int64_t workspace_floats, int32_t flags, void* stream);
+
 /* ---- histone-mark occlusion: the logits with marks removed over bin windows of one pCRE --------------------------
  * For B genes with I = i_max slots (S = I + 1 tokens), n_res resolutions of n_r bins and V variants.  Variant v is gene
  * g = var_gene[v] with
